@@ -2,6 +2,7 @@
 """bench.py -- throughput of the MaD local-feature hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|c2|c4|c5]
+                    [--dump-outputs DIR]
 
 Headline (`value`, `e2e`, `roofline`): one *step* = one pass of the hot path over one synthetic map of BASELINE.json
 configs[1] (C2): a 256^3 assembly map (8 A, 2 A/voxel, 6 random-walk components) through
@@ -20,8 +21,11 @@ the two paths that shard (SURVEY.md 8e), total work fixed ("strong"):
 `verified` (N > 1): the N-GPU results are compared inside the run with the 1-GPU results of the same inputs.
 
 `--impl reference` times the CPU restatement of the reference (oracle/mad_oracle.py, NumPy/SciPy -- the reference is
-pure Python and /root/reference does not exist on the GPU box) on a bounded, STAGE-WISE sample of the same C2 map,
+pure Python and not part of this repository) on a bounded, STAGE-WISE sample of the same C2 map,
 one process per host core (see cpu_stage_sample).
+
+`--dump-outputs DIR` (rank 0): after each workload's timed steps, what its last timed step returned goes to DIR/<name>.npy
+(see OutputDump), so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -310,16 +314,65 @@ class Ctx(object):
 
 
 def timed(ctx, fn, steps):
-    """K calls of fn between barrier + synchronize on both sides, CUDA events on the current stream -> ms."""
+    """K calls of fn between barrier + synchronize on both sides, CUDA events on the current stream -> (ms, what the
+    last call returned).  Only the last call's result is held, so every earlier step frees its outputs as before."""
     torch = ctx.torch
     ctx.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(steps):
+    for _ in range(steps - 1):
         fn()
+    last = fn()
     e1.record()
     ctx.barrier()
-    return e0.elapsed_time(e1)
+    return e0.elapsed_time(e1), last
+
+
+class OutputDump(object):
+    """--dump-outputs DIR: arrays a caller of a timed path receives, as DIR/<name>.npy.  Integer and float32 fields are
+    stored as float32 (exact: every index and count here is below 2^24), float64 scores as float64.  Tables too large
+    for the 64 MB budget are stored as a fixed, seeded sample of rows (``rows``), identical from run to run."""
+    LIMIT = 64 * 10 ** 6
+
+    def __init__(self, path):
+        self.path = path
+        self.nbytes = 0
+        os.makedirs(path, exist_ok=True)
+
+    @staticmethod
+    def rows(n, k, seed):
+        """k of n row positions (all when n <= k) in ascending order, fixed by the seed."""
+        if n <= k:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+
+    def put(self, name, a, dtype=np.float32):
+        a = np.ascontiguousarray(a, dtype=dtype)
+        self.nbytes += a.nbytes
+        if self.nbytes > self.LIMIT:
+            raise RuntimeError("--dump-outputs: %s takes the dump past %d bytes" % (name, self.LIMIT))
+        np.save(os.path.join(self.path, name + ".npy"), a)
+
+    def sample(self, t, k, seed):
+        """A seeded sample of k rows of the device tensor t (its first axis)."""
+        import torch
+        return t[torch.from_numpy(self.rows(int(t.shape[0]), k, seed)).to(t.device)]
+
+    def put_rows(self, name, t, k, seed, dtype=np.float32):
+        self.put(name, self.sample(t, k, seed).cpu().numpy(), dtype)
+
+    def put_keypoints(self, name, table):
+        """MadKeypoint rows (int32 [K, 12] on the device): vox[3], oct, off[3], val, peak[3], accepted."""
+        a = table.cpu().numpy()
+        out = a.astype(np.float32)
+        out[:, 4:8] = a[:, 4:8].view(np.float32)
+        self.put(name, out)
+
+    def put_oriented(self, name, table):
+        """MadOriented rows (int32 [D, 2] on the device) as (keypoint, main bin, secondary bin)."""
+        from mad_b200._lib import ORIENTED_DTYPE
+        a = np.ascontiguousarray(table.cpu().numpy()).view(ORIENTED_DTYPE).reshape(-1)
+        self.put(name, np.stack([a["kp"], a["main"], a["sec"]], 1))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -337,6 +390,21 @@ def c2_stages(V0, V1, K, D):
         "orient": (("orient_kernel", "compact_oriented_kernel", "cub_exclusive_sum"), 58956 * K),
         "describe": (("describe_kernel",), 51200 * D),
     }
+
+
+def dump_c2(dump, sp, kp, ori, dsc, pairs):
+    """One C2 step: the counts (keypoints, oriented features, pairs), the keypoint and oriented-feature tables, and seeded
+    samples of the descriptor rows, of the pair list (hi row, lo row, score) and of both octaves' LoG grids."""
+    ph, pl, sc = pairs
+    dump.put("c2_counts", [len(kp), len(ori), int(ph.numel())], np.float64)
+    dump.put_keypoints("c2_keypoints", kp.table[:len(kp)])
+    dump.put_oriented("c2_oriented", ori.table[:len(ori)])
+    dump.put_rows("c2_descriptors", dsc, 2048, 1)
+    dump.put_rows("c2_pair_hi", ph, 1 << 19, 2)
+    dump.put_rows("c2_pair_lo", pl, 1 << 19, 2)
+    dump.put_rows("c2_pair_score", sc, 1 << 19, 2, np.float64)
+    for o in range(2):
+        dump.put_rows("c2_log%d" % o, sp.logs[o].reshape(-1), 1 << 19, 3 + o)
 
 
 def bench_c2(ctx, args):
@@ -401,17 +469,20 @@ def bench_c2(ctx, args):
     P.profile_enable(True)
     l0 = P.launch_count()
     t_wall0 = time.perf_counter()
-    ms = timed(ctx, step_device, args.steps)
+    ms, last = timed(ctx, step_device, args.steps)
     t_wall1 = time.perf_counter()
     launches = P.launch_count() - l0
     recs = P.profile_records()
     P.profile_enable(False)
+    if args.dump is not None:
+        dump_c2(args.dump, *last)
+    del last
 
     # ---- e2e: host buffers in and out
     out = run_e2e(2)
     d2h = int(sum(t.numel() * t.element_size() for t in out.values()))
     d2h_detail = {k: int(t.numel() * t.element_size()) for k, t in out.items()}
-    ms_e2e = timed(ctx, lambda: run_e2e(args.steps), 1)
+    ms_e2e, _ = timed(ctx, lambda: run_e2e(args.steps), 1)
     clocks = sampler.summary(t_wall0, t_wall1) if ctx.rank == 0 else None
     if ctx.rank == 0:
         sampler.stop()
@@ -546,7 +617,7 @@ def bench_c5(ctx, args):
         stage.sync()
         return out
 
-    steps = max(3, min(args.steps, 20))
+    steps = args.steps
     for _ in range(max(args.warmup, 3)):
         idx, sc = step_device()
     # ---- parity inside the run: sampled hi rows against the whole lo set on ONE GPU (the same kernel, unsharded)
@@ -561,13 +632,17 @@ def bench_c5(ctx, args):
         del full, sub
     P.profile_enable(True)
     l0 = P.launch_count()
-    ms = timed(ctx, step_device, steps)
+    ms, last = timed(ctx, step_device, steps)
     launches = P.launch_count() - l0
     recs = P.profile_records()
     P.profile_enable(False)
+    if args.dump is not None:
+        args.dump.put("c5_topk_index", last[0].cpu().numpy())
+        args.dump.put("c5_topk_score", last[1].cpu().numpy(), np.float64)
+    del last
     out = step_e2e()
     d2h = int(sum(t.numel() * t.element_size() for t in out))
-    ms_e2e = timed(ctx, step_e2e, steps)
+    ms_e2e, _ = timed(ctx, step_e2e, steps)
     ms, ms_e2e = ctx.max_over_ranks(ms, ms_e2e)
     kms = [t for nm, t in recs if nm == "match_u8_topk_kernel"]
     # device time of the matching kernel per step (a step may take two launches: the full waves and the tail rows)
@@ -613,6 +688,16 @@ def bench_c5(ctx, args):
 # ---------------------------------------------------------------------------------------------
 # C4: a batch of 64 snapshot maps, map i -> rank i mod N (SURVEY 8e)
 # ---------------------------------------------------------------------------------------------
+def dump_c4(dump, res):
+    """One C4 step (this rank's maps, in order): per map (keypoints, oriented features), and seeded samples of the rows of
+    the maps' keypoint, oriented-feature and descriptor tables put end to end (keypoint indices stay per map)."""
+    import torch
+    dump.put("c4_counts", [[r["n_kp"], r["n_dsc"]] for r in res], np.float64)
+    dump.put_keypoints("c4_keypoints", dump.sample(torch.cat([r["kp"] for r in res]), 1 << 16, 4))
+    dump.put_oriented("c4_oriented", dump.sample(torch.cat([r["ori"] for r in res]), 1 << 17, 5))
+    dump.put_rows("c4_descriptors", torch.cat([r["dsc"] for r in res]), 1024, 6)
+
+
 def bench_c4(ctx, args):
     torch = ctx.torch
     from mad_b200 import pipeline as P
@@ -647,15 +732,18 @@ def bench_c4(ctx, args):
             ok = ok and torch.equal(d1, tabs[u])
         verified = ctx.all_true(ok)
         del tabs
-    steps = max(2, min(args.steps, 10))
+    steps = args.steps
     P.profile_enable(True)
     l0 = P.launch_count()
-    ms = timed(ctx, lambda: step(False), steps)
+    ms, last = timed(ctx, lambda: step(False), steps)
     launches = P.launch_count() - l0
     recs = P.profile_records()
     P.profile_enable(False)
+    if args.dump is not None:
+        dump_c4(args.dump, last[0])
+    del last
     step(True)
-    ms_e2e = timed(ctx, lambda: step(True), steps)
+    ms_e2e, _ = timed(ctx, lambda: step(True), steps)
     ms, ms_e2e = ctx.max_over_ranks(ms, ms_e2e)
     K_tot = float(sum(int(r["n_kp"]) for r in res))
     D_tot = float(sum(int(r["n_dsc"]) for r in res))
@@ -713,7 +801,15 @@ def main():
     ap.add_argument("--match-impl", type=int, default=None, help="default: product (uint8 tcgen05 one-pass); 1 = SIMT check, 2 = fp16 tcgen05")
     ap.add_argument("--exact", type=int, default=1, help="1 = float64 line accumulation (bit-exact with SciPy)")
     ap.add_argument("--full-format", action="store_true", help="e2e downloads int16 descriptors and float64 scores instead of the compact format")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each workload returned to DIR/<name>.npy (at most 64 MB); "
+                         "under torchrun rank 0 writes its own results only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computes (--impl ours)")
+    args.dump = OutputDump(args.dump_outputs) if args.dump_outputs and int(os.environ.get("RANK", "0")) == 0 else None
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

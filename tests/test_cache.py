@@ -2,7 +2,6 @@
 import os
 
 import numpy as np
-import pytest
 
 import helpers as H
 
@@ -37,35 +36,18 @@ def test_descriptor_cache_round_trip(tmp_path):
         assert np.array_equal(a.subv_map_coords, b.subv_map_coords) and np.array_equal(a.coords, b.coords)
 
 
-REF_DF_PY = "/root/reference/mad/DensityFeature.py"
-
-
-def _reference_density_feature():
-    """The reference's record class, loaded from its own file (its one relative import, the EQSP sphere used by the VMD
-    helpers only, is satisfied by a stand-in package)."""
-    import importlib.util
-    import sys
-    import types
-    pkg, sub, mod = types.ModuleType("_refpkg"), types.ModuleType("_refpkg.eqsp"), types.ModuleType("_refpkg.eqsp.eqsp")
-    pkg.__path__, sub.__path__ = [], []
-    mod.EQSP_Sphere = object
-    sys.modules.update({"_refpkg": pkg, "_refpkg.eqsp": sub, "_refpkg.eqsp.eqsp": mod})
-    spec = importlib.util.spec_from_file_location("_refpkg.DensityFeature", REF_DF_PY)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m.DensityFeature
-
-
 def _plain(v):
     return v.tolist() if isinstance(v, np.ndarray) else v
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_DF_PY), reason="needs the reference tree (build container only)")
 def test_density_feature_record_equals_the_reference_record():
     """Every attribute our record carries has the reference's value after the same constructor / setter calls
-    (mad/DensityFeature.py:6-84); the reference's extra attributes are its per-feature scratch arrays."""
+    (mad/DensityFeature.py:6-84); the reference's extra attributes are its per-feature scratch arrays.
+    tests/golden/density_feature_record.json holds, per call sequence below, the reference record's attributes outside
+    those scratch arrays (vars() of the reference's DensityFeature, values as plain lists / numbers); the reference
+    creates lin_ar_subeqsp only when a descriptor is set (mad/Descriptor.py:198, set_from_file_dsc)."""
+    import json
     from mad_b200.DensityFeature import DensityFeature
-    Ref = _reference_density_feature()
     rf = np.arange(9.0).reshape(3, 3)
     calls = [
         [],
@@ -75,19 +57,21 @@ def test_density_feature_record_equals_the_reference_record():
         [("set_from_file_ori", (3, 5, 17, 1, 112, [1, 2, 3], [4.0, 5.0, 6.0], [4.5, 5.5, 6.5], rf, np.arange(112)))],
         [("set_from_file_dsc", (3, 5, 17, 0, 112, 16, [1, 2, 3], [4.0, 5.0, 6.0], [4.5, 5.5, 6.5], rf, np.arange(1024)))],
     ]
+    with open(os.path.join(H.GOLD, "density_feature_record.json")) as f:
+        reference = json.load(f)
+    assert len(reference) == len(calls)
     scratch = {"grad_box", "magn_box", "ar_magn", "ar_count", "norm_zone_counts", "interp_grad_box", "ar_subcount",
                "lin_magn_sudo", "step_ar_counts", "step_v_counts"}
-    for seq in calls:
-        ours, ref = DensityFeature(), Ref()
+    for seq, theirs in zip(calls, reference):
+        ours = DensityFeature()
         for name, args in seq:
             getattr(ours, name)(*args)
-            getattr(ref, name)(*args)
-        mine, theirs = vars(ours), vars(ref)
+        mine = vars(ours)
         for k, v in mine.items():
             if k == "lin_ar_subeqsp" and k not in theirs:      # the reference creates it in step06 only (mad/Descriptor.py:198)
                 assert v == []
                 continue
             assert k in theirs, k
-            assert _plain(v) == _plain(theirs[k]), (seq, k)
+            assert _plain(v) == theirs[k], (seq, k)
         missing = set(theirs) - set(mine) - scratch
         assert not missing, missing

@@ -1,10 +1,11 @@
 """The ``mad`` drop-in package (SURVEY.md 8b: "run_MaD.py and the notebooks drop in unchanged"): the reference's module
 names bound to mad_b200, and the reference's own orchestrator file loaded on top of them (mad/MaD.py of this repo).
 
-CPU: name binding, the loader's error without the orchestrator file, and -- in the build container, where
-/root/reference exists -- that the reference's MaD.py executes on top of the package with every hot-path name resolved to
-mad_b200 (no compute).  GPU: the call sequences of ``MaD._describe_struct`` (mad/MaD.py:358-368) and ``MaD._match_dsc``
-(mad/MaD.py:414-453) written against the ``mad.*`` names, on config C1 and the matching fixtures."""
+CPU: name binding, the loader's error without the orchestrator file, and -- when MAD_REFERENCE_MAD_PY names the
+reference's mad/MaD.py, which is not part of this repository -- that it executes on top of the package with every
+hot-path name resolved to mad_b200 (no compute).  GPU: the call sequences of ``MaD._describe_struct``
+(mad/MaD.py:358-368) and ``MaD._match_dsc`` (mad/MaD.py:414-453) written against the ``mad.*`` names, on config C1 and
+the matching fixtures."""
 import importlib
 import os
 import sys
@@ -14,7 +15,7 @@ import pytest
 
 import helpers as H
 
-REF_MAD_PY = "/root/reference/mad/MaD.py"
+REF_MAD_PY = os.environ.get("MAD_REFERENCE_MAD_PY", "")
 
 
 def test_reference_module_names_are_bound_to_mad_b200():
@@ -37,7 +38,7 @@ def test_orchestrator_is_not_shipped(monkeypatch):
         importlib.import_module("mad.MaD")
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_MAD_PY), reason="needs the reference tree (build container only)")
+@pytest.mark.skipif(not os.path.isfile(REF_MAD_PY), reason="needs the reference's mad/MaD.py (MAD_REFERENCE_MAD_PY)")
 def test_reference_orchestrator_loads_on_top_of_the_package(monkeypatch, tmp_path):
     """run_MaD.py:63-76 up to the first compute call: ``MaD.MaD()``, ``add_map``, ``add_subunit``."""
     import ref_shims
