@@ -34,6 +34,7 @@ extern "C" {
 
 #define MAD_MAX_ORI 36        /* <= 6 main x 6 secondary orientations per keypoint            */
 #define MAD_DSC_LEN 1024      /* 64 sub-blocks x 16 zones                                      */
+#define MAD_DSC_REFUSED (1 << 30) /* max_entry of a set that is not a descriptor set (see mad_dsc_prepare) */
 
 /* One detected keypoint (mad/Detector.py:30-45, mad/DensityFeature.py:35-41). */
 typedef struct MadKeypoint {
@@ -202,8 +203,14 @@ int mad_describe(const float* grad4_oct0, const float* grad4_oct1, const int* di
  * tcgen05 kind::i8 kernel, exact while
  * max_entry <= 255 (true for every patch size <= 24: an entry counts the votes of one sub-block).
  * rnorm: float 1/sqrt(norm2) per padded row (0 for zero rows), the fp32 pre-filter's scale.
- * half: optional fp16 copy for the general tensor-core kernel (impl = 2, entries <= 2048).
- * dsc is only read by the SIMT check kernel (impl = 1). */
+ * half: optional fp16 copy for the general tensor-core kernel (impl = 2).  That kernel accumulates in fp32, which is
+ * exact while every partial sum of a dot product stays <= 2^24: it accepts a pair of sets only if every entry lies in
+ * [0, 2048] (exact in fp16) and max_norm2(hi) * max_norm2(lo) <= 2^48 (by Cauchy-Schwarz every dot product, and so
+ * every partial sum of non-negative terms, is then <= 2^24).  The SIMT kernel (impl = 1) is exact in int32 for any
+ * set whose squared norms fit int32.
+ * dsc is only read by the SIMT check kernel (impl = 1).
+ * A set with a negative entry or a squared norm >= 2^31 is not a descriptor set: mad_dsc_prepare reports it with
+ * max_entry = MAD_DSC_REFUSED, and every matching entry point refuses it (MAD_ERR_ARG). */
 typedef struct MadDscSet {
     const int16_t* dsc;   /* [rows][1024] */
     const void* half;     /* [rows_padded][1024] fp16, or NULL */
@@ -212,13 +219,16 @@ typedef struct MadDscSet {
     const float* rnorm;   /* [rows_padded], or NULL */
     int32_t rows;
     int32_t rows_padded;
-    int32_t max_entry;    /* largest descriptor entry (host copy of what mad_dsc_prepare found) */
+    int32_t max_entry;    /* largest descriptor entry (host copy of what mad_dsc_prepare found; -1 = not known) */
+    int32_t max_norm2;    /* largest squared norm (host copy of what mad_dsc_prepare found; -1 = not known) */
 } MadDscSet;
 
 /* Fills norm2[rows], rnorm[rows_padded], u8[rows_padded][1024] (may be NULL) and atomically
- * raises *max_entry (device int32, caller zeroes it) to the largest entry seen. */
+ * raises *max_entry (device int32, caller zeroes it) to the largest entry seen -- MAD_DSC_REFUSED if an entry is
+ * negative or a squared norm is >= 2^31 -- and *max_norm2 (device int32, caller zeroes it; may be NULL) to the
+ * largest squared norm. */
 int mad_dsc_prepare(const int16_t* dsc, int rows, int rows_padded, int32_t* norm2, float* rnorm,
-                    uint8_t* u8, int32_t* max_entry, void* stream);
+                    uint8_t* u8, int32_t* max_entry, int32_t* max_norm2, void* stream);
 int mad_dsc_norms(const int16_t* dsc, int rows, int32_t* norm2, void* stream);
 int mad_dsc_to_half(const int16_t* dsc, int rows, int rows_padded, void* half_out, void* stream);
 
@@ -229,7 +239,7 @@ int mad_dsc_to_half(const int16_t* dsc, int rows, int rows_padded, void* half_ou
  * exclusive scan over that array in memory order (mad_exclusive_scan_i32_to_i64, n = M*n_seg)
  * FILL writes pair_hi / pair_lo / pair_score starting at seg_offset[i][s], lo ascending -- i.e. the
  * row-major order of np.where(preds > cc) (mad/MaD.py:423-424).
- * impl: 1 = SIMT integer kernel (device-side check), 2 = fp16 tcgen05 kernel (entries <= 2048).
+ * impl: 1 = SIMT integer kernel (device-side check), 2 = fp16 tcgen05 kernel (only where it is exact: see MadDscSet).
  * The product path for threshold matching is the ONE-pass mad_match_pairs below; impl 0 (that kernel) has no
  * count / fill form and is REJECTED here with MAD_ERR_ARG and a message (never silently remapped).
  * mad_match_segments(M, N, 0) only sizes the top-k workspace of the uint8 kernel. */
@@ -263,16 +273,20 @@ int mad_match_pairs_finish_dot(const uint64_t* cand_key, const int32_t* cand_dot
                                int32_t* pair_hi, int32_t* pair_lo, int32_t* pair_dot, void* workspace, size_t workspace_bytes,
                                void* stream);
 
-/* Top-k mode (extension, SURVEY.md 8c): per hi row the k best lo rows by (score desc, index asc);
- * lo_index_base is added to the stored indices (sharded reference axis).  k <= 32.
- * topk_idx[M][k] (-1 padded), topk_score[M][k] float64 (-inf padded).  Workspace: per-segment
- * partial lists (mad_match_topk_workspace_bytes).  impl: 0 = uint8 tcgen05 kernel (product; needs
- * max_entry <= 255), 1 = SIMT check kernel, 2 = fp16 tcgen05 kernel. */
+/* Top-k mode (extension, SURVEY.md 8c): per hi row the k best lo rows by (score desc, index asc), where the score is
+ * the float64 cosine of the threshold mode (bit for bit) and equal scores go to the lower index; lo_index_base is added
+ * to the stored indices (sharded reference axis).  k <= 32.
+ * topk_idx[M][k] (-1 padded), topk_score[M][k] float64 (-inf padded); a row whose indices are all -2
+ * (MAD_TOPK_INCOMPLETE: an internal hand-off of the kernel timed out) means the list is incomplete -- discard the call's
+ * result.  Workspace: per-segment partial lists (mad_match_topk_workspace_bytes).  impl: 0 = uint8 tcgen05 kernel
+ * (product; needs max_entry <= 255), 1 = SIMT check kernel, 2 = fp16 tcgen05 kernel (see MadDscSet). */
 size_t mad_match_topk_workspace_bytes(int M, int N, int k, int impl);
 int mad_match_topk(const MadDscSet* hi, const MadDscSet* lo, int k, int lo_index_base,
                    int32_t* topk_idx, double* topk_score, void* workspace, size_t workspace_bytes,
                    int impl, void* stream);
-/* Merges G per-shard top-k lists [G][M][k] into one [M][k] with the same ordering rule. */
+/* Merges G per-shard top-k lists [G][M][k] into one [M][k] with the same ordering rule (-1 entries are padding); a row
+ * with a -2 entry in any input list comes out as all -2 (list incomplete, discard the call's result). */
+#define MAD_TOPK_INCOMPLETE (-2)
 int mad_topk_merge(const int32_t* idx_in, const double* score_in, int G, int M, int k,
                    int32_t* idx_out, double* score_out, void* stream);
 

@@ -29,6 +29,8 @@ ORIENTED_DTYPE = np.dtype([("kp", "<i4"), ("main", "<i2"), ("sec", "<i2")])
 assert KEYPOINT_DTYPE.itemsize == 48 and ORIENTED_DTYPE.itemsize == 8
 MAX_ORI = 36
 DSC_LEN = 1024
+DSC_REFUSED = 1 << 30          # max_entry of a set that is not a descriptor set (negative entry / squared norm >= 2^31)
+TOPK_INCOMPLETE = -2           # top-k index of an incomplete list (kernel hand-off time-out): discard the result
 TOPK_MAX = 32
 ZONE_FAST_BYTES = 2048
 
@@ -40,7 +42,8 @@ class MadZoneTable(C.Structure):
 
 class MadDscSet(C.Structure):
     _fields_ = [("dsc", C.c_void_p), ("half", C.c_void_p), ("norm2", C.c_void_p), ("u8", C.c_void_p),
-                ("rnorm", C.c_void_p), ("rows", C.c_int32), ("rows_padded", C.c_int32), ("max_entry", C.c_int32)]
+                ("rnorm", C.c_void_p), ("rows", C.c_int32), ("rows_padded", C.c_int32), ("max_entry", C.c_int32),
+                ("max_norm2", C.c_int32)]
 
 
 _P = C.c_void_p
@@ -81,7 +84,7 @@ SIGNATURES = {
     "mad_compact_oriented_workspace_bytes": (_SZ, [_I]),
     "mad_compact_oriented": (_I, [_P, _P, _I, _P, _I, _P, _P, _SZ, _P]),
     "mad_describe": (_I, [_P, _P, _P, _P, _P, _I, _I, C.POINTER(MadZoneTable), _P, _P, _I, _P, _P]),
-    "mad_dsc_prepare": (_I, [_P, _I, _I, _P, _P, _P, _P, _P]),
+    "mad_dsc_prepare": (_I, [_P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mad_match_pairs": (_I, [C.POINTER(MadDscSet), C.POINTER(MadDscSet), C.c_double, _P, _P, C.c_uint64, _P, _P]),
     "mad_match_pairs_finish_workspace_bytes": (_SZ, [C.c_longlong]),
     "mad_match_pairs_finish": (_I, [_P, _P, C.c_longlong, _I, _I, _P, _P, _P, _P, _P, _P, _SZ, _P]),

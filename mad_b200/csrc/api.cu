@@ -94,15 +94,38 @@ extern "C" int mad_device_info(int* sm_count, int* cc_major, int* cc_minor) {
     return MAD_OK;
 }
 
+int mad_check_descriptor_sets(const MadDscSet* hi, const MadDscSet* lo, const char* who) {
+    if (hi->max_entry >= MAD_DSC_REFUSED || lo->max_entry >= MAD_DSC_REFUSED) {
+        mad_set_error("%s: not a descriptor set (a negative entry, or a squared norm >= 2^31)", who);
+        return MAD_ERR_ARG;
+    }
+    return MAD_OK;
+}
+
+// The fp16 kernel accumulates in fp32: exact while every partial sum of a dot product is <= 2^24.  Entries in [0, 2048]
+// are exact in fp16, and with max |hi|^2 * max |lo|^2 <= 2^48 every dot product is <= 2^24 (Cauchy-Schwarz).
+static bool fp16_exact(const MadDscSet* hi, const MadDscSet* lo) {
+    return hi->max_entry >= 0 && lo->max_entry >= 0 && hi->max_entry <= 2048 && lo->max_entry <= 2048 &&
+           hi->max_norm2 >= 0 && lo->max_norm2 >= 0 && (double)hi->max_norm2 * (double)lo->max_norm2 <= 281474976710656.0;
+}
+
 static int check_sets(const MadDscSet* hi, const MadDscSet* lo, int impl) {
     MAD_CHECK_ARG(hi && lo && hi->rows >= 0 && lo->rows >= 0);
     MAD_CHECK_ARG(impl == 0 || impl == 1 || impl == 2);
     if (hi->rows == 0 || lo->rows == 0) return MAD_OK;
     MAD_CHECK_ARG(hi->norm2 && lo->norm2);
+    const int rc = mad_check_descriptor_sets(hi, lo, "mad_match");
+    if (rc != MAD_OK) return rc;
     if (impl == 1) {
         MAD_CHECK_ARG(hi->dsc && lo->dsc);
     } else {
         if (impl == 2) MAD_CHECK_ARG(hi->half && lo->half);
+        if (impl == 2 && !fp16_exact(hi, lo)) {
+            mad_set_error("mad_match: the fp16 kernel (impl = 2) is exact only for entries in [0, 2048] and max |hi|^2 * max "
+                          "|lo|^2 <= 2^48 (here max entry %d / %d, max |.|^2 %d / %d; -1 = not known): use impl = 1",
+                          hi->max_entry, lo->max_entry, hi->max_norm2, lo->max_norm2);
+            return MAD_ERR_ARG;
+        }
         if (impl == 0) MAD_CHECK_ARG(hi->u8 && lo->u8 && lo->rnorm);
         MAD_CHECK_ARG(hi->rows_padded >= hi->rows && hi->rows_padded % 128 == 0);
         MAD_CHECK_ARG(lo->rows_padded >= lo->rows && lo->rows_padded % 128 == 0);

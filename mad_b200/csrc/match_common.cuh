@@ -48,56 +48,28 @@ __device__ __forceinline__ void mad_top8_insert(double (&bs)[8], int (&bi)[8], d
     bi[0] = c[0] ? id : bi[0];
 }
 
-// Integer-keyed variant: an entry is (dot, |lo|^2, index) and, the hi row being the same for the whole list,
-// score_a > score_b  <=>  dot_a^2 * n_b > dot_b^2 * n_a  -- exact in 128-bit integers (dot^2 < 2^53, n < 2^27), no square
-// root or division per candidate.  Equal ratios fall back to the index like equal scores do.  (Two different ratios that
-// round to the same float64 score are ordered by their true value here and by index in an argsort of the rounded scores: a
-// difference below 1e-16 relative, outside what the tests -- "away from exact ties" -- and any consumer can see.)
-__device__ __forceinline__ bool mad_ratio_before(int d, int n, int id, int pd, int pn, int pi) {
-    if (pi < 0) return true;                                          // empty slots rank last
-    const unsigned long long a = (unsigned long long)((long long)d * d), b = (unsigned long long)((long long)pd * pd);
-    const unsigned long long alo = a * (unsigned long long)pn, ahi = __umul64hi(a, (unsigned long long)pn);
-    const unsigned long long blo = b * (unsigned long long)n, bhi = __umul64hi(b, (unsigned long long)n);
-    if (ahi != bhi) return ahi > bhi;
-    if (alo != blo) return alo > blo;
-    return id < pi;
-}
-
-__device__ __forceinline__ void mad_top8i_insert(int (&td)[8], int (&tn)[8], int (&bi)[8], int d, int n, int id) {
-    bool c[8];
-#pragma unroll
-    for (int q = 0; q < 8; ++q) c[q] = mad_ratio_before(d, n, id, td[q], tn[q], bi[q]);
-#pragma unroll
-    for (int q = 7; q >= 1; --q) {
-        td[q] = c[q - 1] ? td[q - 1] : (c[q] ? d : td[q]);
-        tn[q] = c[q - 1] ? tn[q - 1] : (c[q] ? n : tn[q]);
-        bi[q] = c[q - 1] ? bi[q - 1] : (c[q] ? id : bi[q]);
-    }
-    td[0] = c[0] ? d : td[0];
-    tn[0] = c[0] ? n : tn[0];
-    bi[0] = c[0] ? id : bi[0];
-}
-
-// The same list with a float32 image of every entry's score (relative error < 1e-6): the order of two entries is decided on
-// the images whenever they differ by more than 4e-6 of the larger one, and on the exact integer ratios otherwise -- the same
-// order as mad_top8i_insert's at a fraction of the instructions (the 128-bit products are needed for near-ties only).
+// Register list of 8 entries (float32 image of the score, dot, |lo|^2, index) for ONE hi row (|hi|^2 = n2a).  The images have
+// a relative error < 1e-6, so two entries whose images differ by more than 4e-6 of the larger one are ordered by them; closer
+// ones are ordered as every other path orders them: by the float64 mad_score, then by the index.  (Equal integer ratios
+// dot^2 / |lo|^2 do not imply equal float64 scores: a lo row b and its multiple m b have the same cosine, yet their two
+// roundings of d / sqrt(n_a n_b) and m d / sqrt(n_a m^2 n_b) differ by one ulp in about a third of the cases.)
 // (out of line: it runs for near-ties only and must not bloat its callers -- the matcher's warps share one instruction cache)
-static __device__ __noinline__ bool mad_ratio_before_nl(int d, int n, int id, int pd, int pn, int pi) {
-    return mad_ratio_before(d, n, id, pd, pn, pi);
+static __device__ __noinline__ bool mad_score_before_nl(int d, int n, int id, int pd, int pn, int pi, double n2a) {
+    return mad_topk_before(mad_score(d, n2a, (double)n), id, mad_score(pd, n2a, (double)pn), pi);
 }
-__device__ __forceinline__ bool mad_score32_before(float s, int d, int n, int id, float ps, int pd, int pn, int pi) {
+__device__ __forceinline__ bool mad_score32_before(float s, int d, int n, int id, float ps, int pd, int pn, int pi, double n2a) {
     if (pi < 0) return true;
     const float tol = 4e-6f * fmaxf(s, ps);
     if (s > ps + tol) return true;
     if (s < ps - tol) return false;
-    return mad_ratio_before_nl(d, n, id, pd, pn, pi);
+    return mad_score_before_nl(d, n, id, pd, pn, pi, n2a);
 }
 
 // Called by ALL lanes of a warp (`active` = this lane has a candidate).  The eight position decisions are taken on the
 // images; only if some lane of the warp has an image within the tolerance of one of its entries does the warp redo the
-// decisions on the exact ratios (one warp-uniform branch: the 128-bit products stay off the common path).
+// decisions on the float64 scores (one warp-uniform branch: square roots and divisions stay off the common path).
 __device__ __forceinline__ void mad_top8f_insert(float (&ts)[8], int (&td)[8], int (&tn)[8], int (&bi)[8], bool active, float s,
-                                                 int d, int n, int id) {
+                                                 int d, int n, int id, double n2a) {
     bool c[8];
     bool amb = false;
 #pragma unroll
@@ -111,7 +83,7 @@ __device__ __forceinline__ void mad_top8f_insert(float (&ts)[8], int (&td)[8], i
     }
     if (__any_sync(0xFFFFFFFFu, amb)) {
 #pragma unroll
-        for (int q = 0; q < 8; ++q) c[q] = active && mad_score32_before(s, d, n, id, ts[q], td[q], tn[q], bi[q]);
+        for (int q = 0; q < 8; ++q) c[q] = active && mad_score32_before(s, d, n, id, ts[q], td[q], tn[q], bi[q], n2a);
     }
 #pragma unroll
     for (int q = 7; q >= 1; --q) {
@@ -154,6 +126,9 @@ __device__ __forceinline__ uint32_t mad_select32(const uint32_t (&v)[32], int j)
 
 // Both kernels cut the lo axis into S segments of `tiles_per_seg` 256-column tiles.
 #define MAD_MATCH_SEG_TILE 256
+
+// MAD_ERR_ARG (with a message naming `who`) if either set is flagged as not a descriptor set (MAD_DSC_REFUSED).
+int mad_check_descriptor_sets(const MadDscSet* hi, const MadDscSet* lo, const char* who);
 
 int mad_match_simt(const int16_t* hi, int M, const int16_t* lo, int N, const int32_t* hi_n2, const int32_t* lo_n2,
                    double cc, int mode, int S, int32_t* seg_count, const int64_t* seg_offset, int32_t* pair_hi,

@@ -9,10 +9,12 @@
 namespace {
 
 // One warp per (padded) row: squared norm, 1/sqrt(norm) as float, uint8 copy (values clamped to
-// 255 -- max_entry tells the host whether the copy is exact), zero rows beyond `rows`.
+// 255 -- max_entry tells the host whether the copy is exact), zero rows beyond `rows`; the set's largest
+// squared norm (which kernels compute the dot products exactly) goes to max_norm2.
 __global__ void __launch_bounds__(256)
 dsc_prepare_kernel(const int16_t* __restrict__ dsc, int rows, int rows_padded, int32_t* __restrict__ norm2,
-                   float* __restrict__ rnorm, uint8_t* __restrict__ u8, int32_t* __restrict__ max_entry) {
+                   float* __restrict__ rnorm, uint8_t* __restrict__ u8, int32_t* __restrict__ max_entry,
+                   int32_t* __restrict__ max_norm2) {
     const int row = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5);
     const int lane = threadIdx.x & 31;
     if (row >= rows_padded) return;
@@ -31,7 +33,7 @@ dsc_prepare_kernel(const int16_t* __restrict__ dsc, int rows, int rows_padded, i
                 const int e0 = (int)(int16_t)(w[h] & 0xFFFFu), e1 = (int)(int16_t)(w[h] >> 16);
                 acc += (long long)e0 * e0 + (long long)e1 * e1;
                 mx = max(mx, max(e0, e1));
-                if (e0 < 0 || e1 < 0) mx = 1 << 30;             // negative entries: not a descriptor
+                if (e0 < 0 || e1 < 0) mx = MAD_DSC_REFUSED;     // negative entries: not a descriptor
                 const uint32_t b0 = (uint32_t)min(max(e0, 0), 255), b1 = (uint32_t)min(max(e1, 0), 255);
                 const int slot = q * 8 + h * 2;                  // byte index within the lane's 32 bytes
                 if ((slot & 3) == 0) packed[slot >> 2] = b0 | (b1 << 8);
@@ -53,10 +55,11 @@ dsc_prepare_kernel(const int16_t* __restrict__ dsc, int rows, int rows_padded, i
         mx = max(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, o));
     }
     if (lane == 0) {
-        if (acc > 0x7FFFFFFFLL) mx = 1 << 30;                    // norm does not fit int32: refuse the set
+        if (acc > 0x7FFFFFFFLL) mx = MAD_DSC_REFUSED;           // norm does not fit int32: refuse the set
         if (row < rows) norm2[row] = (int32_t)acc;
         rnorm[row] = acc > 0 ? (float)(1.0 / sqrt((double)acc)) : 0.f;
         if (mx > 0) atomicMax(max_entry, mx);
+        if (max_norm2 && acc > 0) atomicMax(max_norm2, (int32_t)min(acc, 0x7FFFFFFFLL));
     }
 }
 
@@ -113,14 +116,14 @@ FinishLayout finish_layout(long long n) {
 }  // namespace
 
 extern "C" int mad_dsc_prepare(const int16_t* dsc, int rows, int rows_padded, int32_t* norm2, float* rnorm,
-                               uint8_t* u8, int32_t* max_entry, void* stream) {
+                               uint8_t* u8, int32_t* max_entry, int32_t* max_norm2, void* stream) {
     MAD_CHECK_ARG(rows >= 0 && rows_padded >= rows);
     if (rows_padded == 0) return MAD_OK;
     MAD_CHECK_ARG((rows == 0 || dsc) && norm2 && rnorm && max_entry);
     MAD_CHECK_ARG((reinterpret_cast<uintptr_t>(dsc) & 15) == 0 && (reinterpret_cast<uintptr_t>(u8) & 15) == 0);
     MAD_PROF("dsc_prepare_kernel", stream);
     dsc_prepare_kernel<<<(unsigned)mad_ceil_div((long long)rows_padded * 32, 256), 256, 0, (cudaStream_t)stream>>>(
-        dsc, rows, rows_padded, norm2, rnorm, u8, max_entry);
+        dsc, rows, rows_padded, norm2, rnorm, u8, max_entry, max_norm2);
     MAD_LAUNCH_OK();
     return MAD_OK;
 }
@@ -138,9 +141,11 @@ extern "C" int mad_match_pairs(const MadDscSet* hi, const MadDscSet* lo, double 
     MAD_CHECK_ARG(hi->u8 && lo->u8 && hi->norm2 && lo->norm2 && lo->rnorm && cand_key && cand_dot);
     MAD_CHECK_ARG(hi->rows_padded >= hi->rows && hi->rows_padded % 128 == 0);
     MAD_CHECK_ARG(lo->rows_padded >= lo->rows && lo->rows_padded % 128 == 0);
+    int rc = mad_check_descriptor_sets(hi, lo, "mad_match_pairs");
+    if (rc != MAD_OK) return rc;
     if (hi->max_entry > 255 || lo->max_entry > 255) {
         mad_set_error("mad_match_pairs: descriptor entries up to %d do not fit the uint8 tensor-core operand "
-                      "(use mad_match_count/mad_match_fill with impl = 2, the fp16 kernel)",
+                      "(use mad_match_count/mad_match_fill with impl = 2 or 1)",
                       hi->max_entry > lo->max_entry ? hi->max_entry : lo->max_entry);
         return MAD_ERR_ARG;
     }

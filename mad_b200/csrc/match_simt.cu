@@ -127,13 +127,18 @@ __global__ void topk_merge_kernel(const int32_t* __restrict__ idx_in, const doub
     double bs[MAD_TOPK_MAX];
     int bi[MAD_TOPK_MAX];
     for (int q = 0; q < MAD_TOPK_MAX; ++q) { bs[q] = -INFINITY; bi[q] = -1; }
+    bool incomplete = false;                    // an input list of this row is incomplete (-2): so is the merged one
     for (int g = 0; g < G; ++g)
         for (int q = 0; q < k; ++q) {
             const long long p = ((long long)g * M + row) * k + q;
             const int id = idx_in[p];
             if (id >= 0) mad_topk_insert(bs, bi, k, score_in[p], id);
+            incomplete |= id == MAD_TOPK_INCOMPLETE;
         }
-    for (int q = 0; q < k; ++q) { idx_out[(long long)row * k + q] = bi[q]; score_out[(long long)row * k + q] = bs[q]; }
+    for (int q = 0; q < k; ++q) {
+        idx_out[(long long)row * k + q] = incomplete ? MAD_TOPK_INCOMPLETE : bi[q];
+        score_out[(long long)row * k + q] = incomplete ? -INFINITY : bs[q];
+    }
 }
 
 struct CastI64 {

@@ -2,7 +2,8 @@
 //
 // Replaces  preds = np.dot(hi_unit, lo_unit.T); np.where(preds > cc)  (mad/MaD.py:416-424).
 // Descriptor entries are small non-negative integers, so the raw dot product is computed EXACTLY
-// by one fp16 x fp16 -> fp32 UMMA pass (products <= 2^22, sums < 2^24); the cosine
+// by one fp16 x fp16 -> fp32 UMMA pass while entries are <= 2048 (products <= 2^22) and every dot product
+// is <= 2^24 -- guaranteed by max |hi|^2 * max |lo|^2 <= 2^48, which the dispatch checks; the cosine
 // dot / sqrt(n_i n_j) is then evaluated in float64 from exact integers, only for the pairs an
 // fp32 pre-filter cannot rule out.  The M x N score matrix is never written.
 //

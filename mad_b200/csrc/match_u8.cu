@@ -23,8 +23,8 @@
 //        PAIRS mode: hits (row, col, dot) are staged per warp in shared memory and appended to a
 //                    global candidate list by the drain warps (one atomicAdd per half buffer); a radix sort by
 //                    (row, col) afterwards restores np.where's row-major order (match_finish).
-//        TOPK mode : per-row running top-k in the thread (k <= 8: a register list keyed by the exact integer ratio
-//                    dot^2 / |lo|^2), one partial list per (lo segment, epilogue group), thresholds of the two groups
+//        TOPK mode : per-row running top-k in the thread (k <= 8: a register list keyed by float32 score images, near-ties
+//                    decided on the float64 score), one partial list per (lo segment, epilogue group), thresholds of the two groups
 //                    shared through shared memory.
 #include <cuda.h>
 #include <stdlib.h>
@@ -429,7 +429,7 @@ match_u8_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
     } else if ((warp == 2 || warp == 3 || warp >= 4 + EPI_WARPS) && MODE == MODE_TOP8) {
         // ===================== drain warps (TOP8): warps 2, 3, 12, 13 own the lists of one 32-row quadrant each ==========
         // Lane l keeps the top-8 list of row 32 dq + l in registers: (float32 score image, dot, |lo|^2, index), ordered by the
-        // exact integer ratio dot^2 / |lo|^2 wherever the images are closer than 4e-6.  The epilogue warps of BOTH groups stage
+        // float64 score and then the index wherever the images are closer than 4e-6.  The epilogue warps of BOTH groups stage
         // their candidates per lane (lane l of an epilogue warp of quadrant q owns row 32 q + l), so a published half is
         // consumed by all 32 lanes at once: every lane inserts its own row's (at most TOP_SLOTS) entries -- no routing, no
         // atomics, one list per row for both column halves of a tile.
@@ -477,7 +477,7 @@ match_u8_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
                         // stale candidates (staged under an older threshold) are dropped on the image of the 8th entry
                         const bool live = has && (bi[7] < 0 || s32 >= ts[7] * (1.f - 4e-6f));
                         if (!__any_sync(0xFFFFFFFFu, live)) { n_stale += has; continue; }
-                        mad_top8f_insert(ts, td, tn, bi, live, s32, nz ? dot : 0, nz ? n2b : 1, id);
+                        mad_top8f_insert(ts, td, tn, bi, live, s32, nz ? dot : 0, nz ? n2b : 1, id, (double)n2a_i);
                         changed |= live;
                         n_ins += live;
                         n_stale += has && !live;
@@ -508,7 +508,7 @@ match_u8_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
 #pragma unroll
             for (int i = 0; i < 8; ++i)
                 if (i < a.k) {
-                    a.topk_idx[o + i] = timeout ? -2 : bi[i];
+                    a.topk_idx[o + i] = timeout ? MAD_TOPK_INCOMPLETE : bi[i];
                     a.topk_score[o + i] = bi[i] < 0 ? -INFINITY : (td[i] == 0 ? 0.0 : mad_score(td[i], (double)n2a_i, (double)tn[i]));
                 }
         }
@@ -522,8 +522,9 @@ match_u8_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
         const int n2a_i = row_ok ? a.hi_n2[row] : 0;
         const double n2a = (double)n2a_i;
         const float ra = n2a_i > 0 ? (float)(1.0 / sqrt(n2a)) : 0.f;
-        // fp32 pre-filter: dot * rb > (cc - 4e-6) / ra   (|approx - exact| < 1e-6); never for zero rows
-        const float thr_pairs = (row_ok && n2a_i > 0) ? ((float)a.cc - 4e-6f) / ra : INFINITY;
+        // fp32 pre-filter: dot * rb > (cc - 4e-6) / ra   (|approx - exact| < 1e-6).  A zero row scores 0 against every
+        // column: all of them pass when cc < 0, none otherwise.
+        const float thr_pairs = !row_ok ? INFINITY : (n2a_i > 0 ? ((float)a.cc - 4e-6f) / ra : (a.cc < 0.0 ? -INFINITY : INFINITY));
         unsigned long long* my_key = stg_key + ew * STG;
         int* my_dot = stg_dot + ew * STG;
         constexpr bool kTop = (MODE == MODE_TOPK || MODE == MODE_TOP8);
@@ -686,7 +687,7 @@ match_u8_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constan
                             const float s32 = nz ? (float)dot * rbt[c0 + j] * ra : 0.f;
                             const bool live = has && (li[7] < 0 || s32 >= ls[7] * (1.f - 4e-6f));
                             if (__any_sync(0xFFFFFFFFu, live))
-                                mad_top8f_insert(ls, ld, ln, li, live, s32, nz ? dot : 0, nz ? n2b : 1, a.lo_index_base + n0 + c0 + j);
+                                mad_top8f_insert(ls, ld, ln, li, live, s32, nz ? dot : 0, nz ? n2b : 1, a.lo_index_base + n0 + c0 + j, n2a);
                         }
                         continue;
                     }

@@ -231,6 +231,9 @@ def match_topk_grid(hi_block_set, lo_shard_set, k, m_total, grid, group=None, im
             mi, ms = P.topk_merge(idx_g, sc_g)
         else:
             mi, ms = _merge_lists_host(idx_g, sc_g)
+            if bool((mi == -2).any()):                        # the lists are on the host already: checking costs nothing
+                from ._lib import MadError
+                raise MadError("match_topk_grid: a shard's top-k list is incomplete (kernel hand-off time-out)")
     else:
         mi, ms = idx_g.view(gh * rows_max, k), sc_g.view(gh * rows_max, k)
     if m_total % gh:                                          # drop the padding rows of the shorter blocks
@@ -240,7 +243,8 @@ def match_topk_grid(hi_block_set, lo_shard_set, k, m_total, grid, group=None, im
 
 
 def _merge_lists_host(idx_g, sc_g):
-    """(score desc, index asc) k-way merge of [G, M, k] lists on CPU tensors (gloo tests; the GPU path uses mad_topk_merge)."""
+    """(score desc, index asc) k-way merge of [G, M, k] lists on CPU tensors (gloo tests; the GPU path uses mad_topk_merge).
+    Index -1 is padding; a row with a -2 (incomplete list) in any input comes out as all -2 / -inf, as mad_topk_merge does."""
     g, m, k = idx_g.shape
     idx = idx_g.permute(1, 0, 2).reshape(m, g * k)
     sc = sc_g.permute(1, 0, 2).reshape(m, g * k)
@@ -249,7 +253,9 @@ def _merge_lists_host(idx_g, sc_g):
     order = torch.argsort(key_i, dim=1, stable=True)          # index asc first, then a STABLE sort by score desc
     sc1, idx1 = torch.gather(sc, 1, order), torch.gather(idx, 1, order)
     order2 = torch.argsort(-sc1, dim=1, stable=True)[:, :k]
-    return torch.gather(idx1, 1, order2), torch.gather(sc1, 1, order2)
+    mi, ms = torch.gather(idx1, 1, order2), torch.gather(sc1, 1, order2)
+    bad = (idx == -2).any(dim=1, keepdim=True)
+    return torch.where(bad, torch.full_like(mi, -2), mi), torch.where(bad, torch.full_like(ms, float("-inf")), ms)
 
 
 def match_topk_grid_sets(hi_block_set, lo_shard_set, k, m_total, lo_index_base, grid, group=None, impl=None):

@@ -425,11 +425,12 @@ class DescriptorSet(object):
         self.norm2 = torch.empty(max(self.rows, 1), dtype=torch.int32, device=dev)
         self.rnorm = torch.empty(self.rows_padded, dtype=torch.float32, device=dev)
         self.u8 = torch.empty((self.rows_padded, DSC_LEN), dtype=torch.uint8, device=dev)
-        mx = torch.zeros(1, dtype=torch.int32, device=dev)
+        mx = torch.zeros(2, dtype=torch.int32, device=dev)           # largest entry, largest squared norm
         call("mad_dsc_prepare", _ptr(self.dsc), self.rows, self.rows_padded, _ptr(self.norm2), _ptr(self.rnorm),
-             _ptr(self.u8), _ptr(mx), st)
+             _ptr(self.u8), _ptr(mx), _ptr(mx[1:]), st)
         self._max_dev = mx
         self._max_entry = None
+        self._max_norm2 = None
         self.half = None
         s = _lib.MadDscSet()
         s.dsc = self.dsc.data_ptr()
@@ -439,17 +440,21 @@ class DescriptorSet(object):
         s.rnorm = self.rnorm.data_ptr()
         s.rows, s.rows_padded = self.rows, self.rows_padded
         s.max_entry = -1
+        s.max_norm2 = -1
         self.c = s
         if need_half:
             self.ensure_half()
 
     @property
     def max_entry(self):
-        """Largest descriptor entry (one device->host read, cached)."""
+        """Largest descriptor entry (one device->host read, cached); DSC_REFUSED if the set is not a descriptor set."""
         if self._max_entry is None:
-            self._max_entry = int(self._max_dev.item())
-            self.c.max_entry = self._max_entry
+            self._set_maxima(*self._max_dev.tolist())
         return self._max_entry
+
+    def _set_maxima(self, max_entry, max_norm2):
+        self._max_entry, self._max_norm2 = int(max_entry), int(max_norm2)
+        self.c.max_entry, self.c.max_norm2 = self._max_entry, self._max_norm2
 
     def ensure_half(self):
         if self.half is None:
@@ -463,9 +468,26 @@ def _as_set(x):
     return x if isinstance(x, DescriptorSet) else DescriptorSet(x)
 
 
+def _check_descriptors(hi, lo):
+    if max(hi._max_entry, lo._max_entry) >= _lib.DSC_REFUSED:
+        raise _lib.MadError("mad_match: not a descriptor set (a negative entry, or a squared norm >= 2^31)")
+
+
+def _exact_impl(hi, lo):
+    """Product choice for sets whose maxima are known: the uint8 kernel while every entry is <= 255; else the fp16 kernel
+    where its fp32 sums are exact (entries <= 2048 and max |hi|^2 max |lo|^2 <= 2^48, so every dot product is <= 2^24),
+    else the SIMT kernel (exact in int32)."""
+    _check_descriptors(hi, lo)
+    if max(hi._max_entry, lo._max_entry) <= 255:
+        return 0
+    if max(hi._max_entry, lo._max_entry) <= 2048 and hi._max_norm2 * lo._max_norm2 <= 1 << 48:
+        return 2
+    return 1
+
+
 def _pick_impl(hi, lo, impl):
-    """impl None = product choice: the uint8 tcgen05 kernel, or the fp16 one if an entry exceeds 255.
-    Returns (impl, verify).  When the largest entry of a set has not been read back yet, the uint8
+    """impl None = product choice (``_exact_impl``): the uint8 tcgen05 kernel, or, if an entry exceeds 255, a kernel that
+    is exact for the set.  Returns (impl, verify).  When the largest entry of a set has not been read back yet, the uint8
     kernel runs optimistically and the check is folded into the read-back the call makes anyway
     (verify = True): a separate 4-byte device-to-host read here would queue behind any large
     copy-out in flight on another stream and stall the matching kernel for its whole duration."""
@@ -473,13 +495,12 @@ def _pick_impl(hi, lo, impl):
     if impl is None:
         if hi._max_entry is None or lo._max_entry is None:
             return 0, True
-        impl = 0 if max(hi._max_entry, lo._max_entry) <= 255 else 2
+        impl = _exact_impl(hi, lo)
     return _pick_impl_explicit(hi, lo, impl), verify
 
 
 def _pick_impl_explicit(hi, lo, impl):
-    if impl == 0:
-        hi.max_entry, lo.max_entry          # noqa: B018  (fills the C structs)
+    hi.max_entry, lo.max_entry              # noqa: B018  (fills the C structs: the library checks the sets' maxima)
     if impl == 2:
         hi.ensure_half()
         lo.ensure_half()
@@ -542,10 +563,10 @@ def match_threshold(hi, lo, cc=0.6, impl=None, want="score"):
 
 
 def _read_counts(count, hi, lo):
-    """One device->host read: (pairs found, largest entry of hi, of lo); caches the maxima."""
+    """One device->host read: (pairs found, largest entry and squared norm of hi, of lo); caches the maxima."""
     vals = _Readback.read(count, hi._max_dev, lo._max_dev)
-    hi._max_entry, lo._max_entry = int(vals[1]), int(vals[2])
-    hi.c.max_entry, lo.c.max_entry = hi._max_entry, lo._max_entry
+    hi._set_maxima(vals[1], vals[2])
+    lo._set_maxima(vals[3], vals[4])
     return int(vals[0])
 
 
@@ -561,10 +582,10 @@ def _match_threshold_onepass(hi, lo, cc, dev, st, verify=False, want="score"):
         p = _read_counts(count, hi, lo)
         if p >= (1 << 62):
             raise _lib.MadError("mad_match_pairs: the kernel's internal hand-off timed out (pair list incomplete)")
-        if verify and max(hi._max_entry, lo._max_entry) > 255:
+        if verify and _exact_impl(hi, lo) != 0:
             if want != "score":
-                raise _lib.MadError("match_threshold: entries above 255 need the fp16 kernel, which has no want='dot' form")
-            return match_threshold(hi, lo, cc, impl=2)      # entries above 255: the fp16 tensor-core kernel
+                raise _lib.MadError("match_threshold: entries above 255 need the fp16 or SIMT kernel, which have no want='dot' form")
+            return match_threshold(hi, lo, cc)              # entries above 255: the kernel that is exact for the sets
         if p <= cap:
             break
         cap = p + p // 8 + 1024            # the candidate list overflowed: repeat with room
@@ -789,7 +810,7 @@ class MapBatch(object):
                     r.update(kp=st.fetch("kp%d" % j, kp.table[:len(kp)]), ori=st.fetch("ori%d" % j, ori.table[:len(ori)]))
                     if self.compact:
                         ds = DescriptorSet(dsc)
-                        r["_max"] = ds._max_dev
+                        r["_max"] = ds._max_dev[:1]
                         r["dsc_u8"] = st.fetch("dsc8_%d" % j, ds.u8[:ds.rows])
                         r["_dsc_dev"] = dsc
                     else:
@@ -842,8 +863,8 @@ def match_topk(hi, lo, k=8, lo_index_base=0, impl=None):
          ws_bytes, impl, st)
     if verify:
         _read_counts(torch.zeros(1, dtype=torch.int64, device=dev), hi, lo)
-        if max(hi._max_entry, lo._max_entry) > 255:
-            return match_topk(hi, lo, k, lo_index_base, impl=2)
+        if _exact_impl(hi, lo) != 0:
+            return match_topk(hi, lo, k, lo_index_base)
     return idx, score
 
 

@@ -36,7 +36,7 @@ def test_struct_layouts_match_the_header(lib):
     assert lib.KEYPOINT_DTYPE.itemsize == 48          # MadKeypoint
     assert lib.ORIENTED_DTYPE.itemsize == 8           # MadOriented
     assert C.sizeof(lib.MadZoneTable) == 40
-    assert C.sizeof(lib.MadDscSet) == 56          # 5 pointers + 3 int32 (+4 padding)
+    assert C.sizeof(lib.MadDscSet) == 56          # 5 pointers + 4 int32
 
 
 def test_bad_arguments_are_rejected_without_touching_the_device(lib):
