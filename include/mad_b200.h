@@ -306,6 +306,40 @@ int mad_repeatability(const int32_t* pair_hi, const int32_t* pair_lo, const doub
                       const double* hi_cloud, int n_hi_cloud, const double* lo_sorted, const int32_t* cell_start,
                       const uint32_t* near_bits, const double* grid_org_host, const int* grid_dims_host,
                       double dist, double* results, void* stream);
+/* mad_repeatability in two parts, so that the pairs can be shared out (mad_b200.parallel.match_dsc_sharded):
+ * mad_repeat_counts writes counts[p - p0] = #{q with a lo-cloud point closer than dist} for the pairs p in [p0, p1)
+ * (mad/MaD.py:430-448, the cKDTree query per pair); mad_repeat_rows writes results[p][23] for all n_pairs pairs from
+ * those counts with mad_repeatability's formulas (mad/MaD.py:449-451: repeatability = 100 * count / n_hi_cloud).
+ * The arguments mean what they mean for mad_repeatability; counts + rows == mad_repeatability, bit for bit. */
+int mad_repeat_counts(const int32_t* pair_hi, const int32_t* pair_lo, long long p0, long long p1,
+                      const double* hi_subv, const double* lo_subv, const int32_t* hi_meta, const int32_t* lo_meta,
+                      const double* rf_table, const double* rf_inv_table, int rf_zones,
+                      const double* hi_cloud, int n_hi_cloud, const double* lo_sorted, const int32_t* cell_start,
+                      const uint32_t* near_bits, const double* grid_org_host, const int* grid_dims_host,
+                      double dist, int32_t* counts, void* stream);
+int mad_repeat_rows(const int32_t* pair_hi, const int32_t* pair_lo, const double* pair_score, long long n_pairs,
+                    const double* hi_subv, const double* lo_subv, const int32_t* hi_meta, const int32_t* lo_meta,
+                    const double* rf_table, const double* rf_inv_table, int rf_zones, const int32_t* counts,
+                    int n_hi_cloud, double* results, void* stream);
+
+/* The anchor clouds and the lo grid of the repeatability loop, on the device (mad/MaD.py:427-428 and the grid above).
+ * mad_anchor_cloud: cloud[0..n) = np.unique(subv[used], axis=0) -- the distinct rows of subv [n_rows][3] whose used flag
+ * is set, in lexicographic (x, y, z) order, bit for bit (-0.0 is taken as +0.0, as NumPy compares them equal);
+ * cloud has room for n_rows rows.  info (device int64[8], written by the call): [0] n, [1] number of used rows with a
+ * non-finite coordinate (the caller must refuse the set: the cloud is then meaningless), [2..4] grid dims =
+ * floor((max - org) / cell) + 2 (clamped to 2^40), [5..7] the bits of grid_org (device double[3]) = min - cell, all in
+ * float64 as NumPy evaluates them.  Read info back once and pass dims / org to the calls below.
+ * mad_cloud_grid: for the cloud of n rows (n >= 1), sorted [n][3] = the cloud stably sorted by cell id
+ * (np.argsort(kind="stable")), cell_start [ncell + 1] = points in lower cells, near_bits [ceil(ncell / 32)] = cells whose
+ * 27-cell neighbourhood (clipped to the grid) holds a point.  ncell = dims0 dims1 dims2 must be < 2^31 (MAD_ERR_ARG
+ * otherwise: the repeatability kernel indexes cells in int32). */
+size_t mad_anchor_cloud_workspace_bytes(int n_rows);
+int mad_anchor_cloud(const double* subv, const uint8_t* used, int n_rows, double cell, double* cloud, double* grid_org,
+                     long long* info, void* workspace, size_t workspace_bytes, void* stream);
+size_t mad_cloud_grid_workspace_bytes(int n);
+int mad_cloud_grid(const double* cloud, int n, const double* grid_org, const long long* grid_dims_host, double cell,
+                   double* sorted, int32_t* cell_start, uint32_t* near_bits, void* workspace, size_t workspace_bytes,
+                   void* stream);
 
 /* ---- next component (SURVEY.md 8f rank 2): atoms -> density, mad/PDB.py:131-163,215-292 -------------------- */
 /* Mass-weighted trilinear splat of n_atoms points (xyz [n][3], mass [n], float64) into grid [px][py][pz] float64

@@ -105,6 +105,13 @@ SIGNATURES = {
     "mad_mark_used": (_I, [_P, C.c_longlong, _P, _P]),
     "mad_repeatability": (_I, [_P, _P, _P, C.c_longlong, _P, _P, _P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _P, _P,
                                C.c_double, _P, _P]),
+    "mad_repeat_counts": (_I, [_P, _P, C.c_longlong, C.c_longlong, _P, _P, _P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _P, _P,
+                               C.c_double, _P, _P]),
+    "mad_repeat_rows": (_I, [_P, _P, _P, C.c_longlong, _P, _P, _P, _P, _P, _P, _I, _P, _I, _P, _P]),
+    "mad_anchor_cloud_workspace_bytes": (_SZ, [_I]),
+    "mad_anchor_cloud": (_I, [_P, _P, _I, C.c_double, _P, _P, _P, _P, _SZ, _P]),
+    "mad_cloud_grid_workspace_bytes": (_SZ, [_I]),
+    "mad_cloud_grid": (_I, [_P, _I, _P, _P, C.c_double, _P, _P, _P, _P, _SZ, _P]),
     "mad_box_scores_workspace_bytes": (_SZ, [_I, _I, _I]),
     "mad_box_scores": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, C.c_float, _P, _P, _SZ, _P]),
     "mad_grid_count_gt": (_I, [_P, C.c_longlong, C.c_float, _P, _P]),

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libmad_b200.so")
-SOURCES = ["dmap.cu", "density.cu", "scale_space.cu", "detect.cu", "orient.cu", "describe.cu", "match_simt.cu", "match_tc.cu", "match_u8.cu", "match_prep.cu", "repeat.cu", "score.cu", "api.cu"]
+SOURCES = ["dmap.cu", "density.cu", "scale_space.cu", "detect.cu", "orient.cu", "describe.cu", "match_simt.cu", "match_tc.cu", "match_u8.cu", "match_prep.cu", "repeat.cu", "cloud.cu", "score.cu", "api.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

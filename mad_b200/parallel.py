@@ -9,6 +9,9 @@
   a result bit-identical to one GPU.  Threshold mode (the parity contract, ``MaD.py:423-424``): every rank lists its
   pairs with GLOBAL lo indices; pair counts are all-gathered, the lists travel in one padded all-gather and are merged
   in (hi, lo) order -- the row-major order of ``np.where`` on the whole score matrix.
+* ``MaD._match_dsc`` (``MaD.py:414-453``): the threshold matching and the anchor clouds are replicated (cheap next to the
+  per-pair repeatability); the pairs are cut into G contiguous shares, every rank counts the hits of its share, one
+  all_gather of the int32 counts and the row expansion on every rank give the 1-GPU table.
 """
 import torch
 import torch.distributed as dist
@@ -264,3 +267,81 @@ def match_topk_grid_sets(hi_block_set, lo_shard_set, k, m_total, lo_index_base, 
     from . import pipeline as P
     idx, sc = P.match_topk(hi_block_set, lo_shard_set, k, lo_index_base=lo_index_base, impl=impl)
     return match_topk_grid(hi_block_set, lo_shard_set, k, m_total, grid, group=group, impl=impl, local=(idx, sc))
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# MaD._match_dsc with the per-pair repeatability shared out over the ranks
+# ---------------------------------------------------------------------------------------------------------------------
+def pad_counts(local, n_pairs, world):
+    """This rank's counts (its share of ``shard_bounds(n_pairs, world)``) padded to the longest share, the first."""
+    per = shard_bounds(n_pairs, world)[0][1]
+    out = torch.zeros(per, dtype=torch.int32, device=local.device)
+    out[:local.numel()] = local
+    return out
+
+
+def join_counts(gathered, n_pairs):
+    """[G, per] padded shares in rank order -> the counts of all ``n_pairs`` pairs."""
+    g = gathered.shape[0]
+    return torch.cat([gathered[r, :e - s] for r, (s, e) in enumerate(shard_bounds(n_pairs, g))])
+
+
+def check_same_problem(rows_hi, rows_lo, n_pairs, device, group=None):
+    """One all_reduce (max of (x, -x)): raises MadError on every rank if the ranks do not hold the same sets and pair
+    count, where a gather of differently sized shares would hang."""
+    t = torch.tensor([rows_hi, rows_lo, n_pairs], dtype=torch.int64, device=device)
+    both = torch.cat([t, -t])
+    dist.all_reduce(both, op=dist.ReduceOp.MAX, group=group)
+    hi_, lo_ = both[:3].tolist(), [-v for v in both[3:].tolist()]
+    if hi_ != lo_:
+        from ._lib import MadError
+        raise MadError("match_dsc_sharded: the ranks disagree on (hi rows, lo rows, pairs): from %r to %r" % (lo_, hi_))
+
+
+def gather_pair_counts(local, n_pairs, rows_hi, rows_lo, group=None):
+    """The counts of all ``n_pairs`` pairs on every rank from each rank's share (``shard_bounds(n_pairs, G)[rank]``):
+    the consistency check, then ONE all_gather of the shares padded to equal size (``all_gather_into_tensor``, or the list
+    form on a backend without it).  No collective at all for n_pairs == 0, so the check cannot catch one rank with no
+    pairs while another has some: the ranks with pairs then wait in the check's all_reduce until the backend's time-out."""
+    g = _world(group)
+    if g == 1 or n_pairs == 0:
+        return local
+    check_same_problem(rows_hi, rows_lo, n_pairs, local.device, group)
+    pad = pad_counts(local, n_pairs, g)
+    out = torch.empty((g, pad.numel()), dtype=torch.int32, device=local.device)
+    try:
+        dist.all_gather_into_tensor(out, pad, group=group)
+    except (RuntimeError, NotImplementedError):             # a backend without the tensor form
+        dist.all_gather(list(out.unbind(0)), pad, group=group)
+    return join_counts(out, n_pairs)
+
+
+def match_dsc_local(m, rank, world):
+    """This rank's step of ``match_dsc_sharded`` on a ``pipeline.DscMatch``: the counts of its share of the pairs."""
+    s, e = shard_bounds(m.p, world)[rank]
+    return m.counts(s, e)
+
+
+def match_dsc_sharded(lo, hi, anchor_dist_thresh=4, cc_threshold=0.65, group=None, impl=None):
+    """``pipeline.match_dsc`` with the per-pair repeatability shared out over the ranks of ``group``.  Every rank holds
+    both FeatureTables and computes the same pair list and anchor clouds (threshold matching is replicated, not sharded:
+    it is cheap next to the per-pair loop); rank r counts the hits of its contiguous share of the pairs
+    (``shard_bounds(P, G)[r]``, equal work per pair), the counts are all-gathered and every rank expands all P rows.
+    Every rank returns what ``pipeline.match_dsc`` returns on one GPU, bit for bit."""
+    from . import pipeline as P
+    m = P.DscMatch(lo, hi, anchor_dist_thresh, cc_threshold, impl)
+    if m.p == 0:
+        return m.result(m.empty())
+    g = _world(group)
+    rank = dist.get_rank(group) if g > 1 else 0
+    counts = gather_pair_counts(match_dsc_local(m, rank, g), m.p, hi.set.rows, lo.set.rows, group)
+    return m.result(m.rows(counts))
+
+
+def match_dsc_lists_sharded(lo_dsc_list, hi_dsc_list, anchor_dist_thresh=4, cc_threshold=0.65, group=None):
+    """Drop-in for ``MaD._match_dsc`` under torchrun (INTEGRATION.md): the arguments and return value of
+    ``pipeline.match_dsc_lists``, computed by ``match_dsc_sharded``."""
+    from . import pipeline as P
+    res, lo_cloud, hi_cloud = match_dsc_sharded(P.FeatureTable.from_features(lo_dsc_list), P.FeatureTable.from_features(hi_dsc_list),
+                                                anchor_dist_thresh, cc_threshold, group=group)
+    return list(res.cpu().numpy()), lo_cloud, hi_cloud

@@ -904,58 +904,150 @@ class FeatureTable(object):
                    [df.sec_bin for df in df_list], np.array([df.subv_map_coords for df in df_list], dtype=np.float64))
 
 
-def _cloud_grid(cloud, cell):
-    """Uniform grid (cell size = the distance threshold) over the lo cloud: cell-sorted points, cell_start,
-    and the bitmap of cells whose 27-cell neighbourhood holds a point.  Host glue (a few thousand points)."""
-    org = cloud.min(0) - cell
-    dims = (np.floor((cloud.max(0) - org) / cell).astype(np.int64) + 2)
-    cidx = np.floor((cloud - org) / cell).astype(np.int64)
-    lin = (cidx[:, 0] * dims[1] + cidx[:, 1]) * dims[2] + cidx[:, 2]
-    order = np.argsort(lin, kind="stable")
-    ncell = int(dims.prod())
-    cell_start = np.zeros(ncell + 1, dtype=np.int32)
-    np.cumsum(np.bincount(lin, minlength=ncell), out=cell_start[1:])
-    occ = np.zeros(tuple(dims), dtype=bool)
-    occ[cidx[:, 0], cidx[:, 1], cidx[:, 2]] = True
-    near = np.zeros_like(occ)
-    p = np.pad(occ, 1)
-    for dx in range(3):
-        for dy in range(3):
-            for dz in range(3):
-                near |= p[dx:dx + dims[0], dy:dy + dims[1], dz:dz + dims[2]]
-    bits = np.packbits(near.reshape(-1), bitorder="little")
-    bits = np.concatenate([bits, np.zeros((-len(bits)) % 4, dtype=np.uint8)]).view(np.uint32)
-    return np.ascontiguousarray(cloud[order]), cell_start, bits, org.astype(np.float64), dims.astype(np.int32)
+class AnchorCloud(object):
+    """np.unique(subv[used], axis=0) built on the device (``mad_anchor_cloud``) and, for the lo side, the uniform grid of
+    cell size ``cell`` the repeatability kernel searches (``mad_cloud_grid``): the cell-sorted cloud, cell_start and the
+    27-neighbourhood bitmap.  ``org`` float64 [3] / ``dims`` int32 [3] are host copies."""
+
+    def __init__(self, subv, used, cell):
+        dev = subv.device
+        st = _stream()
+        d = int(subv.shape[0])
+        self.cell = float(cell)
+        self._buf = torch.empty((max(d, 1), 3), dtype=torch.float64, device=dev)
+        self.org_dev = torch.empty(3, dtype=torch.float64, device=dev)
+        self.info = torch.empty(8, dtype=torch.int64, device=dev)
+        ws_bytes = _lib.lib.mad_anchor_cloud_workspace_bytes(d)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        call("mad_anchor_cloud", _ptr(subv), _ptr(used), d, C.c_double(self.cell), _ptr(self._buf), _ptr(self.org_dev),
+             _ptr(self.info), _ptr(ws), ws_bytes, st)
+        self.n = None
+
+    def take_info(self, vals):
+        """The eight values of ``info`` read back (see ``read_clouds``); refuses a cloud with a non-finite coordinate."""
+        n, bad = int(vals[0]), int(vals[1])
+        if bad:
+            raise _lib.MadError("anchor cloud: %d used feature(s) with a non-finite coordinate" % bad)
+        self.n = n
+        self.dims64 = np.array(vals[2:5], dtype=np.int64)
+        self.org = np.array(vals[5:8], dtype=np.int64).view(np.float64)
+        self.dims = self.dims64.astype(np.int32)
+        self.cloud = self._buf[:n]
+        return self
+
+    def build_grid(self):
+        """mad_cloud_grid: lo_sorted, cell_start, near_bits (refused with MadError for a grid of >= 2^31 cells)."""
+        dev = self._buf.device
+        ncell = int(np.prod([int(v) for v in self.dims64], dtype=object))
+        fits = ncell < (1 << 31)
+        self.sorted = torch.empty((max(self.n, 1), 3), dtype=torch.float64, device=dev)
+        self.cell_start = torch.empty(ncell + 1 if fits else 1, dtype=torch.int32, device=dev)
+        self.near_bits = torch.zeros((ncell + 31) // 32 if fits else 1, dtype=torch.int32, device=dev)
+        ws_bytes = _lib.lib.mad_cloud_grid_workspace_bytes(self.n)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        call("mad_cloud_grid", _ptr(self.cloud), self.n, _ptr(self.org_dev), _dptr(self.dims64), C.c_double(self.cell),
+             _ptr(self.sorted), _ptr(self.cell_start) if fits else None, _ptr(self.near_bits) if fits else None, _ptr(ws),
+             ws_bytes, _stream())
+        self.sorted = self.sorted[:self.n]
+        return self
+
+    def host(self):
+        return self.cloud.cpu().numpy()
+
+
+def read_clouds(*clouds):
+    """One device -> host read of the (n, status, dims, org) of several AnchorClouds."""
+    vals = _Readback.read(*[c.info for c in clouds])
+    return [c.take_info(vals[8 * i:8 * i + 8]) for i, c in enumerate(clouds)]
+
+
+def anchor_cloud(subv, used, cell):
+    """One AnchorCloud with its grid: ``subv`` float64 [D, 3] and ``used`` uint8 [D] device tensors."""
+    c, = read_clouds(AnchorCloud(subv.contiguous(), used.contiguous(), cell))
+    return c.build_grid()
+
+
+class DscMatch(object):
+    """What ``match_dsc`` computes before the per-pair loop, and what every rank of ``parallel.match_dsc_sharded`` computes
+    alike: the pair list above cc (hi, lo, score device tensors, ``p`` pairs), the hi anchor cloud and the lo anchor cloud
+    with its grid (AnchorCloud)."""
+
+    def __init__(self, lo, hi, anchor_dist_thresh=4, cc_threshold=0.65, impl=None, pairs=None):
+        """pairs: the (hi, lo, score) list of ``match_threshold(hi.set, lo.set, cc_threshold)`` if already computed."""
+        self.lo, self.hi = lo, hi
+        self.dist = float(anchor_dist_thresh)
+        dev = hi.set.dsc.device
+        if pairs is None:
+            pairs = match_threshold(hi.set, lo.set, cc_threshold, impl=impl)
+        self.ph, self.pl, self.sc = pairs
+        self.p = int(self.ph.numel())
+        self.hi_cloud = self.lo_cloud = None
+        if self.p == 0:
+            return
+        st = _stream()
+        used_hi = torch.zeros(hi.set.rows, dtype=torch.uint8, device=dev)
+        used_lo = torch.zeros(lo.set.rows, dtype=torch.uint8, device=dev)
+        call("mad_mark_used", _ptr(self.ph), self.p, _ptr(used_hi), st)
+        call("mad_mark_used", _ptr(self.pl), self.p, _ptr(used_lo), st)
+        self.hi_cloud, self.lo_cloud = read_clouds(AnchorCloud(hi.subv, used_hi, self.dist),       # mad/MaD.py:427
+                                                   AnchorCloud(lo.subv, used_lo, self.dist))       # mad/MaD.py:428
+        self.lo_cloud.build_grid()
+        self.tb = device_tables(dev)
+
+    def _common(self):
+        return (_ptr(self.hi.subv), _ptr(self.lo.subv), _ptr(self.hi.meta), _ptr(self.lo.meta), _ptr(self.tb.rf),
+                _ptr(self.tb.rf_inv), self.tb.ori_zones)
+
+    def _grid(self):
+        g = self.lo_cloud
+        return (_ptr(self.hi_cloud.cloud), self.hi_cloud.n, _ptr(g.sorted), _ptr(g.cell_start), _ptr(g.near_bits), _dptr(g.org),
+                _dptr(g.dims), C.c_double(self.dist))
+
+    def counts(self, p0, p1):
+        """int32 [p1 - p0]: hits of the pairs [p0, p1) (mad_repeat_counts)."""
+        out = torch.empty(max(p1 - p0, 1), dtype=torch.int32, device=self.ph.device)
+        if p1 > p0:
+            call("mad_repeat_counts", _ptr(self.ph), _ptr(self.pl), int(p0), int(p1), *self._common(), *self._grid(), _ptr(out),
+                 _stream())
+        return out[:p1 - p0]
+
+    def rows(self, counts):
+        """float64 [P, 23] result table from the hits of all P pairs (mad_repeat_rows)."""
+        if counts.numel() != self.p or counts.dtype != torch.int32 or counts.device != self.ph.device:
+            raise _lib.MadError("DscMatch.rows: needs int32 counts of all %d pairs on %s, got %s [%d] on %s"
+                                % (self.p, self.ph.device, counts.dtype, counts.numel(), counts.device))
+        res = torch.empty((self.p, 23), dtype=torch.float64, device=self.ph.device)
+        call("mad_repeat_rows", _ptr(self.ph), _ptr(self.pl), _ptr(self.sc), self.p, *self._common(), _ptr(counts.contiguous()),
+             self.hi_cloud.n, _ptr(res), _stream())
+        return res
+
+    def table(self):
+        """float64 [P, 23] in one call (mad_repeatability: counts + rows without a counts buffer)."""
+        res = torch.empty((self.p, 23), dtype=torch.float64, device=self.ph.device)
+        call("mad_repeatability", _ptr(self.ph), _ptr(self.pl), _ptr(self.sc), self.p, *self._common(), *self._grid(), _ptr(res),
+             _stream())
+        return res
+
+    def result(self, table):
+        """(table, lo_mapcoords, hi_mapcoords as NumPy arrays): ``match_dsc``'s return value."""
+        if self.p == 0:
+            return table, np.zeros((0, 3)), np.zeros((0, 3))
+        return table, self.lo_cloud.host(), self.hi_cloud.host()
+
+    def empty(self):
+        return torch.empty((0, 23), dtype=torch.float64, device=self.ph.device)
 
 
 def match_dsc(lo, hi, anchor_dist_thresh=4, cc_threshold=0.65, impl=None):
     """``MaD._match_dsc`` (mad/MaD.py:414-453) on the device: cosine matching above ``cc_threshold`` and, per pair, the
     rigid transform R = inv(Rfinal_lo) . Rfinal_hi and the repeatability of the matched hi anchors under it.
     ``lo`` / ``hi``: FeatureTable.  Returns (results float64 [P, 23] device tensor in the reference's row layout,
-    lo_mapcoords, hi_mapcoords as NumPy arrays)."""
-    dev = hi.set.dsc.device
-    st = _stream()
-    ph, pl, sc = match_threshold(hi.set, lo.set, cc_threshold, impl=impl)
-    p = int(ph.numel())
-    if p == 0:
-        return torch.empty((0, 23), dtype=torch.float64, device=dev), np.zeros((0, 3)), np.zeros((0, 3))
-    used_hi = torch.zeros(hi.set.rows, dtype=torch.uint8, device=dev)
-    used_lo = torch.zeros(lo.set.rows, dtype=torch.uint8, device=dev)
-    call("mad_mark_used", _ptr(ph), p, _ptr(used_hi), st)
-    call("mad_mark_used", _ptr(pl), p, _ptr(used_lo), st)
-    hi_cloud = np.unique(hi.subv_host[used_hi.cpu().numpy().astype(bool)], axis=0)        # mad/MaD.py:427
-    lo_cloud = np.unique(lo.subv_host[used_lo.cpu().numpy().astype(bool)], axis=0)        # mad/MaD.py:428
-    lo_sorted, cell_start, bits, org, dims = _cloud_grid(lo_cloud, float(anchor_dist_thresh))
-    tb = device_tables(dev)
-    d_hi_cloud = torch.from_numpy(np.ascontiguousarray(hi_cloud)).to(dev)
-    d_lo_sorted = torch.from_numpy(lo_sorted).to(dev)
-    d_cell_start = torch.from_numpy(cell_start).to(dev)
-    d_bits = torch.from_numpy(bits.view(np.int32)).to(dev)
-    results = torch.empty((p, 23), dtype=torch.float64, device=dev)
-    call("mad_repeatability", _ptr(ph), _ptr(pl), _ptr(sc), p, _ptr(hi.subv), _ptr(lo.subv), _ptr(hi.meta), _ptr(lo.meta),
-         _ptr(tb.rf), _ptr(tb.rf_inv), tb.ori_zones, _ptr(d_hi_cloud), len(hi_cloud), _ptr(d_lo_sorted), _ptr(d_cell_start),
-         _ptr(d_bits), _dptr(org), _dptr(dims), C.c_double(float(anchor_dist_thresh)), _ptr(results), st)
-    return results, lo_cloud, hi_cloud
+    lo_mapcoords, hi_mapcoords as NumPy arrays).  The anchor clouds and the lo grid are built on the device (AnchorCloud);
+    the host reads one small record between the matching and the per-pair loop.  The clouds equal np.unique's
+    (np.array_equal) and are byte for byte the same except that a coordinate equal to zero is always +0.0, where np.unique
+    may keep a -0.0 (it treats the two as equal; so does every later use of the clouds)."""
+    m = DscMatch(lo, hi, anchor_dist_thresh, cc_threshold, impl)
+    return m.result(m.table() if m.p else m.empty())
 
 
 def match_dsc_lists(lo_dsc_list, hi_dsc_list, anchor_dist_thresh=4, cc_threshold=0.65):
