@@ -341,6 +341,64 @@ int mad_cloud_grid(const double* cloud, int n, const double* grid_org, const lon
                    double* sorted, int32_t* cell_start, uint32_t* near_bits, void* workspace, size_t workspace_bytes,
                    void* stream);
 
+/* ---- one map against G structures in one batch (mad_b200.pipeline.match_dsc_many) ----------------------------------
+ * The hi rows of the G structures are stacked (structure g owns rows [hi_row_off[g], hi_row_off[g+1])) and matched
+ * against lo once; the pairs come out hi-row-major, so structure g owns the pairs [pair_off[g], pair_off[g+1]).  Every
+ * structure keeps its own anchor clouds and lo grid; the calls below build all of them in one pass, and the results
+ * of structure g equal those of the single-structure calls above on its rows and pairs, bit for bit.
+ *
+ * mad_mark_used_many: pair_off [G + 1] (device) = lower bounds of hi_row_off [G + 1] (device) in pair_hi; used_hi
+ * [hi rows] and used_lo [G][n_lo] (both zeroed by the caller) flag the rows each structure's pairs use. */
+int mad_mark_used_many(const int32_t* pair_hi, const int32_t* pair_lo, long long n_pairs, const long long* hi_row_off, int G,
+                       int n_lo, uint8_t* used_hi, uint8_t* used_lo, long long* pair_off, void* stream);
+/* mad_anchor_cloud_many: mad_anchor_cloud for G segments of n_entries entries at once.  Segment g holds the entries
+ * [seg_off[g], seg_off[g+1]) (seg_off: device int64 [G + 1]); entry e reads row e of subv (shared_rows = 0: the
+ * segments are consecutive slices of subv) or row e - seg_off[g] (shared_rows = 1: every segment indexes the same
+ * rows).  cloud [n_entries][3] receives the G clouds one after the other; grid_org [G][3] and info [G][8] hold per
+ * segment what mad_anchor_cloud's grid_org and info hold (info[8 g] = n_g; segment g's cloud starts after the clouds of
+ * the segments before it).  Equal rows of two segments stay two rows. */
+size_t mad_anchor_cloud_many_workspace_bytes(int n_entries);
+int mad_anchor_cloud_many(const double* subv, const uint8_t* used, int n_entries, const long long* seg_off, int G,
+                          int shared_rows, double cell, double* cloud, double* grid_org, long long* info, void* workspace,
+                          size_t workspace_bytes, void* stream);
+/* One structure of a batch, as the segmented grid and repeatability calls read it. */
+typedef struct MadCloudSeg {
+    long long hi_off;      /* first row of its hi cloud in the concatenated hi clouds */
+    long long lo_off;      /* first row of its lo cloud in the concatenated (and in the cell-sorted) lo clouds */
+    long long cell_off;    /* its first cell in the concatenated cell space of cell_start */
+    long long word_off;    /* its first word of near_bits */
+    double org[3];         /* lo grid origin (the bits mad_anchor_cloud_many recorded) */
+    int hi_n, lo_n;        /* cloud sizes (0 for a structure without pairs) */
+    int dims[3];           /* lo grid dims (ignored when lo_n == 0) */
+    int pad;
+} MadCloudSeg;
+/* mad_cloud_segs_layout (host only): fills hi_off, lo_off, cell_off and word_off of segs[G] from hi_n, lo_n and dims,
+ * and totals[4] = (hi cloud rows, lo cloud rows, cells, near_bits words).  MAD_ERR_ARG if a structure's grid has a dim
+ * < 1 or 2^31 cells or more (the repeatability kernel indexes a structure's cells in int32); the total over the
+ * structures may exceed 2^31 (offsets are int64).
+ * mad_cloud_grid_many: mad_cloud_grid for the G lo clouds of cloud [n][3] (n = totals[1]) at once.  segs_host = the
+ * table mad_cloud_segs_layout laid out (checked: MAD_ERR_ARG otherwise), segs = its device copy, made by the caller (the
+ * repeatability calls below read it too).  sorted [n][3] = the points stably sorted by the global cell id cell_off +
+ * local cell id; cell_start [totals[2] + 1] = points in lower global cells (so its entries index sorted); near_bits
+ * [totals[3]], each structure's bitmap on its own words. */
+int mad_cloud_segs_layout(MadCloudSeg* segs, int G, long long* totals);
+size_t mad_cloud_grid_many_workspace_bytes(int n);
+int mad_cloud_grid_many(const double* cloud, int n, const MadCloudSeg* segs_host, int G, double cell,
+                        const MadCloudSeg* segs, double* sorted, int32_t* cell_start, uint32_t* near_bits, void* workspace,
+                        size_t workspace_bytes, void* stream);
+/* mad_repeat_counts / mad_repeat_rows over the pairs of a batch: pair p belongs to the structure g with pair_off[g] <=
+ * p < pair_off[g+1] (pair_off: device int64 [G + 1]) and is counted against that structure's hi cloud (hi_clouds +
+ * segs[g].hi_off) and lo grid; its row uses 100 * count / segs[g].hi_n.  [p0, p1) may cross structure boundaries. */
+int mad_repeat_counts_many(const int32_t* pair_hi, const int32_t* pair_lo, long long p0, long long p1, const long long* pair_off,
+                           int G, const double* hi_subv, const double* lo_subv, const int32_t* hi_meta, const int32_t* lo_meta,
+                           const double* rf_table, const double* rf_inv_table, int rf_zones, const double* hi_clouds,
+                           const double* lo_sorted, const int32_t* cell_start, const uint32_t* near_bits,
+                           const MadCloudSeg* segs, double dist, int32_t* counts, void* stream);
+int mad_repeat_rows_many(const int32_t* pair_hi, const int32_t* pair_lo, const double* pair_score, long long n_pairs,
+                         const long long* pair_off, int G, const double* hi_subv, const double* lo_subv, const int32_t* hi_meta,
+                         const int32_t* lo_meta, const double* rf_table, const double* rf_inv_table, int rf_zones,
+                         const int32_t* counts, const MadCloudSeg* segs, double* results, void* stream);
+
 /* ---- next component (SURVEY.md 8f rank 2): atoms -> density, mad/PDB.py:131-163,215-292 -------------------- */
 /* Mass-weighted trilinear splat of n_atoms points (xyz [n][3], mass [n], float64) into grid [px][py][pz] float64
  * (zeroed by the call); min_host = lattice-registered minimum corner, margin = 2 + pad (mad/PDB.py:246-285). */

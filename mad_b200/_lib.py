@@ -46,6 +46,11 @@ class MadDscSet(C.Structure):
                 ("max_norm2", C.c_int32)]
 
 
+class MadCloudSeg(C.Structure):
+    _fields_ = [("hi_off", C.c_longlong), ("lo_off", C.c_longlong), ("cell_off", C.c_longlong), ("word_off", C.c_longlong),
+                ("org", C.c_double * 3), ("hi_n", C.c_int32), ("lo_n", C.c_int32), ("dims", C.c_int32 * 3), ("pad", C.c_int32)]
+
+
 _P = C.c_void_p
 _I = C.c_int
 _SZ = C.c_size_t
@@ -112,6 +117,15 @@ SIGNATURES = {
     "mad_anchor_cloud": (_I, [_P, _P, _I, C.c_double, _P, _P, _P, _P, _SZ, _P]),
     "mad_cloud_grid_workspace_bytes": (_SZ, [_I]),
     "mad_cloud_grid": (_I, [_P, _I, _P, _P, C.c_double, _P, _P, _P, _P, _SZ, _P]),
+    "mad_mark_used_many": (_I, [_P, _P, C.c_longlong, _P, _I, _I, _P, _P, _P, _P]),
+    "mad_anchor_cloud_many_workspace_bytes": (_SZ, [_I]),
+    "mad_anchor_cloud_many": (_I, [_P, _P, _I, _P, _I, _I, C.c_double, _P, _P, _P, _P, _SZ, _P]),
+    "mad_cloud_segs_layout": (_I, [_P, _I, _P]),
+    "mad_cloud_grid_many_workspace_bytes": (_SZ, [_I]),
+    "mad_cloud_grid_many": (_I, [_P, _I, _P, _I, C.c_double, _P, _P, _P, _P, _P, _SZ, _P]),
+    "mad_repeat_counts_many": (_I, [_P, _P, C.c_longlong, C.c_longlong, _P, _I, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P,
+                                    C.c_double, _P, _P]),
+    "mad_repeat_rows_many": (_I, [_P, _P, _P, C.c_longlong, _P, _I, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P]),
     "mad_box_scores_workspace_bytes": (_SZ, [_I, _I, _I]),
     "mad_box_scores": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, C.c_float, _P, _P, _SZ, _P]),
     "mad_grid_count_gt": (_I, [_P, C.c_longlong, C.c_float, _P, _P]),

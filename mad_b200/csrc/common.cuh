@@ -37,6 +37,18 @@ __host__ __device__ __forceinline__ int mad_reflect(int i, int n) {
     return i;
 }
 
+// Segment of entry e of a batch whose G segments start at off(0) <= off(1) <= ... (off(0) <= e < total): the largest g
+// with off(g) <= e, which is the non-empty segment holding e (an empty segment shares its start with the next one).
+template <typename Off>
+__host__ __device__ __forceinline__ int mad_segment_of(Off off, int G, long long e) {
+    int lo = 0, hi = G - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (off(mid) <= e) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
 int mad_sm_count();
 
 // ---- launch accounting / optional per-kernel CUDA-event timing (mad_profile_*, api.cu) ----------

@@ -50,12 +50,11 @@ struct CloudArgs {
     double dist;
 };
 
-// counts == nullptr: the count of pair p goes to results[p][1] as a double (mad_repeatability's in-place form)
-__global__ void __launch_bounds__(128)
-repeat_counts_kernel(RepeatArgs a, CloudArgs g, long long p0, int32_t* __restrict__ counts, double* __restrict__ results) {
+// Hits of pair pi: the CTA's threads share the hi cloud; the total is valid in thread 0.  The one body of the per-point
+// arithmetic, for the single-structure and the batched kernel alike.
+__device__ __forceinline__ int count_pair(const RepeatArgs& a, const CloudArgs& g, long long pi) {
     __shared__ double sR[9], shi[3], slo[3];
     __shared__ int s_count;
-    const long long pi = p0 + blockIdx.x;
     const int tid = threadIdx.x;
     const int h = a.pair_hi[pi], l = a.pair_lo[pi];
     if (tid < 9) sR[tid] = pair_rotation(a, h, l, tid);
@@ -90,32 +89,74 @@ repeat_counts_kernel(RepeatArgs a, CloudArgs g, long long p0, int32_t* __restric
     for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xFFFFFFFFu, cnt, o);
     if ((tid & 31) == 0 && cnt) atomicAdd(&s_count, cnt);
     __syncthreads();
-    if (tid == 0) {
-        if (counts) counts[blockIdx.x] = s_count;
-        else results[pi * 23 + 1] = (double)s_count;
+    return s_count;
+}
+
+// counts == nullptr: the count of pair p goes to results[p][1] as a double (mad_repeatability's in-place form)
+__global__ void __launch_bounds__(128)
+repeat_counts_kernel(RepeatArgs a, CloudArgs g, long long p0, int32_t* __restrict__ counts, double* __restrict__ results) {
+    const long long pi = p0 + blockIdx.x;
+    const int n = count_pair(a, g, pi);
+    if (threadIdx.x == 0) {
+        if (counts) counts[blockIdx.x] = n;
+        else results[pi * 23 + 1] = (double)n;
     }
 }
 
-// counts == nullptr: the count is read from results[p][1] (where repeat_counts_kernel left it), by the thread that
-// then overwrites it
+// The pairs [p0, p0 + gridDim.x) of a batch: each CTA counts its pair against the hi cloud and lo grid of the pair's
+// structure (mad_repeat_counts_many).  lo_sorted and cell_start are those of the whole batch: cell_start holds indices
+// into the concatenated cell-sorted clouds, so only the structure's cell and word offsets apply.  The structure's grid
+// arguments sit in registers, not in the constant bank as in repeat_counts_kernel: left alone ptxas gives the kernel 72
+// registers (7 CTAs per SM instead of 8) and it ran 13 % slower per pair on B200; capped at 64 registers (8 CTAs) it
+// spills 52 bytes and runs 8 % slower (DESIGN.md section 6).
+__global__ void __launch_bounds__(128, 8)
+repeat_counts_many_kernel(RepeatArgs a, const long long* __restrict__ pair_off, int G, const MadCloudSeg* __restrict__ segs,
+                          const double* __restrict__ hi_clouds, const double* __restrict__ lo_sorted,
+                          const int32_t* __restrict__ cell_start, const uint32_t* __restrict__ near_bits, double dist,
+                          long long p0, int32_t* __restrict__ counts) {
+    const long long pi = p0 + blockIdx.x;
+    const MadCloudSeg& s = segs[mad_segment_of([&](int k) { return pair_off[k]; }, G, pi)];
+    CloudArgs g;
+    g.hi_cloud = hi_clouds + 3 * s.hi_off; g.H = s.hi_n;
+    g.lo_sorted = lo_sorted; g.cell_start = cell_start + s.cell_off; g.near_bits = near_bits + s.word_off;
+    for (int q = 0; q < 3; ++q) { g.org[q] = s.org[q]; g.dims[q] = s.dims[q]; }
+    g.cell = dist; g.dist = dist;
+    const int n = count_pair(a, g, pi);
+    if (threadIdx.x == 0) counts[blockIdx.x] = n;
+}
+
+// Element e = 23 pi + col of the rows; counts == nullptr: the count is read from results[e] (where repeat_counts_kernel
+// left it), by the thread that then overwrites it.
+__device__ __forceinline__ double row_value(const RepeatArgs& a, const double* __restrict__ pair_score,
+                                            const int32_t* __restrict__ counts, const double* results, long long e, int H) {
+    const long long pi = e / 23;
+    const int col = (int)(e - pi * 23);
+    const int h = a.pair_hi[pi], l = a.pair_lo[pi];
+    if (col == 0) return pair_score[pi];
+    if (col == 1) {
+        const long long cnt = counts ? counts[pi] : (long long)results[e];
+        return (double)(100LL * cnt) / (double)H;                          // 100 * count / l
+    }
+    if (col < 5) return a.lo_meta[4 * l + (col - 2)];                       // lo index, oct, main
+    if (col < 8) return a.hi_meta[4 * h + (col - 5)];                       // hi index, oct, main
+    if (col < 11) return a.hi_subv[3 * (long long)h + (col - 8)];
+    if (col < 14) return a.lo_subv[3 * (long long)l + (col - 11)];
+    return pair_rotation(a, h, l, col - 14);
+}
+
 __global__ void repeat_rows_kernel(RepeatArgs a, const double* __restrict__ pair_score, long long n_pairs,
                                    const int32_t* __restrict__ counts, int H, double* __restrict__ results) {
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n_pairs * 23; e += (long long)gridDim.x * blockDim.x)
+        results[e] = row_value(a, pair_score, counts, results, e, H);
+}
+
+// H of each pair: the hi cloud size of the pair's structure
+__global__ void repeat_rows_many_kernel(RepeatArgs a, const double* __restrict__ pair_score, long long n_pairs,
+                                        const long long* __restrict__ pair_off, int G, const MadCloudSeg* __restrict__ segs,
+                                        const int32_t* __restrict__ counts, double* __restrict__ results) {
     for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n_pairs * 23; e += (long long)gridDim.x * blockDim.x) {
-        const long long pi = e / 23;
-        const int col = (int)(e - pi * 23);
-        const int h = a.pair_hi[pi], l = a.pair_lo[pi];
-        double v;
-        if (col == 0) v = pair_score[pi];
-        else if (col == 1) {
-            const long long cnt = counts ? counts[pi] : (long long)results[e];
-            v = (double)(100LL * cnt) / (double)H;                          // 100 * count / l
-        }
-        else if (col < 5) v = a.lo_meta[4 * l + (col - 2)];                  // lo index, oct, main
-        else if (col < 8) v = a.hi_meta[4 * h + (col - 5)];                  // hi index, oct, main
-        else if (col < 11) v = a.hi_subv[3 * (long long)h + (col - 8)];
-        else if (col < 14) v = a.lo_subv[3 * (long long)l + (col - 11)];
-        else v = pair_rotation(a, h, l, col - 14);
-        results[e] = v;
+        const int H = segs[mad_segment_of([&](int k) { return pair_off[k]; }, G, e / 23)].hi_n;
+        results[e] = row_value(a, pair_score, counts, results, e, H);
     }
 }
 
@@ -221,4 +262,88 @@ extern "C" int mad_repeatability(const int32_t* pair_hi, const int32_t* pair_lo,
                        nullptr, results, stream);
     if (rc != MAD_OK) return rc;
     return launch_rows(a, pair_score, n_pairs, nullptr, n_hi_cloud, results, stream);
+}
+
+namespace {
+
+// Pair p of a batch marks its hi row and, in its structure's row of used_lo, its lo row; threads 0..G write the lower
+// bounds of hi_row_off in pair_hi (pairs are hi-row-major), i.e. pair_off.
+__global__ void mark_used_many_kernel(const int32_t* __restrict__ pair_hi, const int32_t* __restrict__ pair_lo, long long n,
+                                      const long long* __restrict__ hi_row_off, int G, int n_lo, uint8_t* __restrict__ used_hi,
+                                      uint8_t* __restrict__ used_lo, long long* __restrict__ pair_off) {
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n || i <= G; i += (long long)gridDim.x * blockDim.x) {
+        if (i <= G) {
+            long long lo = 0, hi = n;
+            const long long r = hi_row_off[i];
+            while (lo < hi) {
+                const long long mid = (lo + hi) >> 1;
+                if (pair_hi[mid] < r) lo = mid + 1; else hi = mid;
+            }
+            pair_off[i] = lo;
+        }
+        if (i < n) {
+            const int h = pair_hi[i];
+            const int g = mad_segment_of([&](int k) { return hi_row_off[k]; }, G, h);
+            used_hi[h] = 1;
+            used_lo[(long long)g * n_lo + pair_lo[i]] = 1;
+        }
+    }
+}
+
+int launch_counts_many(const RepeatArgs& a, const long long* pair_off, int G, const MadCloudSeg* segs, const double* hi_clouds,
+                       const double* lo_sorted, const int32_t* cell_start, const uint32_t* near_bits, double dist, long long p0,
+                       long long p1, int32_t* counts, void* stream) {
+    MAD_CHECK_ARG(pair_off && G >= 1 && segs && hi_clouds && lo_sorted && cell_start && near_bits && dist > 0.0 && counts);
+    MAD_PROF("repeat_counts_many_kernel", stream);
+    repeat_counts_many_kernel<<<(unsigned)(p1 - p0), 128, 0, (cudaStream_t)stream>>>(a, pair_off, G, segs, hi_clouds, lo_sorted,
+                                                                                    cell_start, near_bits, dist, p0, counts);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}
+
+}  // namespace
+
+extern "C" int mad_mark_used_many(const int32_t* pair_hi, const int32_t* pair_lo, long long n_pairs, const long long* hi_row_off,
+                                  int G, int n_lo, uint8_t* used_hi, uint8_t* used_lo, long long* pair_off, void* stream) {
+    MAD_CHECK_ARG(n_pairs >= 0 && G >= 1 && n_lo >= 0 && hi_row_off && pair_off);
+    MAD_CHECK_ARG(n_pairs == 0 || (pair_hi && pair_lo && used_hi && used_lo));
+    const long long work = std::max<long long>(n_pairs, G + 1);
+    const int blocks = (int)std::min<long long>(mad_ceil_div(work, 256), (long long)mad_sm_count() * 8);
+    MAD_PROF("mark_used_many_kernel", stream);
+    mark_used_many_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(pair_hi, pair_lo, n_pairs, hi_row_off, G, n_lo, used_hi,
+                                                                    used_lo, pair_off);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}
+
+extern "C" int mad_repeat_counts_many(const int32_t* pair_hi, const int32_t* pair_lo, long long p0, long long p1,
+                                      const long long* pair_off, int G, const double* hi_subv, const double* lo_subv,
+                                      const int32_t* hi_meta, const int32_t* lo_meta, const double* rf_table,
+                                      const double* rf_inv_table, int rf_zones, const double* hi_clouds, const double* lo_sorted,
+                                      const int32_t* cell_start, const uint32_t* near_bits, const MadCloudSeg* segs, double dist,
+                                      int32_t* counts, void* stream) {
+    MAD_CHECK_ARG(p0 >= 0 && p0 <= p1 && p1 - p0 < (1LL << 31));
+    if (p1 == p0) return MAD_OK;
+    RepeatArgs a;
+    int rc = fill_args(a, pair_hi, pair_lo, hi_subv, lo_subv, hi_meta, lo_meta, rf_table, rf_inv_table, rf_zones);
+    if (rc != MAD_OK) return rc;
+    return launch_counts_many(a, pair_off, G, segs, hi_clouds, lo_sorted, cell_start, near_bits, dist, p0, p1, counts, stream);
+}
+
+extern "C" int mad_repeat_rows_many(const int32_t* pair_hi, const int32_t* pair_lo, const double* pair_score, long long n_pairs,
+                                    const long long* pair_off, int G, const double* hi_subv, const double* lo_subv,
+                                    const int32_t* hi_meta, const int32_t* lo_meta, const double* rf_table,
+                                    const double* rf_inv_table, int rf_zones, const int32_t* counts, const MadCloudSeg* segs,
+                                    double* results, void* stream) {
+    MAD_CHECK_ARG(n_pairs >= 0 && n_pairs < (1LL << 31));
+    if (n_pairs == 0) return MAD_OK;
+    MAD_CHECK_ARG(pair_score && pair_off && G >= 1 && counts && segs && results);
+    RepeatArgs a;
+    int rc = fill_args(a, pair_hi, pair_lo, hi_subv, lo_subv, hi_meta, lo_meta, rf_table, rf_inv_table, rf_zones);
+    if (rc != MAD_OK) return rc;
+    const int blocks = (int)std::min<long long>(mad_ceil_div(n_pairs * 23, 256), (long long)mad_sm_count() * 16);
+    MAD_PROF("repeat_rows_many_kernel", stream);
+    repeat_rows_many_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(a, pair_score, n_pairs, pair_off, G, segs, counts, results);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
 }

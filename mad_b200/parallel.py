@@ -272,48 +272,60 @@ def match_topk_grid_sets(hi_block_set, lo_shard_set, k, m_total, lo_index_base, 
 # ---------------------------------------------------------------------------------------------------------------------
 # MaD._match_dsc with the per-pair repeatability shared out over the ranks
 # ---------------------------------------------------------------------------------------------------------------------
-def pad_counts(local, n_pairs, world):
-    """This rank's counts (its share of ``shard_bounds(n_pairs, world)``) padded to the longest share, the first."""
-    per = shard_bounds(n_pairs, world)[0][1]
+def pad_counts(local, n_pairs, world, bounds=None):
+    """This rank's counts padded to the longest share: of ``bounds`` if given, else of ``shard_bounds(n_pairs, world)``
+    (the first)."""
+    per = max(e - s for s, e in bounds) if bounds is not None else shard_bounds(n_pairs, world)[0][1]
     out = torch.zeros(per, dtype=torch.int32, device=local.device)
     out[:local.numel()] = local
     return out
 
 
-def join_counts(gathered, n_pairs):
-    """[G, per] padded shares in rank order -> the counts of all ``n_pairs`` pairs."""
+def join_counts(gathered, n_pairs, bounds=None):
+    """[G, per] padded shares in rank order -> the counts of all ``n_pairs`` pairs (shares ``bounds``, by default
+    ``shard_bounds(n_pairs, G)``)."""
     g = gathered.shape[0]
-    return torch.cat([gathered[r, :e - s] for r, (s, e) in enumerate(shard_bounds(n_pairs, g))])
+    bounds = shard_bounds(n_pairs, g) if bounds is None else bounds
+    return torch.cat([gathered[r, :e - s] for r, (s, e) in enumerate(bounds)])
 
 
-def check_same_problem(rows_hi, rows_lo, n_pairs, device, group=None):
+def check_same_problem(rows_hi, rows_lo, n_pairs, device, group=None, n_structures=None):
     """One all_reduce (max of (x, -x)): raises MadError on every rank if the ranks do not hold the same sets and pair
-    count, where a gather of differently sized shares would hang."""
-    t = torch.tensor([rows_hi, rows_lo, n_pairs], dtype=torch.int64, device=device)
+    count -- and, for a batch, the same number of structures -- where a gather of differently sized shares would hang."""
+    if n_structures is None:
+        names, vals = "(hi rows, lo rows, pairs)", [rows_hi, rows_lo, n_pairs]
+    else:
+        names, vals = "(structures, lo rows, hi rows, pairs)", [n_structures, rows_lo, rows_hi, n_pairs]
+    t = torch.tensor(vals, dtype=torch.int64, device=device)
     both = torch.cat([t, -t])
     dist.all_reduce(both, op=dist.ReduceOp.MAX, group=group)
-    hi_, lo_ = both[:3].tolist(), [-v for v in both[3:].tolist()]
+    k = len(vals)
+    hi_, lo_ = both[:k].tolist(), [-v for v in both[k:].tolist()]
     if hi_ != lo_:
         from ._lib import MadError
-        raise MadError("match_dsc_sharded: the ranks disagree on (hi rows, lo rows, pairs): from %r to %r" % (lo_, hi_))
+        what = "match_dsc_sharded" if n_structures is None else "match_dsc_many_sharded"
+        raise MadError("%s: the ranks disagree on %s: from %r to %r" % (what, names, lo_, hi_))
 
 
-def gather_pair_counts(local, n_pairs, rows_hi, rows_lo, group=None):
-    """The counts of all ``n_pairs`` pairs on every rank from each rank's share (``shard_bounds(n_pairs, G)[rank]``):
-    the consistency check, then ONE all_gather of the shares padded to equal size (``all_gather_into_tensor``, or the list
-    form on a backend without it).  No collective at all for n_pairs == 0, so the check cannot catch one rank with no
-    pairs while another has some: the ranks with pairs then wait in the check's all_reduce until the backend's time-out."""
+def gather_pair_counts(local, n_pairs, rows_hi, rows_lo, group=None, bounds=None, n_structures=None):
+    """The counts of all ``n_pairs`` pairs on every rank from each rank's share (``bounds[rank]``; by default
+    ``shard_bounds(n_pairs, G)[rank]``): the consistency check, then ONE all_gather of the shares padded to equal size
+    (``all_gather_into_tensor``, or the list form on a backend without it).  ``n_structures``: the batch size of a
+    ``match_dsc_many_sharded`` call, also checked.  No collective at all for n_pairs == 0, so the check cannot catch one
+    rank with no pairs while another has some: the ranks with pairs then wait in the check's all_reduce until the
+    backend's time-out."""
     g = _world(group)
     if g == 1 or n_pairs == 0:
         return local
-    check_same_problem(rows_hi, rows_lo, n_pairs, local.device, group)
-    pad = pad_counts(local, n_pairs, g)
+    check_same_problem(rows_hi, rows_lo, n_pairs, local.device, group, n_structures)
+    bounds = shard_bounds(n_pairs, g) if bounds is None else bounds
+    pad = pad_counts(local, n_pairs, g, bounds)
     out = torch.empty((g, pad.numel()), dtype=torch.int32, device=local.device)
     try:
         dist.all_gather_into_tensor(out, pad, group=group)
     except (RuntimeError, NotImplementedError):             # a backend without the tensor form
         dist.all_gather(list(out.unbind(0)), pad, group=group)
-    return join_counts(out, n_pairs)
+    return join_counts(out, n_pairs, bounds)
 
 
 def match_dsc_local(m, rank, world):
@@ -345,3 +357,62 @@ def match_dsc_lists_sharded(lo_dsc_list, hi_dsc_list, anchor_dist_thresh=4, cc_t
     res, lo_cloud, hi_cloud = match_dsc_sharded(P.FeatureTable.from_features(lo_dsc_list), P.FeatureTable.from_features(hi_dsc_list),
                                                 anchor_dist_thresh, cc_threshold, group=group)
     return list(res.cpu().numpy()), lo_cloud, hi_cloud
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# one map against G structures in one batch, the per-pair repeatability shared out by work
+# ---------------------------------------------------------------------------------------------------------------------
+def shard_bounds_weighted(pair_off, H, world):
+    """Contiguous shares [(start, end)] * world of the pairs of a batch, of about equal work: a pair of structure g (the
+    pairs [pair_off[g], pair_off[g+1])) costs H[g], the size of that structure's hi cloud.  Rank r's share starts at the
+    first pair p whose preceding work is >= r / world of the total, so every share is within one pair's work of an equal
+    split.  Exact integer arithmetic on values every rank holds: every rank computes the same bounds."""
+    pair_off = [int(v) for v in pair_off]
+    H = [int(h) for h in H]
+    world = int(world)
+    n_pairs = pair_off[-1]
+    before = [0]                                              # work of the pairs before structure g
+    for g in range(len(H)):
+        before.append(before[-1] + (pair_off[g + 1] - pair_off[g]) * H[g])
+    total = before[-1]
+    cuts = [0]
+    for r in range(1, world):
+        t, p = r * total, n_pairs                             # first p with world * work(pairs < p) >= t
+        for g in range(len(H)):
+            n_g = pair_off[g + 1] - pair_off[g]
+            if n_g and before[g + 1] * world >= t:
+                need = t - before[g] * world
+                k = -(-need // (H[g] * world)) if H[g] > 0 and need > 0 else 0
+                p = pair_off[g] + min(k, n_g)
+                break
+        cuts.append(max(p, cuts[-1]))
+    cuts.append(n_pairs)
+    return [(cuts[r], cuts[r + 1]) for r in range(world)]
+
+
+def match_dsc_many_local(m, rank, world):
+    """This rank's step of ``match_dsc_many_sharded`` on a ``pipeline.DscMatchMany``: the counts of its weighted share."""
+    s, e = shard_bounds_weighted(m.pair_off, m.hi_n, world)[rank]
+    return m.counts(s, e)
+
+
+def match_dsc_many_sharded(lo, his, anchor_dist_thresh=4, cc_threshold=0.65, group=None, impl=None):
+    """``pipeline.match_dsc_many`` with the per-pair repeatability shared out over the ranks of ``group``.  Every rank holds
+    the map and all structures and computes the same pairs, clouds and grids; rank r counts the hits of its contiguous
+    share ``shard_bounds_weighted(pair_off, H, G)[r]`` (equal work, not equal pair count: a pair of structure g visits
+    its H_g hi anchors), the counts are all-gathered and every rank expands all rows.  Every rank returns what
+    ``pipeline.match_dsc_many`` returns on one GPU, bit for bit.  Ranks holding different batches raise MadError (the
+    check compares structures, lo rows, hi rows and pairs), except that, as for ``match_dsc_sharded``, a batch without
+    pairs returns at once without a collective: a rank with no pairs next to ranks with pairs leaves those waiting in
+    the check until the backend's time-out."""
+    from . import pipeline as P
+    m = P.DscMatchMany(lo, his, anchor_dist_thresh, cc_threshold, impl)
+    if m.p == 0:
+        return m.results(m.empty())
+    g = _world(group)
+    rank = dist.get_rank(group) if g > 1 else 0
+    bounds = shard_bounds_weighted(m.pair_off, m.hi_n, g)
+    s, e = bounds[rank]
+    counts = gather_pair_counts(m.counts(s, e), m.p, int(m.hi_row_off[-1]), lo.set.rows, group, bounds=bounds,
+                                n_structures=m.G)
+    return m.results(m.rows(counts))

@@ -64,21 +64,31 @@ class _Readback(object):
 
     @classmethod
     def read(cls, *tensors):
-        """Values of the given small int32 / int64 device tensors as Python ints (one synchronisation)."""
+        """Values of the given small int32 / int64 device tensors as Python ints (one synchronisation).  A tensor of more
+        than 4096 bytes (the per-structure records of a large ``match_dsc_many`` batch) travels by one mad_copy_to_host
+        launch, or, if it is not 16-byte aligned, in 4096-byte pieces."""
         dev = tensors[0].device
         key = (dev.index, torch.cuda.current_stream().cuda_stream)
         slot = cls._slots.get(key)
-        if slot is None:
-            slot = cls._slots[key] = torch.zeros(512, dtype=torch.int64).pin_memory()
+        need = sum((t.numel() * t.element_size() + 15) // 16 * 2 for t in tensors)
+        if slot is None or slot.numel() < need:
+            slot = cls._slots[key] = torch.zeros(max(512, need), dtype=torch.int64).pin_memory()
         st = _stream()
         off, views = 0, []
         for t in tensors:
             t = t.contiguous().view(-1)
             nbytes = t.numel() * t.element_size()
             assert nbytes % 4 == 0 and off + nbytes <= slot.numel() * 8
-            call("mad_publish_small", _ptr(t), C.c_void_p(slot.data_ptr() + off), nbytes, st)
+            dst = slot.data_ptr() + off
+            if nbytes <= 4096:
+                call("mad_publish_small", _ptr(t), C.c_void_p(dst), nbytes, st)
+            elif t.data_ptr() % 16 == 0:
+                call("mad_copy_to_host", _ptr(t), C.c_void_p(dst), nbytes, 1, st)
+            else:
+                for o in range(0, nbytes, 4096):
+                    call("mad_publish_small", C.c_void_p(t.data_ptr() + o), C.c_void_p(dst + o), min(4096, nbytes - o), st)
             views.append((off, t.dtype, t.numel()))
-            off += (nbytes + 7) // 8 * 8
+            off += (nbytes + 15) // 16 * 16
         torch.cuda.current_stream().synchronize()
         raw = slot.numpy()
         out = []
@@ -1056,3 +1066,213 @@ def match_dsc_lists(lo_dsc_list, hi_dsc_list, anchor_dist_thresh=4, cc_threshold
     res, lo_cloud, hi_cloud = match_dsc(FeatureTable.from_features(lo_dsc_list), FeatureTable.from_features(hi_dsc_list),
                                         anchor_dist_thresh, cc_threshold)
     return list(res.cpu().numpy()), lo_cloud, hi_cloud
+
+
+# ---------------------------------------------------------------------------------------------
+# one map against G structures (subunits of an assembly, frames of an ensemble) in one batch
+# ---------------------------------------------------------------------------------------------
+def _to_device(values, dev):
+    """Small int64 host list -> device tensor through pinned memory (no synchronisation)."""
+    return torch.tensor(np.asarray(values, dtype=np.int64)).pin_memory().to(dev, non_blocking=True)
+
+
+class AnchorClouds(object):
+    """AnchorCloud for G segments in one pass (``mad_anchor_cloud_many``): segment g holds the entries [off[g], off[g+1]) of
+    ``used``; shared_rows=False: the entries are rows of ``subv`` (the stacked hi rows), True: entry e of segment g is row
+    e - off[g] of ``subv`` (every structure's flags over the same lo rows).  The clouds lie one after the other in
+    ``cloud``; ``build_grids`` builds every lo grid in one pass (``mad_cloud_grid_many``)."""
+
+    def __init__(self, subv, used, seg_off, n_entries, cell, shared_rows=False):
+        dev = subv.device
+        self.G = int(seg_off.numel()) - 1
+        self.cell = float(cell)
+        self._buf = torch.empty((max(n_entries, 1), 3), dtype=torch.float64, device=dev)
+        self.org_dev = torch.empty((self.G, 3), dtype=torch.float64, device=dev)
+        self.info = torch.empty((self.G, 8), dtype=torch.int64, device=dev)
+        ws_bytes = _lib.lib.mad_anchor_cloud_many_workspace_bytes(n_entries)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        call("mad_anchor_cloud_many", _ptr(subv), _ptr(used), int(n_entries), _ptr(seg_off), self.G, 1 if shared_rows else 0,
+             C.c_double(self.cell), _ptr(self._buf), _ptr(self.org_dev), _ptr(self.info), _ptr(ws), ws_bytes, _stream())
+        self.n = None
+
+    def take_info(self, vals, what):
+        """The 8 G values of ``info`` read back; refuses, naming the structure, a cloud with a non-finite coordinate."""
+        v = np.array(vals, dtype=np.int64).reshape(self.G, 8)
+        for g in range(self.G):
+            if v[g, 1]:
+                raise _lib.MadError("%s: structure %d: %d used feature(s) with a non-finite coordinate" % (what, g, v[g, 1]))
+        self.n = v[:, 0].copy()
+        self.off = np.concatenate([[0], np.cumsum(self.n)]).astype(np.int64)
+        self.dims64 = v[:, 2:5].copy()
+        self.org = v[:, 5:8].copy().view(np.float64)
+        self.cloud = self._buf[:int(self.off[-1])]
+        return self
+
+    def cloud_of(self, g):
+        return self._buf[int(self.off[g]):int(self.off[g + 1])]
+
+    def build_grids(self, hi_n, what):
+        """The lo grids of all segments (refused, naming the structure, for a grid of >= 2^31 cells) and the segment table
+        ``segs`` the repeatability kernels read; ``hi_n`` = the hi cloud size of every structure."""
+        dev = self._buf.device
+        segs = (_lib.MadCloudSeg * self.G)()
+        for g in range(self.G):
+            s = segs[g]
+            s.hi_n, s.lo_n = int(hi_n[g]), int(self.n[g])
+            if s.lo_n:
+                ncell = int(np.prod([int(d) for d in self.dims64[g]], dtype=object))
+                if ncell >= 1 << 31:
+                    raise _lib.MadError("%s: structure %d: a lo grid of %d cells (>= 2^31, which the repeatability kernel "
+                                        "cannot index)" % (what, g, ncell))
+                for q in range(3):
+                    s.dims[q], s.org[q] = int(self.dims64[g, q]), float(self.org[g, q])
+        totals = (C.c_longlong * 4)()
+        call("mad_cloud_segs_layout", segs, self.G, totals)
+        self.segs_host = segs
+        self.cells, self.words = int(totals[2]), int(totals[3])
+        L = int(totals[1])
+        # the table goes to the device from pinned memory through torch, which keeps the pinned block from reuse until
+        # the copy has run: no host synchronisation
+        pinned = torch.frombuffer(bytearray(segs), dtype=torch.uint8).pin_memory()
+        self.segs = torch.empty(pinned.numel(), dtype=torch.uint8, device=dev)
+        self.segs.copy_(pinned, non_blocking=True)
+        self.sorted = torch.empty((max(L, 1), 3), dtype=torch.float64, device=dev)
+        self.cell_start = torch.empty(self.cells + 1, dtype=torch.int32, device=dev)
+        self.near_bits = torch.zeros(max(self.words, 1), dtype=torch.int32, device=dev)
+        if L:
+            ws_bytes = _lib.lib.mad_cloud_grid_many_workspace_bytes(L)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            call("mad_cloud_grid_many", _ptr(self.cloud), L, segs, self.G, C.c_double(self.cell), _ptr(self.segs),
+                 _ptr(self.sorted), _ptr(self.cell_start), _ptr(self.near_bits), _ptr(ws), ws_bytes, _stream())
+        self.sorted = self.sorted[:L]
+        return self
+
+    def grid_of(self, g):
+        """(sorted, cell_start, near_bits) of structure g as ``AnchorCloud.build_grid`` makes them alone."""
+        s = self.segs_host[g]
+        ncell = s.dims[0] * s.dims[1] * s.dims[2] if s.lo_n else 0
+        return (self.sorted[s.lo_off:s.lo_off + s.lo_n], self.cell_start[s.cell_off:s.cell_off + ncell + 1] - int(s.lo_off),
+                self.near_bits[s.word_off:s.word_off + (ncell + 31) // 32])
+
+
+def anchor_clouds(subvs, useds, cell):
+    """Segmented clouds and grids of several (subv float64 [D_g, 3], used uint8 [D_g]) device tensors: one AnchorClouds
+    over the stacked rows, the counterpart of ``anchor_cloud`` per structure."""
+    dev = subvs[0].device
+    off = np.concatenate([[0], np.cumsum([int(s.shape[0]) for s in subvs])]).astype(np.int64)
+    c = AnchorClouds(torch.cat(list(subvs)).contiguous(), torch.cat(list(useds)).contiguous(), _to_device(off, dev), int(off[-1]),
+                     cell)
+    c.take_info(_Readback.read(c.info), "anchor_clouds")
+    return c.build_grids(np.zeros(c.G, dtype=np.int64), "anchor_clouds")
+
+
+def stack_sets(his):
+    """One DescriptorSet over the rows of the FeatureTables ``his``, in order.  The matching kernel is chosen for the
+    stacked set (by its largest entry over all structures); every kernel gives the same pairs with bit-identical scores
+    (tests/test_match_edges.py), so each structure's pairs are those its own set gives."""
+    return his[0].set if len(his) == 1 else DescriptorSet(torch.cat([h.set.dsc for h in his]))
+
+
+class DscMatchMany(object):
+    """``DscMatch`` for one map ``lo`` against G structures ``his`` in one batch.  The stacked hi rows are matched once;
+    pairs come out hi-row-major, so structure g owns the pairs [pair_off[g], pair_off[g+1]) (``p`` in all).  Every
+    structure keeps its own hi cloud, lo cloud and lo grid (AnchorClouds), built for all structures in one pass.  Two host
+    read-backs in all, as for one DscMatch: the pair count, then pair_off with every structure's cloud records."""
+
+    def __init__(self, lo, his, anchor_dist_thresh=4, cc_threshold=0.65, impl=None, pairs=None):
+        """pairs: the (hi, lo, score) list of ``match_threshold(stack_sets(his), lo.set, cc_threshold)`` if already
+        computed."""
+        self.lo, self.his = lo, list(his)
+        self.G = len(self.his)
+        self.dist = float(anchor_dist_thresh)
+        self.hi_row_off = np.concatenate([[0], np.cumsum([h.set.rows for h in self.his])]).astype(np.int64)
+        self.pair_off = np.zeros(self.G + 1, dtype=np.int64)
+        self.hi_n = np.zeros(self.G, dtype=np.int64)
+        self.p = 0
+        self.hi_clouds = self.lo_clouds = None
+        if self.G == 0:
+            return
+        dev = lo.set.dsc.device
+        what = "match_dsc_many"
+        d_lo = lo.set.rows
+        if self.G * d_lo >= 1 << 31:
+            raise _lib.MadError("%s: %d structures x %d lo rows: the lo used flags need < 2^31 entries" % (what, self.G, d_lo))
+        # one descriptor set over all structures' rows: every matching kernel gives the same pairs and bit-identical scores
+        self.hi_subv = torch.cat([h.subv for h in self.his]).contiguous()
+        self.hi_meta = torch.cat([h.meta for h in self.his]).contiguous()
+        if pairs is None:
+            pairs = match_threshold(stack_sets(self.his), lo.set, cc_threshold, impl=impl)
+        self.ph, self.pl, self.sc = pairs
+        self.p = int(self.ph.numel())
+        if self.p == 0:
+            return
+        st = _stream()
+        row_off = _to_device(self.hi_row_off, dev)
+        used_hi = torch.zeros(int(self.hi_row_off[-1]), dtype=torch.uint8, device=dev)
+        used_lo = torch.zeros(self.G * d_lo, dtype=torch.uint8, device=dev)
+        self.pair_off_dev = torch.empty(self.G + 1, dtype=torch.int64, device=dev)
+        call("mad_mark_used_many", _ptr(self.ph), _ptr(self.pl), self.p, _ptr(row_off), self.G, d_lo, _ptr(used_hi), _ptr(used_lo),
+             _ptr(self.pair_off_dev), st)
+        hc = AnchorClouds(self.hi_subv, used_hi, row_off, int(self.hi_row_off[-1]), self.dist)                  # mad/MaD.py:427
+        lo_off = torch.arange(self.G + 1, dtype=torch.int64, device=dev) * d_lo
+        lc = AnchorClouds(lo.subv, used_lo, lo_off, self.G * d_lo, self.dist, shared_rows=True)                # mad/MaD.py:428
+        vals = _Readback.read(self.pair_off_dev, hc.info, lc.info)
+        g1 = self.G + 1
+        self.pair_off = np.array(vals[:g1], dtype=np.int64)
+        self.hi_clouds = hc.take_info(vals[g1:g1 + 8 * self.G], what)
+        self.lo_clouds = lc.take_info(vals[g1 + 8 * self.G:], what)
+        self.hi_n = self.hi_clouds.n
+        self.lo_clouds.build_grids(self.hi_n, what)
+        self.tb = device_tables(dev)
+
+    def _common(self):
+        return (_ptr(self.hi_subv), _ptr(self.lo.subv), _ptr(self.hi_meta), _ptr(self.lo.meta), _ptr(self.tb.rf),
+                _ptr(self.tb.rf_inv), self.tb.ori_zones)
+
+    def counts(self, p0, p1):
+        """int32 [p1 - p0]: hits of the batch's pairs [p0, p1), which may span several structures (mad_repeat_counts_many)."""
+        out = torch.empty(max(p1 - p0, 1), dtype=torch.int32, device=self.ph.device)
+        if p1 > p0:
+            g = self.lo_clouds
+            call("mad_repeat_counts_many", _ptr(self.ph), _ptr(self.pl), int(p0), int(p1), _ptr(self.pair_off_dev), self.G,
+                 *self._common(), _ptr(self.hi_clouds.cloud), _ptr(g.sorted), _ptr(g.cell_start), _ptr(g.near_bits), _ptr(g.segs),
+                 C.c_double(self.dist), _ptr(out), _stream())
+        return out[:p1 - p0]
+
+    def rows(self, counts):
+        """float64 [P, 23]: the rows of all P pairs of the batch from their hits (mad_repeat_rows_many)."""
+        if counts.numel() != self.p or counts.dtype != torch.int32 or counts.device != self.ph.device:
+            raise _lib.MadError("DscMatchMany.rows: needs int32 counts of all %d pairs on %s, got %s [%d] on %s"
+                                % (self.p, self.ph.device, counts.dtype, counts.numel(), counts.device))
+        res = torch.empty((self.p, 23), dtype=torch.float64, device=self.ph.device)
+        call("mad_repeat_rows_many", _ptr(self.ph), _ptr(self.pl), _ptr(self.sc), self.p, _ptr(self.pair_off_dev), self.G,
+             *self._common(), _ptr(counts.contiguous()), _ptr(self.lo_clouds.segs), _ptr(res), _stream())
+        return res
+
+    def empty(self):
+        return torch.empty((0, 23), dtype=torch.float64, device=self.lo.set.dsc.device)
+
+    def results(self, table):
+        """[(table, lo_mapcoords, hi_mapcoords)] per structure: what ``match_dsc`` returns for each, the tables as slices
+        of ``table``."""
+        hi_host = self.hi_clouds.cloud.cpu().numpy() if self.p else None
+        lo_host = self.lo_clouds.cloud.cpu().numpy() if self.p else None
+        out = []
+        for g in range(self.G):
+            a, b = int(self.pair_off[g]), int(self.pair_off[g + 1])
+            if a == b:
+                out.append((table[a:b], np.zeros((0, 3)), np.zeros((0, 3))))
+            else:
+                lo_o, hi_o = self.lo_clouds.off, self.hi_clouds.off
+                out.append((table[a:b], lo_host[lo_o[g]:lo_o[g + 1]], hi_host[hi_o[g]:hi_o[g + 1]]))
+        return out
+
+
+def match_dsc_many(lo, his, anchor_dist_thresh=4, cc_threshold=0.65, impl=None):
+    """``match_dsc`` of one map ``lo`` against each FeatureTable of ``his`` (the subunits of an assembly, the frames of an
+    ensemble) in one batch: result g equals ``match_dsc(lo, his[g], anchor_dist_thresh, cc_threshold, impl)`` -- the
+    table bit for bit (a slice of one device tensor), the clouds byte for byte.  The work per batch does not grow with
+    len(his): one threshold matching over the stacked hi rows, one pass for all clouds and grids, one launch each for the
+    counts and the rows, and two host read-backs, as for one ``match_dsc`` call."""
+    m = DscMatchMany(lo, his, anchor_dist_thresh, cc_threshold, impl)
+    return m.results(m.rows(m.counts(0, m.p)) if m.p else m.empty())
