@@ -298,8 +298,16 @@ int mad_mark_used(const int32_t* idx, long long n, uint8_t* used, void* stream);
  * repeatability = 100 * #{q with a lo-cloud point closer than dist} / n_hi_cloud.
  * results[p][23] = score, repeatability, lo (index, oct, main), hi (index, oct, main), subv_hi[3], subv_lo[3], R[9]
  * -- the row layout of the reference (mad/MaD.py:451).  *_meta: int32 [D][4] = index, oct_scale, main_bin, sec_bin.
- * The lo cloud comes cell-sorted for a uniform grid of cell size dist: lo_sorted [L][3], cell_start [ncell + 1],
- * near_bits = bitmap of cells whose 27-cell neighbourhood is non-empty; grid_org_host / grid_dims_host (host). */
+ * The exact float64 sequence (fma = one rounding of the exact a b + c; A = inv(Rfinal_lo), B = Rfinal_hi):
+ *     R[i][j] = fma(A[i][2], B[2][j], fma(A[i][1], B[1][j], A[i][0] * B[0][j]))
+ *     d = c - subv_hi;  q[i] = fma(d[2], R[i][2], fma(d[1], R[i][1], d[0] * R[i][0])) + subv_lo[i]
+ *     e = l - q;  q counts if some lo-cloud point l has sqrt(fma(e[2], e[2], fma(e[1], e[1], e[0] * e[0]))) < dist
+ *     (strictly), and repeatability = (double)(100 * count) / (double)n_hi_cloud (one correctly rounded division).
+ * The lo cloud comes cell-sorted for a uniform grid of cell size mad_repeat_grid_cell(dist) (mad_cloud_grid with that
+ * cell): lo_sorted [L][3], cell_start [ncell + 1], near_bits = bitmap of cells whose 27-cell neighbourhood is non-empty;
+ * grid_org_host / grid_dims_host (host).  Every q with a lo point closer than dist is found (csrc/repeat.cu states why). */
+/* The lo grid's cell for the distance dist: dist * (1 + 2^-16), a little larger than dist (host function). */
+double mad_repeat_grid_cell(double dist);
 int mad_repeatability(const int32_t* pair_hi, const int32_t* pair_lo, const double* pair_score, long long n_pairs,
                       const double* hi_subv, const double* lo_subv, const int32_t* hi_meta, const int32_t* lo_meta,
                       const double* rf_table, const double* rf_inv_table, int rf_zones,
@@ -388,7 +396,8 @@ int mad_cloud_grid_many(const double* cloud, int n, const MadCloudSeg* segs_host
                         size_t workspace_bytes, void* stream);
 /* mad_repeat_counts / mad_repeat_rows over the pairs of a batch: pair p belongs to the structure g with pair_off[g] <=
  * p < pair_off[g+1] (pair_off: device int64 [G + 1]) and is counted against that structure's hi cloud (hi_clouds +
- * segs[g].hi_off) and lo grid; its row uses 100 * count / segs[g].hi_n.  [p0, p1) may cross structure boundaries. */
+ * segs[g].hi_off) and lo grid (built with the cell mad_repeat_grid_cell(dist)); its row uses 100 * count / segs[g].hi_n.
+ * [p0, p1) may cross structure boundaries. */
 int mad_repeat_counts_many(const int32_t* pair_hi, const int32_t* pair_lo, long long p0, long long p1, const long long* pair_off,
                            int G, const double* hi_subv, const double* lo_subv, const int32_t* hi_meta, const int32_t* lo_meta,
                            const double* rf_table, const double* rf_inv_table, int rf_zones, const double* hi_clouds,

@@ -108,6 +108,7 @@ SIGNATURES = {
     "mad_normalise_f64": (_I, [_P, C.c_longlong, _P, _P]),
     "mad_conv_full_f64": (_I, [_P, C.c_longlong, _I, C.c_longlong, _P, _I, _P, _I, _P]),
     "mad_mark_used": (_I, [_P, C.c_longlong, _P, _P]),
+    "mad_repeat_grid_cell": (C.c_double, [C.c_double]),
     "mad_repeatability": (_I, [_P, _P, _P, C.c_longlong, _P, _P, _P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _P, _P,
                                C.c_double, _P, _P]),
     "mad_repeat_counts": (_I, [_P, _P, C.c_longlong, C.c_longlong, _P, _P, _P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _P, _P,

@@ -7,11 +7,35 @@
 //
 // Two kernels share the per-pair arithmetic (pair_rotation: the roundings are the same by construction):
 // repeat_counts_kernel counts the hits of the pairs [p0, p1), one CTA per pair, threads over the hi cloud; the lo cloud
-// sits in a uniform grid of cell size `dist` (cell-sorted points + cell_start, mad_cloud_grid); a bitmap of the cells
+// sits in a uniform grid of cells a little larger than `dist` (cell-sorted points + cell_start, mad_cloud_grid); a bitmap of the cells
 // whose 27-cell neighbourhood holds any lo point rejects most transformed anchors with one probe.
 // repeat_rows_kernel expands (pair, count) into the 23-column rows, one thread per output value.  Splitting the pair
 // range is what lets several GPUs share the counting (mad_b200.parallel.match_dsc_sharded).
-// All arithmetic is float64 like NumPy's.
+//
+// The arithmetic is float64 with every rounding written out, so that it does not depend on nvcc's contraction choices
+// (fma(a, b, c) below is rounded once, from the exact a b + c; tests/repeat_ref.py evaluates the same sequence exactly):
+//     R[i][j] = fma(A[i][2], B[2][j], fma(A[i][1], B[1][j], A[i][0] B[0][j]))        A = inv(Rfinal_lo), B = Rfinal_hi
+//     d = p - subv_hi,   q[i] = fma(d[2], R[i][2], fma(d[1], R[i][1], d[0] R[i][0])) + subv_lo[i]
+//     e = l - q,         hit  = sqrt(fma(e[2], e[2], fma(e[1], e[1], e[0] e[0]))) < dist   (l: a lo cloud point)
+// and column 1 of a row is (100 count) / H.  NumPy's plain sums differ from this by an ulp at times (the reference's
+// R comes from a dgemm), which is why a count against the reference may flip when a distance is within ulps of dist.
+//
+// Why the 27-cell search finds every hit.  The lo grid is built with the cell c = mad_repeat_grid_cell(dist) =
+// dist (1 + 2^-16), a little more than dist, while a hit still needs a distance < dist.  Let u = 2^-53, org = RN(min - c),
+// dims = floor(t(max)) + 2 per axis, where t(x) = RN(RN(x - org) / c) is the cell coordinate the builder and this kernel
+// both compute (cell index floor(t)).  Take a lo point l and a transformed anchor q whose computed distance is < dist:
+//   (a) on each axis |l - q| < dist (1 + 3u): the computed sum is >= RN(e e) of any one axis (roundings are monotone
+//       and the terms non-negative), so sqrt of it < dist gives |e| < dist (1 + u), and e = RN(l - q).
+//   (b) q >= org: org is the double nearest to min - c, so a double q < org has q <= min - c, and then
+//       l - q >= c > dist (1 + 3u), against (a).  So t(q) >= 0.
+//   (c) t(x) = (x - org) / c (1 + th) with |th| <= 3u.  For the lo point 0 <= t(l) < dims - 1, and each dim is < 2^29
+//       (the builder refuses grids of 2^31 cells or more, and every dim is >= 2), so the rounding terms add less than
+//       3u (2 dims + 1) < 2^-21, and with c >= dist (1 + 2^-16) (1 - u),
+//       |t(l) - t(q)| < (1 + 4u) / (1 + 2^-16) + 2^-21 < 1 - 2^-17 + 2^-21 < 1.
+// So floor(t(q)) is within 1 of l's cell on every axis, and q's cell lies inside the grid (0 <= cq <= dims - 1): q is
+// not skipped, its near bit is set and l's cell is among the ones searched.  With c = dist the first term of (c) is 1
+// and the roundings alone can put l two cells away from q.  A q far outside (up to any finite value) is skipped by
+// the range test: the float64 -> int conversion saturates.
 #include <algorithm>
 
 #include "common.cuh"
@@ -35,7 +59,7 @@ __device__ __forceinline__ double pair_rotation(const RepeatArgs& a, int h, int 
     const double* A = a.rf_inv + ((long long)a.lo_meta[4 * l + 2] * a.zones + a.lo_meta[4 * l + 3]) * 9;
     const double* B = a.rf + ((long long)a.hi_meta[4 * h + 2] * a.zones + a.hi_meta[4 * h + 3]) * 9;
     const int i = tid / 3, j = tid % 3;
-    return (A[3 * i] * B[j] + A[3 * i + 1] * B[3 + j]) + A[3 * i + 2] * B[6 + j];
+    return fma(A[3 * i + 2], B[6 + j], fma(A[3 * i + 1], B[3 + j], __dmul_rn(A[3 * i], B[j])));
 }
 
 struct CloudArgs {
@@ -46,7 +70,7 @@ struct CloudArgs {
     const uint32_t* near_bits;  // [ceil(ncell / 32)]: some lo point in the 27-cell neighbourhood
     double org[3];
     int dims[3];
-    double cell;                // = dist
+    double cell;                // = mad_repeat_grid_cell(dist)
     double dist;
 };
 
@@ -64,9 +88,9 @@ __device__ __forceinline__ int count_pair(const RepeatArgs& a, const CloudArgs& 
     int cnt = 0;
     for (int p = tid; p < g.H; p += blockDim.x) {
         const double dx = g.hi_cloud[3 * p] - shi[0], dy = g.hi_cloud[3 * p + 1] - shi[1], dz = g.hi_cloud[3 * p + 2] - shi[2];
-        const double qx = ((dx * sR[0] + dy * sR[1]) + dz * sR[2]) + slo[0];
-        const double qy = ((dx * sR[3] + dy * sR[4]) + dz * sR[5]) + slo[1];
-        const double qz = ((dx * sR[6] + dy * sR[7]) + dz * sR[8]) + slo[2];
+        const double qx = __dadd_rn(fma(dz, sR[2], fma(dy, sR[1], __dmul_rn(dx, sR[0]))), slo[0]);
+        const double qy = __dadd_rn(fma(dz, sR[5], fma(dy, sR[4], __dmul_rn(dx, sR[3]))), slo[1]);
+        const double qz = __dadd_rn(fma(dz, sR[8], fma(dy, sR[7], __dmul_rn(dx, sR[6]))), slo[2]);
         const int cx = (int)floor((qx - g.org[0]) / g.cell), cy = (int)floor((qy - g.org[1]) / g.cell),
                   cz = (int)floor((qz - g.org[2]) / g.cell);
         if (cx < 0 || cy < 0 || cz < 0 || cx >= g.dims[0] || cy >= g.dims[1] || cz >= g.dims[2]) continue;
@@ -80,7 +104,7 @@ __device__ __forceinline__ int count_pair(const RepeatArgs& a, const CloudArgs& 
                 const int c1 = (ix * g.dims[1] + iy) * g.dims[2] + min(cz + 1, g.dims[2] - 1);
                 for (int s = g.cell_start[c0]; s < g.cell_start[c1 + 1]; ++s) {
                     const double ex = g.lo_sorted[3 * s] - qx, ey = g.lo_sorted[3 * s + 1] - qy, ez = g.lo_sorted[3 * s + 2] - qz;
-                    if (sqrt((ex * ex + ey * ey) + ez * ez) < g.dist) { found = true; break; }
+                    if (sqrt(fma(ez, ez, fma(ey, ey, __dmul_rn(ex, ex)))) < g.dist) { found = true; break; }
                 }
             }
         cnt += found ? 1 : 0;
@@ -112,15 +136,15 @@ repeat_counts_kernel(RepeatArgs a, CloudArgs g, long long p0, int32_t* __restric
 __global__ void __launch_bounds__(128, 8)
 repeat_counts_many_kernel(RepeatArgs a, const long long* __restrict__ pair_off, int G, const MadCloudSeg* __restrict__ segs,
                           const double* __restrict__ hi_clouds, const double* __restrict__ lo_sorted,
-                          const int32_t* __restrict__ cell_start, const uint32_t* __restrict__ near_bits, double dist,
-                          long long p0, int32_t* __restrict__ counts) {
+                          const int32_t* __restrict__ cell_start, const uint32_t* __restrict__ near_bits, double cell,
+                          double dist, long long p0, int32_t* __restrict__ counts) {
     const long long pi = p0 + blockIdx.x;
     const MadCloudSeg& s = segs[mad_segment_of([&](int k) { return pair_off[k]; }, G, pi)];
     CloudArgs g;
     g.hi_cloud = hi_clouds + 3 * s.hi_off; g.H = s.hi_n;
     g.lo_sorted = lo_sorted; g.cell_start = cell_start + s.cell_off; g.near_bits = near_bits + s.word_off;
     for (int q = 0; q < 3; ++q) { g.org[q] = s.org[q]; g.dims[q] = s.dims[q]; }
-    g.cell = dist; g.dist = dist;
+    g.cell = cell; g.dist = dist;
     const int n = count_pair(a, g, pi);
     if (threadIdx.x == 0) counts[blockIdx.x] = n;
 }
@@ -167,6 +191,10 @@ __global__ void mark_used_kernel(const int32_t* __restrict__ idx, long long n, u
 
 }  // namespace
 
+// The cell of the lo grid: a little more than dist, so that no lo point within dist lies outside the 27 cells searched
+// (the argument at the top of this file).
+extern "C" double mad_repeat_grid_cell(double dist) { return dist * (1.0 + 0x1p-16); }
+
 extern "C" int mad_mark_used(const int32_t* idx, long long n, uint8_t* used, void* stream) {
     MAD_CHECK_ARG(n >= 0);
     if (n == 0) return MAD_OK;
@@ -197,7 +225,7 @@ int launch_counts(const RepeatArgs& a, const double* hi_cloud, int n_hi_cloud, c
     CloudArgs g;
     g.hi_cloud = hi_cloud; g.H = n_hi_cloud; g.lo_sorted = lo_sorted; g.cell_start = cell_start; g.near_bits = near_bits;
     for (int q = 0; q < 3; ++q) { g.org[q] = grid_org_host[q]; g.dims[q] = grid_dims_host[q]; }
-    g.cell = dist; g.dist = dist;
+    g.cell = mad_repeat_grid_cell(dist); g.dist = dist;
     MAD_PROF("repeat_counts_kernel", stream);
     repeat_counts_kernel<<<(unsigned)(p1 - p0), 128, 0, (cudaStream_t)stream>>>(a, g, p0, counts, results);
     MAD_LAUNCH_OK();
@@ -296,7 +324,8 @@ int launch_counts_many(const RepeatArgs& a, const long long* pair_off, int G, co
     MAD_CHECK_ARG(pair_off && G >= 1 && segs && hi_clouds && lo_sorted && cell_start && near_bits && dist > 0.0 && counts);
     MAD_PROF("repeat_counts_many_kernel", stream);
     repeat_counts_many_kernel<<<(unsigned)(p1 - p0), 128, 0, (cudaStream_t)stream>>>(a, pair_off, G, segs, hi_clouds, lo_sorted,
-                                                                                    cell_start, near_bits, dist, p0, counts);
+                                                                                    cell_start, near_bits,
+                                                                                    mad_repeat_grid_cell(dist), dist, p0, counts);
     MAD_LAUNCH_OK();
     return MAD_OK;
 }

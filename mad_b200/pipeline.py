@@ -977,6 +977,12 @@ def anchor_cloud(subv, used, cell):
     return c.build_grid()
 
 
+def repeat_grid_cell(dist):
+    """The cell of the lo grid the repeatability kernels search for the distance ``dist``: a little larger than dist
+    (mad_repeat_grid_cell), so that rounding cannot put a lo point within dist outside the 27 cells searched."""
+    return float(_lib.lib.mad_repeat_grid_cell(float(dist)))
+
+
 class DscMatch(object):
     """What ``match_dsc`` computes before the per-pair loop, and what every rank of ``parallel.match_dsc_sharded`` computes
     alike: the pair list above cc (hi, lo, score device tensors, ``p`` pairs), the hi anchor cloud and the lo anchor cloud
@@ -999,8 +1005,9 @@ class DscMatch(object):
         used_lo = torch.zeros(lo.set.rows, dtype=torch.uint8, device=dev)
         call("mad_mark_used", _ptr(self.ph), self.p, _ptr(used_hi), st)
         call("mad_mark_used", _ptr(self.pl), self.p, _ptr(used_lo), st)
-        self.hi_cloud, self.lo_cloud = read_clouds(AnchorCloud(hi.subv, used_hi, self.dist),       # mad/MaD.py:427
-                                                   AnchorCloud(lo.subv, used_lo, self.dist))       # mad/MaD.py:428
+        cell = repeat_grid_cell(self.dist)
+        self.hi_cloud, self.lo_cloud = read_clouds(AnchorCloud(hi.subv, used_hi, cell),            # mad/MaD.py:427
+                                                   AnchorCloud(lo.subv, used_lo, cell))            # mad/MaD.py:428
         self.lo_cloud.build_grid()
         self.tb = device_tables(dev)
 
@@ -1213,9 +1220,10 @@ class DscMatchMany(object):
         self.pair_off_dev = torch.empty(self.G + 1, dtype=torch.int64, device=dev)
         call("mad_mark_used_many", _ptr(self.ph), _ptr(self.pl), self.p, _ptr(row_off), self.G, d_lo, _ptr(used_hi), _ptr(used_lo),
              _ptr(self.pair_off_dev), st)
-        hc = AnchorClouds(self.hi_subv, used_hi, row_off, int(self.hi_row_off[-1]), self.dist)                  # mad/MaD.py:427
+        cell = repeat_grid_cell(self.dist)
+        hc = AnchorClouds(self.hi_subv, used_hi, row_off, int(self.hi_row_off[-1]), cell)                       # mad/MaD.py:427
         lo_off = torch.arange(self.G + 1, dtype=torch.int64, device=dev) * d_lo
-        lc = AnchorClouds(lo.subv, used_lo, lo_off, self.G * d_lo, self.dist, shared_rows=True)                # mad/MaD.py:428
+        lc = AnchorClouds(lo.subv, used_lo, lo_off, self.G * d_lo, cell, shared_rows=True)                     # mad/MaD.py:428
         vals = _Readback.read(self.pair_off_dev, hc.info, lc.info)
         g1 = self.G + 1
         self.pair_off = np.array(vals[:g1], dtype=np.int64)
