@@ -196,6 +196,49 @@ int mad_describe(const float* grad4_oct0, const float* grad4_oct1, const int* di
                  const MadZoneTable* zones16_host, const double* rf_table, const double* rf_inv_table,
                  int rf_zones, int16_t* dsc, void* stream);
 
+/* ---- a5-a12 for a batch of G maps (mad_b200.pipeline.describe_many) ---------------------------------------------
+ * The dense stages and mad_detect run per map; map g's candidates go to rows [g cap, (g + 1) cap) of one candidate
+ * table, counted by counts[g] (device).  The calls below then serve the whole batch, and map g's slice of every output
+ * equals what the single-map call writes for that map alone, bit for bit.  The batch keypoint table holds the maps one
+ * after the other: map g owns rows [kp_off[g], kp_off[g+1]); the oriented table likewise [ori_off[g], ori_off[g+1]),
+ * with MadOriented.kp counted from the map's first keypoint (map-local, as mad_compact_oriented writes it).
+ * dims [G][6] = each map's {nx0,ny0,nz0,nx1,ny1,nz1}; grads_host [G][2] = device addresses of each map's octave
+ * gradients (uint64).  kp_off / ori_off: device int32 [G + 1]; *_host arrays are those values read back.
+ *
+ * mad_sort_keypoints_many: mad_sort_keypoints for every map (n = sum over g of min(counts[g], cap), host value; dims on
+ * the device): out[kp_off[g] ..) = map g's accepted keypoints in canonical order; writes kp_off. */
+size_t mad_sort_keypoints_many_workspace_bytes(int n, int G);
+int mad_sort_keypoints_many(const MadKeypoint* cand, int cap, const int* counts, int G, int n, const int* dims,
+                            MadKeypoint* out, int* kp_off, void* workspace, size_t workspace_bytes, void* stream);
+/* mad_gradient_mark for every keypoint of the batch, in its map's tiles: n_rows (host) >= kp_off[G] CTAs, those at or
+ * beyond kp_off[G] do nothing; dims [G][6] and flags [G][2] (device addresses of each map's octave tile flags) on the
+ * device.  mad_gradient_masked then runs per map and octave. */
+int mad_gradient_mark_many(const MadKeypoint* kp, const int* kp_off, int n_rows, int G, const int* dims,
+                           const uint64_t* flags, int reach_oct0, int reach_oct1, void* stream);
+/* mad_orient for every keypoint of the batch (same device code): n_ori[i] / slots[i*36 ..] for batch row i <
+ * kp_off[G]; n_cand_host[g] (>= map g's keypoints, e.g. its candidate count) sizes the grid.  Maps go 64 to a launch. */
+int mad_orient_many(const uint64_t* grads_host, const int* dims_host, const int* n_cand_host, int G,
+                    const MadKeypoint* kp, const int* kp_off, int r, const MadZoneTable* zones112_host,
+                    const double* r1_table, int lim_main, int lim_sec, int32_t* n_ori, int32_t* slots, void* stream);
+/* mad_compact_oriented over the batch rows [0, kp_off[G]) (n_rows >= kp_off[G], host): oriented[ori_off[g] ..) = map g's
+ * oriented features in emission order; writes ori_off. */
+size_t mad_compact_oriented_many_workspace_bytes(int n_rows);
+int mad_compact_oriented_many(const int32_t* n_ori, const int32_t* slots, int n_rows, const int* kp_off, int G,
+                              MadOriented* oriented, int cap, int* ori_off, void* workspace, size_t workspace_bytes,
+                              void* stream);
+/* mad_describe for every oriented feature of the batch (same device code): dsc[ori_off[g] + j] = map g's descriptor j.
+ * Maps go 64 to a launch. */
+int mad_describe_many(const uint64_t* grads_host, const int* dims_host, const int* kp_off_host, const int* ori_off_host,
+                      int G, const MadKeypoint* kp, const MadOriented* oriented, int r, const MadZoneTable* zones16_host,
+                      const double* rf_table, const double* rf_inv_table, int rf_zones, int16_t* dsc, void* stream);
+/* The FeatureTable columns of n oriented features of G maps (features [ori_off[g], ori_off[g+1]) belong to map g, whose
+ * keypoints start at kp_off[g]): meta[f][4] = (kp, oct, main, sec) and subv[f][3] = the sub-voxel map coordinates of
+ * Detector.find_anchors, from geo [G][5] = (voxel size of octave 0, of octave 1, origin x, y, z) float64, evaluated as
+ *     subv[a] = __dadd_rn(__dmul_rn(__dadd_rn((double)vox[a], (double)off[a]), voxelsp[oct]), origin[a])
+ * i.e. NumPy's (vox + off) * vs + org on int64 vox and float32 off, each operation rounded once, none fused. */
+int mad_feature_meta(const MadKeypoint* kp, const MadOriented* oriented, int n, const int* kp_off, const int* ori_off,
+                     int G, const double* geo, int32_t* meta, double* subv, void* stream);
+
 /* ---- a15: descriptor matching (mad/MaD.py:416-424) ---------------------------------------------- */
 /* A descriptor set prepared for matching (device pointers; the struct itself lives on the host).
  * norm2: exact integer squared L2 norms.  u8: uint8 copy [rows_padded][1024] (zero rows beyond

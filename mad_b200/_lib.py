@@ -89,7 +89,15 @@ SIGNATURES = {
     "mad_compact_oriented_workspace_bytes": (_SZ, [_I]),
     "mad_compact_oriented": (_I, [_P, _P, _I, _P, _I, _P, _P, _SZ, _P]),
     "mad_describe": (_I, [_P, _P, _P, _P, _P, _I, _I, C.POINTER(MadZoneTable), _P, _P, _I, _P, _P]),
-    "mad_dsc_prepare": (_I, [_P, _I, _I, _P, _P, _P, _P, _P, _P]),
+    "mad_sort_keypoints_many_workspace_bytes": (_SZ, [_I, _I]),
+    "mad_sort_keypoints_many": (_I, [_P, _I, _P, _I, _I, _P, _P, _P, _P, _SZ, _P]),
+    "mad_gradient_mark_many": (_I, [_P, _P, _I, _I, _P, _P, _I, _I, _P]),
+    "mad_orient_many": (_I, [_P, _P, _P, _I, _P, _P, _I, C.POINTER(MadZoneTable), _P, _I, _I, _P, _P, _P]),
+    "mad_compact_oriented_many_workspace_bytes": (_SZ, [_I]),
+    "mad_compact_oriented_many": (_I, [_P, _P, _I, _P, _I, _P, _I, _P, _P, _SZ, _P]),
+    "mad_describe_many": (_I, [_P, _P, _P, _P, _I, _P, _P, _I, C.POINTER(MadZoneTable), _P, _P, _I, _P, _P]),
+    "mad_feature_meta": (_I, [_P, _P, _I, _P, _P, _I, _P, _P, _P, _P]),
+    "mad_dsc_prepare":(_I, [_P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mad_match_pairs": (_I, [C.POINTER(MadDscSet), C.POINTER(MadDscSet), C.c_double, _P, _P, C.c_uint64, _P, _P]),
     "mad_match_pairs_finish_workspace_bytes": (_SZ, [C.c_longlong]),
     "mad_match_pairs_finish": (_I, [_P, _P, C.c_longlong, _I, _I, _P, _P, _P, _P, _P, _P, _SZ, _P]),

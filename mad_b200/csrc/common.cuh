@@ -51,6 +51,40 @@ __host__ __device__ __forceinline__ int mad_segment_of(Off off, int G, long long
 
 int mad_sm_count();
 
+// ---- per-map arguments of the batched orientation / description launches (mad_orient_many, mad_describe_many) ----
+// The table travels as one __grid_constant__ kernel parameter, so every read of it is a constant-bank operand, as the
+// single-map kernels' own arguments are; a batch of more maps is split into launches of kMadBatchMaps maps.
+constexpr int kMadBatchMaps = 64;
+struct MadBatchMap {
+    const float4* grad[2];  // gradient of octave 0 / 1
+    int n[2][3];            // dims of octave 0 / 1
+    int kp0;                // first row of the map in the batch keypoint table
+    int row0;               // mad_describe_many: first oriented feature of the map, counted from the launch's first map
+};
+struct MadBatchMaps {
+    static constexpr bool kMaps = true;
+    const int* kp_off;      // mad_orient_many: the batch's kp_off from the launch's first map on (device)
+    int G, pad;             // maps of this launch
+    MadBatchMap m[kMadBatchMaps];
+};
+
+// The table of the maps [g0, g0 + G) (G <= kMadBatchMaps) from the host arrays of a batched call: grads_host [][2]
+// device addresses, dims_host [][6], and (may be NULL) kp_off_host / ori_off_host [] the batch offsets.
+static inline void mad_batch_maps(MadBatchMaps& t, int g0, int G, const uint64_t* grads_host, const int* dims_host,
+                                  const int* kp_off_host, const int* ori_off_host) {
+    t.G = G;
+    t.pad = 0;
+    for (int i = 0; i < G; ++i) {
+        MadBatchMap& m = t.m[i];
+        for (int o = 0; o < 2; ++o) {
+            m.grad[o] = reinterpret_cast<const float4*>(grads_host[2 * (g0 + i) + o]);
+            for (int a = 0; a < 3; ++a) m.n[o][a] = dims_host[6 * (g0 + i) + 3 * o + a];
+        }
+        m.kp0 = kp_off_host ? kp_off_host[g0 + i] : 0;
+        m.row0 = ori_off_host ? ori_off_host[g0 + i] - ori_off_host[g0] : 0;
+    }
+}
+
 // ---- launch accounting / optional per-kernel CUDA-event timing (mad_profile_*, api.cu) ----------
 // Every kernel launch site of the library opens a MadProfScope: it always counts the launch
 // (mad_launch_count) and, while profiling is enabled, brackets it with two events recorded on

@@ -7,12 +7,19 @@
 // float64, classified into the 16 EQSP zones (highest passing index wins, unassigned -> zone 0)
 // and counted per 4x4x4 sub-block in a shared-memory histogram; the int16[1024] row is written
 // with coalesced stores.  Any sample outside the grid zeroes the whole descriptor (:140-149).
+#include <algorithm>
+
 #include "common.cuh"
 #include "eqsp_zones.cuh"
 
 namespace {
 
 struct OctDims { int n[2][3]; };
+
+// The batch form of describe_kernel (mad_describe_many) takes its per-map arguments from a MadBatchMaps table, passed as
+// the last parameter; the single-map form passes NoBatch there and reads its own grad / dims parameters.  Both forms
+// run one body.
+struct NoBatch { static constexpr bool kMaps = false; };
 
 // scipy _rgi nearest rule: i = clip(floor(p), 0, n-2); idx = (p - i <= .5) ? i : i + 1 -- a half rounds
 // DOWN.  For p in [0, n-1] (guaranteed by the bounds vote) this is exactly ceil(p - 0.5): p - 0.5 is
@@ -41,22 +48,31 @@ __device__ __noinline__ int zone_exact_dsc(ZoneTab T, const double* __restrict__
 
 // SIDE = 2 r known at compile time (16 for the default patch: one lattice column per thread, no tail tests) or 0 for
 // any other radius.
-template <int NB, int SIDE, int THREADS>
+template <int NB, int SIDE, int THREADS, class Batch>
 __global__ void __launch_bounds__(THREADS, 768 / THREADS)
 describe_kernel(const float4* __restrict__ grad0, const float4* __restrict__ grad1, OctDims dims,
                 const MadKeypoint* __restrict__ kp, const MadOriented* __restrict__ oriented, int r,
                 ZoneTab T, const double* __restrict__ rf_table, const double* __restrict__ rf_inv_table,
-                int rf_zones, int16_t* __restrict__ dsc) {
+                int rf_zones, int16_t* __restrict__ dsc, const __grid_constant__ Batch batch) {
     __shared__ int cnt[MAD_DSC_LEN];
     __shared__ ZoneFast F;
     __shared__ double xt[32][3];           // lx * Ri[0], lx * Ri[3], lx * Ri[6] for the 2 r values of lx
     const int tid = threadIdx.x;
     if (SIDE) r = SIDE / 2;
     const MadOriented of = oriented[blockIdx.x];
-    const MadKeypoint K = kp[of.kp];
+    int row = of.kp, g = 0;
+    if constexpr (Batch::kMaps) {          // feature b of the launch is in the map g with row0 <= b; kp counts from kp0
+        g = mad_segment_of([&](int k) { return batch.m[k].row0; }, batch.G, blockIdx.x);
+        row += batch.m[g].kp0;
+    }
+    const MadKeypoint K = kp[row];
     const int o = K.oct ? 1 : 0;
     const float4* __restrict__ grad = o ? grad1 : grad0;
-    const int nx = dims.n[o][0], ny = dims.n[o][1], nz = dims.n[o][2];
+    int nx = dims.n[o][0], ny = dims.n[o][1], nz = dims.n[o][2];
+    if constexpr (Batch::kMaps) {
+        grad = batch.m[g].grad[o];
+        nx = batch.m[g].n[o][0]; ny = batch.m[g].n[o][1]; nz = batch.m[g].n[o][2];
+    }
     const long long tab = ((long long)of.main_bin * rf_zones + of.sec_bin) * 9;
     double Ri[9];
     float Rmf[9];
@@ -165,6 +181,39 @@ describe_kernel(const float4* __restrict__ grad0, const float4* __restrict__ gra
 
 }  // namespace
 
+// mad_describe's own per-map arguments (unused by the batch form).
+struct OneMapArgs {
+    const float4* grad0 = nullptr;
+    const float4* grad1 = nullptr;
+    OctDims dims = {};
+};
+
+// One describe_kernel launch of `ctas` CTAs: the checks and the kernel choice of mad_describe, shared by
+// mad_describe_many.
+template <class Batch>
+static int launch_describe(const OneMapArgs& d, const Batch& batch, unsigned ctas, const MadKeypoint* kp, const MadOriented* oriented, int r,
+                           const MadZoneTable* zones_host, const double* rf_table, const double* rf_inv_table, int rf_zones,
+                           int16_t* dsc, void* stream) {
+    MAD_CHECK_ARG(zones_host->n_zones * 64 == MAD_DSC_LEN);   // 64 sub-blocks x 16 zones
+    MAD_CHECK_ARG(r >= 2 && r <= 16 && rf_zones > 0);
+    ZoneTab T;
+    T.bounds = zones_host->bounds; T.belt_first = zones_host->belt_first; T.belt_phi = zones_host->belt_phi;
+    T.n_zones = zones_host->n_zones; T.n_belts = zones_host->n_belts; T.fast = zones_host->fast;
+    MAD_CHECK_ARG(T.n_belts >= 1 && T.n_belts <= MAD_BELT_MAX && T.n_zones <= MAD_ZONE_MAX);
+    MAD_PROF("describe_kernel", stream);
+    auto launch = [&](auto kernel, int threads) {
+        kernel<<<ctas, threads, 0, (cudaStream_t)stream>>>(d.grad0, d.grad1, d.dims, kp, oriented, r, T, rf_table, rf_inv_table,
+                                                           rf_zones, dsc, batch);
+    };
+    // 128-thread CTAs (two lattice columns per thread, 6 CTAs per SM) measured 0.93 ms at C2 against 1.04 ms with 256
+    // threads and 1.01 ms with 64: smaller CTAs lose less time at the two barriers of a feature
+    if (T.n_belts <= 4 && r == 8) launch(describe_kernel<4, 16, 128, Batch>, 128);  // default: 16 zones (caps + 2 belts), patch 16
+    else if (T.n_belts <= 4) launch(describe_kernel<4, 0, 256, Batch>, 256);
+    else launch(describe_kernel<MAD_BELT_MAX, 0, 256, Batch>, 256);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}
+
 extern "C" int mad_describe(const float* grad4_oct0, const float* grad4_oct1, const int* dims_oct_host,
                             const MadKeypoint* kp, const MadOriented* oriented, int n_oriented, int r,
                             const MadZoneTable* zones_host, const double* rf_table, const double* rf_inv_table,
@@ -172,27 +221,38 @@ extern "C" int mad_describe(const float* grad4_oct0, const float* grad4_oct1, co
     MAD_CHECK_ARG(dims_oct_host && zones_host && n_oriented >= 0);
     if (n_oriented == 0) return MAD_OK;
     MAD_CHECK_ARG(grad4_oct0 && grad4_oct1 && kp && oriented && rf_table && rf_inv_table && dsc);
-    MAD_CHECK_ARG(zones_host->n_zones * 64 == MAD_DSC_LEN);   // 64 sub-blocks x 16 zones
-    MAD_CHECK_ARG(r >= 2 && r <= 16 && rf_zones > 0);
-    OctDims d;
-    for (int o = 0; o < 2; ++o) for (int a = 0; a < 3; ++a) d.n[o][a] = dims_oct_host[3 * o + a];
-    ZoneTab T;
-    T.bounds = zones_host->bounds; T.belt_first = zones_host->belt_first; T.belt_phi = zones_host->belt_phi;
-    T.n_zones = zones_host->n_zones; T.n_belts = zones_host->n_belts; T.fast = zones_host->fast;
-    MAD_CHECK_ARG(T.n_belts >= 1 && T.n_belts <= MAD_BELT_MAX && T.n_zones <= MAD_ZONE_MAX);
-    MAD_PROF("describe_kernel", stream);
+    OneMapArgs d;
+    d.grad0 = reinterpret_cast<const float4*>(grad4_oct0);
+    d.grad1 = reinterpret_cast<const float4*>(grad4_oct1);
+    for (int o = 0; o < 2; ++o) for (int a = 0; a < 3; ++a) d.dims.n[o][a] = dims_oct_host[3 * o + a];
     for (int o = 0; o < 2; ++o)                                  // 32-bit voxel indices in the gather
-        MAD_CHECK_ARG((long long)d.n[o][0] * d.n[o][1] * d.n[o][2] < (1LL << 31));
-    auto launch = [&](auto kernel, int threads) {
-        kernel<<<n_oriented, threads, 0, (cudaStream_t)stream>>>(
-            reinterpret_cast<const float4*>(grad4_oct0), reinterpret_cast<const float4*>(grad4_oct1), d, kp, oriented, r,
-            T, rf_table, rf_inv_table, rf_zones, dsc);
-    };
-    // 128-thread CTAs (two lattice columns per thread, 6 CTAs per SM) measured 0.93 ms at C2 against 1.04 ms with 256
-    // threads and 1.01 ms with 64: smaller CTAs lose less time at the two barriers of a feature
-    if (T.n_belts <= 4 && r == 8) launch(describe_kernel<4, 16, 128>, 128);        // default: 16 zones (caps + 2 belts), patch 16
-    else if (T.n_belts <= 4) launch(describe_kernel<4, 0, 256>, 256);
-    else launch(describe_kernel<MAD_BELT_MAX, 0, 256>, 256);
-    MAD_LAUNCH_OK();
+        MAD_CHECK_ARG((long long)d.dims.n[o][0] * d.dims.n[o][1] * d.dims.n[o][2] < (1LL << 31));
+    return launch_describe(d, NoBatch(), (unsigned)n_oriented, kp, oriented, r, zones_host, rf_table, rf_inv_table, rf_zones, dsc, stream);
+}
+
+extern "C" int mad_describe_many(const uint64_t* grads_host, const int* dims_host, const int* kp_off_host,
+                                 const int* ori_off_host, int G, const MadKeypoint* kp, const MadOriented* oriented, int r,
+                                 const MadZoneTable* zones_host, const double* rf_table, const double* rf_inv_table,
+                                 int rf_zones, int16_t* dsc, void* stream) {
+    MAD_CHECK_ARG(grads_host && dims_host && kp_off_host && ori_off_host && zones_host && G >= 1);
+    MAD_CHECK_ARG(ori_off_host[0] == 0);
+    for (int g = 0; g < G; ++g) {
+        MAD_CHECK_ARG(ori_off_host[g + 1] >= ori_off_host[g] && kp_off_host[g + 1] >= kp_off_host[g]);
+        for (int o = 0; o < 2; ++o)                              // 32-bit voxel indices in the gather
+            MAD_CHECK_ARG((long long)dims_host[6 * g + 3 * o] * dims_host[6 * g + 3 * o + 1] * dims_host[6 * g + 3 * o + 2] < (1LL << 31));
+    }
+    if (ori_off_host[G] == 0) return MAD_OK;
+    MAD_CHECK_ARG(kp && oriented && rf_table && rf_inv_table && dsc);
+    for (int g0 = 0; g0 < G; g0 += kMadBatchMaps) {
+        const int cnt = std::min(kMadBatchMaps, G - g0);
+        const int d0 = ori_off_host[g0], d = ori_off_host[g0 + cnt] - d0;
+        if (d == 0) continue;
+        MadBatchMaps t;
+        mad_batch_maps(t, g0, cnt, grads_host, dims_host, kp_off_host, ori_off_host);
+        t.kp_off = nullptr;
+        const int rc = launch_describe(OneMapArgs(), t, (unsigned)d, kp, oriented + d0, r, zones_host, rf_table, rf_inv_table, rf_zones,
+                                       dsc + (long long)d0 * MAD_DSC_LEN, stream);
+        if (rc != MAD_OK) return rc;
+    }
     return MAD_OK;
 }

@@ -310,3 +310,166 @@ extern "C" int mad_sort_keypoints(const MadKeypoint* cand, int n, const int* dim
     MAD_LAUNCH_OK();
     return MAD_OK;
 }
+
+// ---- a batch of G maps (mad_b200.pipeline.describe_many) ------------------------------------------------------------
+namespace {
+
+// cand_off[g] = candidates of the maps before g (each count clamped to cap), g = 0..G: one CTA.
+__global__ void __launch_bounds__(256) cand_offsets_kernel(const int* __restrict__ counts, int G, int cap,
+                                                           int* __restrict__ cand_off) {
+    typedef cub::BlockScan<int, 256> Scan;
+    __shared__ typename Scan::TempStorage tmp;
+    int carry = 0;
+    for (int g0 = 0; g0 < G; g0 += 256) {
+        const int g = g0 + threadIdx.x;
+        const int v = g < G ? min(counts[g], cap) : 0;
+        int ex, total;
+        Scan(tmp).ExclusiveSum(v, ex, total);
+        if (g < G) cand_off[g] = carry + ex;
+        carry += total;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) cand_off[G] = carry;
+}
+
+// The key of mad_sort_keypoints (build_keys_kernel) for candidate j of the packed batch, with its map's dims; the map
+// order comes from the segments of the sort.  idx = the candidate's row in cand (map g's region starts at g cap).
+__global__ void build_keys_many_kernel(const MadKeypoint* __restrict__ cand, int cap, const int* __restrict__ cand_off, int G,
+                                       const int* __restrict__ dims, unsigned long long* __restrict__ keys,
+                                       int* __restrict__ idx) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= cand_off[G]) return;
+    const int g = mad_segment_of([&](int k) { return cand_off[k]; }, G, j);
+    const int row = g * cap + (j - cand_off[g]);
+    const MadKeypoint k = cand[row];
+    const int* d = dims + 6 * g;
+    const int ny = k.oct ? d[4] : d[1], nz = k.oct ? d[5] : d[2];
+    const unsigned long long raster = ((unsigned long long)k.peak[0] * ny + k.peak[1]) * nz + k.peak[2];
+    const unsigned int vb = 0x7FFFFFFFu - (__float_as_uint(k.val) & 0x7FFFFFFFu);  // value descending
+    keys[j] = ((unsigned long long)(k.oct & 1) << 63) | ((unsigned long long)vb << 32) | (raster & 0xFFFFFFFFull);
+    idx[j] = row;
+}
+
+__global__ void flags_many_kernel(const MadKeypoint* __restrict__ cand, const int* __restrict__ order, int n,
+                                  int* __restrict__ flags) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i <= n) flags[i] = i < n ? cand[order[i]].accepted : 0;
+}
+
+__global__ void scatter_many_kernel(const MadKeypoint* __restrict__ cand, const int* __restrict__ order,
+                                    const int* __restrict__ flags, const int* __restrict__ pos, int n,
+                                    const int* __restrict__ cand_off, int G, MadKeypoint* __restrict__ out,
+                                    int* __restrict__ kp_off) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i <= G) kp_off[i] = pos[cand_off[i]];
+    if (i < n && flags[i]) out[pos[i]] = cand[order[i]];
+}
+
+struct SortManyLayout {
+    size_t keys_in, keys_out, idx_in, idx_out, flags, pos, cand_off, cub, total;
+};
+
+SortManyLayout sort_many_layout(int n, int G) {
+    SortManyLayout l;
+    size_t o = 0;
+    auto take = [&](size_t bytes) { size_t r = o; o += mad_align_up(bytes, 256); return r; };
+    const size_t nn = (size_t)(n > 0 ? n : 1);
+    l.keys_in = take(nn * 8); l.keys_out = take(nn * 8);
+    l.idx_in = take(nn * 4); l.idx_out = take(nn * 4);
+    l.flags = take((nn + 1) * 4); l.pos = take((nn + 1) * 4);
+    l.cand_off = take((size_t)(G + 1) * 4);
+    size_t a = 0, b = 0;
+    cub::DeviceSegmentedSort::StableSortPairs(nullptr, a, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                              (const int*)nullptr, (int*)nullptr, (int)nn, G, (const int*)nullptr,
+                                              (const int*)nullptr);
+    cub::DeviceScan::ExclusiveSum(nullptr, b, (const int*)nullptr, (int*)nullptr, (int)nn + 1);
+    l.cub = take(a > b ? a : b);
+    l.total = o;
+    return l;
+}
+
+// subv of mad_feature_meta, the float64 operations of Detector.find_anchors one by one (no contraction).
+__global__ void feature_meta_kernel(const MadKeypoint* __restrict__ kp, const MadOriented* __restrict__ oriented, int n,
+                                    const int* __restrict__ kp_off, const int* __restrict__ ori_off, int G,
+                                    const double* __restrict__ geo, int32_t* __restrict__ meta, double* __restrict__ subv) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= n) return;
+    const int g = mad_segment_of([&](int k) { return ori_off[k]; }, G, f);
+    const MadOriented of = oriented[f];
+    const MadKeypoint K = kp[kp_off[g] + of.kp];
+    const double* q = geo + 5 * g;
+    const double vs = q[K.oct ? 1 : 0];
+    meta[4 * (long long)f + 0] = of.kp;
+    meta[4 * (long long)f + 1] = K.oct;
+    meta[4 * (long long)f + 2] = of.main_bin;
+    meta[4 * (long long)f + 3] = of.sec_bin;
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+        subv[3 * (long long)f + a] = __dadd_rn(__dmul_rn(__dadd_rn((double)K.vox[a], (double)K.off[a]), vs), q[2 + a]);
+}
+
+}  // namespace
+
+extern "C" size_t mad_sort_keypoints_many_workspace_bytes(int n, int G) { return sort_many_layout(n, G).total; }
+
+extern "C" int mad_sort_keypoints_many(const MadKeypoint* cand, int cap, const int* counts, int G, int n, const int* dims,
+                                       MadKeypoint* out, int* kp_off, void* workspace, size_t workspace_bytes, void* stream) {
+    MAD_CHECK_ARG(cand && counts && dims && kp_off && workspace && G >= 1 && cap >= 1 && n >= 0);
+    MAD_CHECK_ARG((long long)G * cap < (1LL << 31) && n <= (long long)G * cap);
+    MAD_CHECK_ARG(n == 0 || out);
+    const SortManyLayout l = sort_many_layout(n, G);
+    MAD_CHECK_ARG(workspace_bytes >= l.total);
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = reinterpret_cast<char*>(workspace);
+    auto* keys_in = reinterpret_cast<unsigned long long*>(ws + l.keys_in);
+    auto* keys_out = reinterpret_cast<unsigned long long*>(ws + l.keys_out);
+    int* idx_in = reinterpret_cast<int*>(ws + l.idx_in);
+    int* idx_out = reinterpret_cast<int*>(ws + l.idx_out);
+    int* flags = reinterpret_cast<int*>(ws + l.flags);
+    int* pos = reinterpret_cast<int*>(ws + l.pos);
+    int* cand_off = reinterpret_cast<int*>(ws + l.cand_off);
+    {
+        MAD_PROF("cand_offsets_kernel", st);
+        cand_offsets_kernel<<<1, 256, 0, st>>>(counts, G, cap, cand_off);
+        MAD_LAUNCH_OK();
+    }
+    const int tb = 256, nb = (int)mad_ceil_div(n + 1, tb);
+    if (n > 0) {
+        {
+            MAD_PROF("build_keys_many_kernel", st);
+            build_keys_many_kernel<<<nb, tb, 0, st>>>(cand, cap, cand_off, G, dims, keys_in, idx_in);
+            MAD_LAUNCH_OK();
+        }
+        size_t cub_bytes = l.total - l.cub;
+        MAD_PROF("cub_segmented_sort_pairs", st);
+        MAD_CUDA(cub::DeviceSegmentedSort::StableSortPairs(ws + l.cub, cub_bytes, keys_in, keys_out, idx_in, idx_out, n, G,
+                                                           cand_off, cand_off + 1, st));
+    }
+    {
+        MAD_PROF("flags_many_kernel", st);
+        flags_many_kernel<<<nb, tb, 0, st>>>(cand, idx_out, n, flags);
+        MAD_LAUNCH_OK();
+    }
+    {
+        size_t cub_bytes = l.total - l.cub;
+        MAD_PROF("cub_exclusive_sum", st);
+        MAD_CUDA(cub::DeviceScan::ExclusiveSum(ws + l.cub, cub_bytes, flags, pos, n + 1, st));
+    }
+    MAD_PROF("scatter_many_kernel", st);
+    scatter_many_kernel<<<(int)mad_ceil_div(std::max(n, G + 1), tb), tb, 0, st>>>(cand, idx_out, flags, pos, n, cand_off, G, out,
+                                                                                 kp_off);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}
+
+extern "C" int mad_feature_meta(const MadKeypoint* kp, const MadOriented* oriented, int n, const int* kp_off,
+                                const int* ori_off, int G, const double* geo, int32_t* meta, double* subv, void* stream) {
+    MAD_CHECK_ARG(kp_off && ori_off && geo && G >= 1 && n >= 0);
+    if (n == 0) return MAD_OK;
+    MAD_CHECK_ARG(kp && oriented && meta && subv);
+    MAD_PROF("feature_meta_kernel", stream);
+    feature_meta_kernel<<<(int)mad_ceil_div(n, 256), 256, 0, (cudaStream_t)stream>>>(kp, oriented, n, kp_off, ori_off, G, geo,
+                                                                                  meta, subv);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}

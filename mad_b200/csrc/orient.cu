@@ -16,6 +16,11 @@ namespace {
 
 struct OctDims { int n[2][3]; };
 
+// The batch form of the kernels below (mad_orient_many) takes its per-map arguments from a MadBatchMaps table, passed as
+// the last parameter; the single-map form passes NoBatch there and reads its own grad / dims parameters.  Both forms
+// run one body.
+struct NoBatch { static constexpr bool kMaps = false; };
+
 __device__ __forceinline__ int norm50(int h, int hmax) {
     return (int)((double)h / (double)hmax * 50.0);   // np.array(h / max * 50, dtype=int32)
 }
@@ -80,12 +85,12 @@ __device__ __forceinline__ int select_zones(bool flag, int zone, int* out, int* 
     return total;
 }
 
-template <int NB>
+template <int NB, class Batch>
 __global__ void __launch_bounds__(128)
 orient_kernel(const float4* __restrict__ grad0, const float4* __restrict__ grad1, OctDims dims,
               const MadKeypoint* __restrict__ kp, int r, const char4* __restrict__ mask_off, int n_mask,
               ZoneTab T, const double* __restrict__ r1_table, int lim_main, int lim_sec,
-              int32_t* __restrict__ n_ori, int32_t* __restrict__ slots) {
+              int32_t* __restrict__ n_ori, int32_t* __restrict__ slots, const __grid_constant__ Batch batch) {
     extern __shared__ float4 pv[];     // [n_mask] RAW gradient (x, y, z) + w: 1/|g| (fast normalisation),
                                        //          0 = no vote (|g| < 1e-5), -1 = |g| == 1e-5 exactly (exact path only)
     __shared__ int hist[128];
@@ -96,11 +101,20 @@ orient_kernel(const float4* __restrict__ grad0, const float4* __restrict__ grad1
     __shared__ ZoneFast F;
 
     const int tid = threadIdx.x;
-    const int ki = blockIdx.x;
+    int ki = blockIdx.x, g = 0;
+    if constexpr (Batch::kMaps) {          // keypoint kp_off[0] + b of the batch; none at or beyond kp_off[G]
+        ki += batch.kp_off[0];
+        if (ki >= batch.kp_off[batch.G]) return;
+        g = mad_segment_of([&](int k) { return batch.kp_off[k]; }, batch.G, ki);
+    }
     const MadKeypoint K = kp[ki];
     const int o = K.oct ? 1 : 0;
     const float4* __restrict__ grad = o ? grad1 : grad0;
-    const int nx = dims.n[o][0], ny = dims.n[o][1], nz = dims.n[o][2];
+    int nx = dims.n[o][0], ny = dims.n[o][1], nz = dims.n[o][2];
+    if constexpr (Batch::kMaps) {
+        grad = batch.m[g].grad[o];
+        nx = batch.m[g].n[o][0]; ny = batch.m[g].n[o][1]; nz = batch.m[g].n[o][2];
+    }
     const int s = o ? 1 : 2;
     const int cx = K.vox[0], cy = K.vox[1], cz = K.vox[2];
     // border rejection of mad/Orientator.py:129-135,149-155 (uniform over the CTA)
@@ -282,6 +296,46 @@ static int ensure_mask(int r, const char4** dev, int* count) {
     return MAD_OK;
 }
 
+// mad_orient's own per-map arguments (unused by the batch form).
+struct OneMapArgs {
+    const float4* grad0 = nullptr;
+    const float4* grad1 = nullptr;
+    OctDims dims = {};
+};
+
+// One orient_kernel launch of `ctas` CTAs: the checks and the kernel choice of mad_orient, shared by mad_orient_many.
+template <class Batch>
+static int launch_orient(const char* what, const OneMapArgs& d, const Batch& batch, unsigned ctas, const MadKeypoint* kp, int r,
+                         const MadZoneTable* zones_host, const double* r1_table, int lim_main, int lim_sec,
+                         int32_t* n_ori, int32_t* slots, void* stream) {
+    MAD_CHECK_ARG(zones_host->n_zones >= 3 && zones_host->n_zones <= 128 && zones_host->n_belts < 32);
+    MAD_CHECK_ARG(lim_main >= 0 && lim_main <= 6 && lim_sec >= 0 && lim_sec <= 6);
+    const char4* mask = nullptr;
+    int n_mask = 0;
+    int rc = ensure_mask(r, &mask, &n_mask);
+    if (rc != MAD_OK) { mad_set_error("%s: cannot build the spherical mask for r=%d", what, r); return rc; }
+    ZoneTab T;
+    T.bounds = zones_host->bounds; T.belt_first = zones_host->belt_first; T.belt_phi = zones_host->belt_phi;
+    T.n_zones = zones_host->n_zones; T.n_belts = zones_host->n_belts; T.fast = zones_host->fast;
+    const size_t smem = (size_t)n_mask * sizeof(float4);
+    if (smem > 200 * 1024) { mad_set_error("%s: patch radius %d too large", what, r); return MAD_ERR_ARG; }
+    MAD_CHECK_ARG(T.n_belts >= 1 && T.n_belts <= MAD_BELT_MAX && T.n_zones <= MAD_ZONE_MAX);
+    auto launch = [&](auto kernel) -> int {
+        MAD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
+        MAD_PROF("orient_kernel", stream);
+        kernel<<<ctas, 128, smem, (cudaStream_t)stream>>>(      // 64 / 256 threads measured 0.75 / 0.53 ms against 0.50 at C2
+            d.grad0, d.grad1, d.dims, kp, r, mask, n_mask, T, r1_table, lim_main, lim_sec, n_ori, slots, batch);
+        return MAD_OK;
+    };
+    int lrc;
+    if (T.n_belts <= 4) lrc = launch(orient_kernel<4, Batch>);
+    else if (T.n_belts <= 12) lrc = launch(orient_kernel<12, Batch>);    // the 112-zone table has 10 belts
+    else lrc = launch(orient_kernel<MAD_BELT_MAX, Batch>);
+    if (lrc != MAD_OK) return lrc;
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}
+
 extern "C" int mad_orient(const float* grad4_oct0, const float* grad4_oct1, const int* dims_oct_host,
                           const MadKeypoint* kp, int n_kp, int r, const MadZoneTable* zones_host,
                           const double* r1_table, int lim_main, int lim_sec, int32_t* n_ori, int32_t* slots,
@@ -289,35 +343,35 @@ extern "C" int mad_orient(const float* grad4_oct0, const float* grad4_oct1, cons
     MAD_CHECK_ARG(dims_oct_host && zones_host && r1_table && n_kp >= 0);
     if (n_kp == 0) return MAD_OK;
     MAD_CHECK_ARG(grad4_oct0 && grad4_oct1 && kp && n_ori && slots);
-    MAD_CHECK_ARG(zones_host->n_zones >= 3 && zones_host->n_zones <= 128 && zones_host->n_belts < 32);
-    MAD_CHECK_ARG(lim_main >= 0 && lim_main <= 6 && lim_sec >= 0 && lim_sec <= 6);
-    const char4* mask = nullptr;
-    int n_mask = 0;
-    int rc = ensure_mask(r, &mask, &n_mask);
-    if (rc != MAD_OK) { mad_set_error("mad_orient: cannot build the spherical mask for r=%d", r); return rc; }
-    OctDims d;
-    for (int o = 0; o < 2; ++o) for (int a = 0; a < 3; ++a) d.n[o][a] = dims_oct_host[3 * o + a];
-    ZoneTab T;
-    T.bounds = zones_host->bounds; T.belt_first = zones_host->belt_first; T.belt_phi = zones_host->belt_phi;
-    T.n_zones = zones_host->n_zones; T.n_belts = zones_host->n_belts; T.fast = zones_host->fast;
-    const size_t smem = (size_t)n_mask * sizeof(float4);
-    if (smem > 200 * 1024) { mad_set_error("mad_orient: patch radius %d too large", r); return MAD_ERR_ARG; }
-    MAD_CHECK_ARG(T.n_belts >= 1 && T.n_belts <= MAD_BELT_MAX && T.n_zones <= MAD_ZONE_MAX);
-    auto launch = [&](auto kernel) -> int {
-        MAD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
-        MAD_PROF("orient_kernel", stream);
-        kernel<<<n_kp, 128, smem, (cudaStream_t)stream>>>(      // 64 / 256 threads measured 0.75 / 0.53 ms against 0.50 at C2
+    OneMapArgs d;
+    d.grad0 = reinterpret_cast<const float4*>(grad4_oct0);
+    d.grad1 = reinterpret_cast<const float4*>(grad4_oct1);
+    for (int o = 0; o < 2; ++o) for (int a = 0; a < 3; ++a) d.dims.n[o][a] = dims_oct_host[3 * o + a];
+    return launch_orient("mad_orient", d, NoBatch(), (unsigned)n_kp, kp, r, zones_host, r1_table, lim_main, lim_sec, n_ori, slots, stream);
+}
 
-            reinterpret_cast<const float4*>(grad4_oct0), reinterpret_cast<const float4*>(grad4_oct1), d, kp, r, mask,
-            n_mask, T, r1_table, lim_main, lim_sec, n_ori, slots);
-        return MAD_OK;
-    };
-    int lrc;
-    if (T.n_belts <= 4) lrc = launch(orient_kernel<4>);
-    else if (T.n_belts <= 12) lrc = launch(orient_kernel<12>);    // the 112-zone table has 10 belts
-    else lrc = launch(orient_kernel<MAD_BELT_MAX>);
-    if (lrc != MAD_OK) return lrc;
-    MAD_LAUNCH_OK();
+extern "C" int mad_orient_many(const uint64_t* grads_host, const int* dims_host, const int* n_cand_host, int G,
+                               const MadKeypoint* kp, const int* kp_off, int r, const MadZoneTable* zones_host,
+                               const double* r1_table, int lim_main, int lim_sec, int32_t* n_ori, int32_t* slots,
+                               void* stream) {
+    MAD_CHECK_ARG(grads_host && dims_host && n_cand_host && zones_host && r1_table && G >= 1);
+    MAD_CHECK_ARG(kp && kp_off && n_ori && slots);
+    for (int g0 = 0; g0 < G; g0 += kMadBatchMaps) {
+        const int cnt = std::min(kMadBatchMaps, G - g0);
+        long long ctas = 0;                              // the candidates of these maps bound their keypoints
+        for (int i = 0; i < cnt; ++i) {
+            MAD_CHECK_ARG(n_cand_host[g0 + i] >= 0);
+            ctas += n_cand_host[g0 + i];
+        }
+        MAD_CHECK_ARG(ctas < (1LL << 31));
+        if (ctas == 0) continue;
+        MadBatchMaps t;
+        mad_batch_maps(t, g0, cnt, grads_host, dims_host, nullptr, nullptr);
+        t.kp_off = kp_off + g0;
+        const int rc = launch_orient("mad_orient_many", OneMapArgs(), t, (unsigned)ctas, kp, r, zones_host, r1_table, lim_main, lim_sec,
+                                     n_ori, slots, stream);
+        if (rc != MAD_OK) return rc;
+    }
     return MAD_OK;
 }
 
@@ -369,6 +423,73 @@ extern "C" int mad_compact_oriented(const int32_t* n_ori, const int32_t* slots, 
     }
     MAD_PROF("compact_oriented_kernel", st);
     compact_oriented_kernel<<<(int)mad_ceil_div(n_kp, 256), 256, 0, st>>>(n_ori, slots, pos, n_kp, oriented, cap, out_count);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}
+
+namespace {
+
+// The scan input of mad_compact_oriented_many: n_ori of the batch's keypoints, 0 for the rows [kp_off[G], n_rows].
+__global__ void ori_counts_many_kernel(const int32_t* __restrict__ n_ori, const int* __restrict__ kp_off, int G, int n_rows,
+                                       int* __restrict__ cnt) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i <= n_rows) cnt[i] = i < kp_off[G] ? n_ori[i] : 0;
+}
+
+__global__ void compact_oriented_many_kernel(const int32_t* __restrict__ n_ori, const int32_t* __restrict__ slots,
+                                             const int* __restrict__ pos, const int* __restrict__ kp_off, int G,
+                                             MadOriented* __restrict__ out, int cap, int* __restrict__ ori_off) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i <= G) ori_off[i] = pos[kp_off[i]];
+    if (i >= kp_off[G]) return;
+    const int g = mad_segment_of([&](int k) { return kp_off[k]; }, G, i);
+    const int n = n_ori[i], p = pos[i];
+    for (int q = 0; q < n; ++q) {
+        if (p + q < cap) {
+            const int v = slots[(long long)i * MAD_MAX_ORI + q];
+            MadOriented of;
+            of.kp = i - kp_off[g];                       // map-local, as mad_compact_oriented writes it for the map alone
+            of.main_bin = (int16_t)(v & 0xFFFF);
+            of.sec_bin = (int16_t)(v >> 16);
+            out[p + q] = of;
+        }
+    }
+}
+
+}  // namespace
+
+extern "C" size_t mad_compact_oriented_many_workspace_bytes(int n_rows) {
+    size_t b = 0;
+    const int n = n_rows + 1;
+    cub::DeviceScan::ExclusiveSum(nullptr, b, (const int*)nullptr, (int*)nullptr, n);
+    return 2 * mad_align_up((size_t)n * sizeof(int), 256) + mad_align_up(b, 256);
+}
+
+extern "C" int mad_compact_oriented_many(const int32_t* n_ori, const int32_t* slots, int n_rows, const int* kp_off, int G,
+                                         MadOriented* oriented, int cap, int* ori_off, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+    MAD_CHECK_ARG(kp_off && ori_off && G >= 1 && n_rows >= 0 && n_rows < (1 << 30) && cap >= 0);
+    MAD_CHECK_ARG(workspace && workspace_bytes >= mad_compact_oriented_many_workspace_bytes(n_rows));
+    MAD_CHECK_ARG(n_rows == 0 || (n_ori && slots && oriented));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int n = n_rows + 1;
+    const size_t arr = mad_align_up((size_t)n * sizeof(int), 256);
+    int* cnt = reinterpret_cast<int*>(workspace);
+    int* pos = reinterpret_cast<int*>(reinterpret_cast<char*>(workspace) + arr);
+    char* cub_ws = reinterpret_cast<char*>(workspace) + 2 * arr;
+    size_t cub_bytes = workspace_bytes - 2 * arr;
+    {
+        MAD_PROF("ori_counts_many_kernel", st);
+        ori_counts_many_kernel<<<(int)mad_ceil_div(n, 256), 256, 0, st>>>(n_ori, kp_off, G, n_rows, cnt);
+        MAD_LAUNCH_OK();
+    }
+    {
+        MAD_PROF("cub_exclusive_sum", st);
+        MAD_CUDA(cub::DeviceScan::ExclusiveSum(cub_ws, cub_bytes, cnt, pos, n, st));
+    }
+    MAD_PROF("compact_oriented_many_kernel", st);
+    compact_oriented_many_kernel<<<(int)mad_ceil_div(std::max(n, G + 1), 256), 256, 0, st>>>(n_ori, slots, pos, kp_off, G,
+                                                                                            oriented, cap, ori_off);
     MAD_LAUNCH_OK();
     return MAD_OK;
 }

@@ -1249,15 +1249,9 @@ __global__ void gradient_flags_done_kernel(uint8_t* __restrict__ flags, size_t n
     if (i < n && flags[i] == 1) flags[i] = 2;
 }
 
-// One CTA per keypoint: requests every tile its box [vox - reach, vox + reach] touches (clipped to the grid).
-__global__ void gradient_mark_kernel(const MadKeypoint* __restrict__ kp, int n_kp, int nx0, int ny0, int nz0, int nx1,
-                                     int ny1, int nz1, int reach0, int reach1, uint8_t* __restrict__ flags0,
-                                     uint8_t* __restrict__ flags1) {
-    const MadKeypoint K = kp[blockIdx.x];
-    const int o = K.oct ? 1 : 0;
-    const int nx = o ? nx1 : nx0, ny = o ? ny1 : ny0, nz = o ? nz1 : nz0;
-    const int reach = o ? reach1 : reach0;
-    uint8_t* __restrict__ flags = o ? flags1 : flags0;
+// Requests every tile the box [vox - reach, vox + reach] of keypoint K touches (clipped to the grid); the CTA's threads
+// share the tiles.
+__device__ __forceinline__ void mark_box(const MadKeypoint& K, int nx, int ny, int nz, int reach, uint8_t* __restrict__ flags) {
     const int ty = (ny + kTile - 1) / kTile, tz = (nz + kTile - 1) / kTile;
     const int ax = max(K.vox[0] - reach, 0) / kTile, bx = min(K.vox[0] + reach, nx - 1) / kTile;
     const int ay = max(K.vox[1] - reach, 0) / kTile, by = min(K.vox[1] + reach, ny - 1) / kTile;
@@ -1269,7 +1263,47 @@ __global__ void gradient_mark_kernel(const MadKeypoint* __restrict__ kp, int n_k
         uint8_t* fl = flags + ((size_t)(ax + i) * ty + (ay + j)) * tz + (az + k);
         if (*fl == 0) *fl = 1;                                    // benign race: every writer stores 1
     }
+}
+
+// One CTA per keypoint: requests every tile its box [vox - reach, vox + reach] touches (clipped to the grid).
+__global__ void gradient_mark_kernel(const MadKeypoint* __restrict__ kp, int n_kp, int nx0, int ny0, int nz0, int nx1,
+                                     int ny1, int nz1, int reach0, int reach1, uint8_t* __restrict__ flags0,
+                                     uint8_t* __restrict__ flags1) {
+    const MadKeypoint K = kp[blockIdx.x];
+    const int o = K.oct ? 1 : 0;
+    const int nx = o ? nx1 : nx0, ny = o ? ny1 : ny0, nz = o ? nz1 : nz0;
+    const int reach = o ? reach1 : reach0;
+    uint8_t* __restrict__ flags = o ? flags1 : flags0;
+    mark_box(K, nx, ny, nz, reach, flags);
     (void)n_kp;
+}
+
+// mad_gradient_mark_many: gradient_mark_kernel's work for keypoint b of a batch (CTA b; none at or beyond kp_off[G]), in
+// the tiles of its map g (dims [g][6], flags [g][2] device addresses).
+__global__ void gradient_mark_many_kernel(const MadKeypoint* __restrict__ kp, const int* __restrict__ kp_off, int G,
+                                          const int* __restrict__ dims, const uint64_t* __restrict__ flags_tab, int reach0,
+                                          int reach1) {
+    const int ki = blockIdx.x;
+    if (ki >= kp_off[G]) return;
+    const int g = mad_segment_of([&](int k) { return kp_off[k]; }, G, ki);
+    const MadKeypoint K = kp[ki];
+    const int o = K.oct ? 1 : 0;
+    const int* d = dims + 6 * g + 3 * o;
+    const int nx = d[0], ny = d[1], nz = d[2];
+    const int reach = o ? reach1 : reach0;
+    uint8_t* __restrict__ flags = reinterpret_cast<uint8_t*>(flags_tab[2 * g + o]);
+    mark_box(K, nx, ny, nz, reach, flags);
+}
+
+extern "C" int mad_gradient_mark_many(const MadKeypoint* kp, const int* kp_off, int n_rows, int G, const int* dims,
+                                      const uint64_t* flags, int reach_oct0, int reach_oct1, void* stream) {
+    MAD_CHECK_ARG(kp_off && dims && flags && G >= 1 && n_rows >= 0 && reach_oct0 >= 0 && reach_oct1 >= 0);
+    if (n_rows == 0) return MAD_OK;
+    MAD_CHECK_ARG(kp);
+    MAD_PROF("gradient_mark_many_kernel", stream);
+    gradient_mark_many_kernel<<<n_rows, 128, 0, (cudaStream_t)stream>>>(kp, kp_off, G, dims, flags, reach_oct0, reach_oct1);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
 }
 
 extern "C" int mad_gradient(const float* gauss, int nx, int ny, int nz, float* grad4, void* stream) {

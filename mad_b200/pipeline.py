@@ -414,6 +414,150 @@ def describe_struct(grid, patch_size=16, map_padding=9, sig_init=2, sig_presmoot
     return sp, kp, ori, dsc
 
 
+def _to_device(values, dev, dtype=np.int64):
+    """Small host table -> device tensor through pinned memory (no synchronisation)."""
+    return torch.from_numpy(np.ascontiguousarray(values, dtype=dtype)).pin_memory().to(dev, non_blocking=True)
+
+
+class DescribedMaps(object):
+    """What ``describe_many`` returns: per map g, ``kp[g]`` (Keypoints), ``ori[g]`` (Oriented) and ``dsc[g]`` (int16
+    [D_g, 1024]), views of the batch tables ``kp_table``, ``ori_table`` and ``dsc_table``; ``kp_off`` / ``ori_off`` (host
+    int64 [G + 1]) delimit the maps in them (and ``kp_off_dev`` / ``ori_off_dev`` on the device), ``counts`` (host int64
+    [G, 2]) = (keypoints, oriented features) per map.  ``Oriented.kp`` is map-local, as ``orient`` writes it."""
+
+    def __init__(self, kp_table, ori_table, dsc_table, kp_off, ori_off, kp_off_dev, ori_off_dev):
+        self.kp_table, self.ori_table, self.dsc_table = kp_table, ori_table, dsc_table
+        self.kp_off, self.ori_off = kp_off, ori_off
+        self.kp_off_dev, self.ori_off_dev = kp_off_dev, ori_off_dev
+        self.G = len(kp_off) - 1
+        self.counts = np.stack([np.diff(kp_off), np.diff(ori_off)], 1)
+        self.kp = [Keypoints(kp_table[kp_off[g]:kp_off[g + 1]], kp_off[g + 1] - kp_off[g]) for g in range(self.G)]
+        self.ori = [Oriented(ori_table[ori_off[g]:ori_off[g + 1]], ori_off[g + 1] - ori_off[g]) for g in range(self.G)]
+        self.dsc = [dsc_table[ori_off[g]:ori_off[g + 1]] for g in range(self.G)]
+
+    def __len__(self):
+        return self.G
+
+    def feature_tables(self, voxelsps, origins):
+        """[FeatureTable] of every map, built on the device in one ``mad_feature_meta`` launch (``FeatureTable.from_device``
+        per map gives the same).  voxelsps[g]: map g's per-octave voxel sizes (``MapSpace.voxelsp_list``), origins[g]:
+        its padded origin (``MapSpace`` (xi, yi, zi))."""
+        if len(voxelsps) != self.G or len(origins) != self.G:
+            raise _lib.MadError("feature_tables: %d maps, got %d voxel sizes and %d origins" % (self.G, len(voxelsps), len(origins)))
+        meta, subv = _feature_meta(self.kp_table, self.ori_table, int(self.ori_off[-1]), self.kp_off_dev, self.ori_off_dev,
+                                   voxelsps, origins)
+        return [FeatureTable._from_columns(self.dsc[g], meta[self.ori_off[g]:self.ori_off[g + 1]],
+                                           subv[self.ori_off[g]:self.ori_off[g + 1]]) for g in range(self.G)]
+
+
+def _feature_meta(kp_table, ori_table, n, kp_off_dev, ori_off_dev, voxelsps, origins):
+    """(meta int32 [n, 4], subv float64 [n, 3]) of mad_feature_meta for the maps delimited by kp_off_dev / ori_off_dev."""
+    dev = kp_table.device
+    geo = np.zeros((len(voxelsps), 5), dtype=np.float64)
+    for g, (vs, org) in enumerate(zip(voxelsps, origins)):
+        vs, org = np.asarray(vs, dtype=np.float64).reshape(-1), np.asarray(org, dtype=np.float64).reshape(-1)
+        if vs.shape != (2,) or org.shape != (3,):
+            raise _lib.MadError("feature meta: map %d needs two octave voxel sizes and a 3-D origin, got %s and %s"
+                                % (g, vs.shape, org.shape))
+        geo[g, :2], geo[g, 2:] = vs, org
+    meta = torch.empty((n, 4), dtype=torch.int32, device=dev)
+    subv = torch.empty((n, 3), dtype=torch.float64, device=dev)
+    call("mad_feature_meta", _ptr(kp_table), _ptr(ori_table), n, _ptr(kp_off_dev), _ptr(ori_off_dev), len(geo),
+         _ptr(_to_device(geo, dev, np.float64)), _ptr(meta), _ptr(subv), _stream())
+    return meta, subv
+
+
+def describe_many(grids, patch_size=16, map_padding=9, sig_init=2, sig_presmooth=1, exact_f64=True, cap=None,
+                  oct_mode="both"):
+    """``describe_struct`` of G maps in one batch: map g's keypoint table, oriented table and descriptors equal
+    ``describe_struct(grids[g], patch_size, map_padding, sig_init, sig_presmooth, exact_f64)``'s bit for bit.
+    ``grids``: float32 [x][y][z] maps of any shapes (CUDA tensors or NumPy arrays).  Returns a DescribedMaps.
+
+    The dense stages (a1-a4) and the detection run per map, back to back on the current stream; the candidates of map g
+    go to rows [g cap, (g+1) cap) of one table (cap: candidates per map, default 2^16).  From there one launch per stage
+    serves the whole batch (keypoint sort, gradient tile marks, orientation, compaction, description; the masked gradient
+    still runs per map and octave), and the host reads the device twice for any G: the candidate counts, then the
+    keypoint and feature offsets.  A map with more than cap candidates makes the detection run again with room (a
+    third read).  Each map's scale space is freed as soon as the batch no longer needs it."""
+    _require_cuda()
+    if oct_mode != "both":
+        raise _lib.MadError("describe_many: oct_mode %r (the batch describes both octaves only)" % (oct_mode,))
+    grids = list(grids)
+    if not grids:
+        raise _lib.MadError("describe_many: no maps")
+    for g, grid in enumerate(grids):
+        if len(grid.shape) != 3:
+            raise _lib.MadError("describe_many: map %d has shape %s, not [x][y][z]" % (g, tuple(grid.shape)))
+    G = len(grids)
+    r = (patch_size - patch_size % 2) // 2
+    st = _stream()
+    spaces = []
+    for grid in grids:
+        sp = build_space(grid, map_padding, sig_init, sig_presmooth, exact_f64=exact_f64, keep_gauss=False, full_gradient=False)
+        sp.grids = []                                               # the padded and upsampled grids: no later stage reads them
+        spaces.append(sp)
+    dev = spaces[0].logs[0].device
+    dims = np.stack([sp.dims_host for sp in spaces]).astype(np.int32)          # [G][6]
+    dims_dev = _to_device(dims, dev, np.int32)
+    cap = int(cap) if cap is not None else 1 << 16
+    while True:                                                     # a5/a6 per map: (mad/Detector.py:18-128)
+        cand = torch.empty((G * cap, 12), dtype=torch.int32, device=dev)
+        counts = torch.zeros(G, dtype=torch.int32, device=dev)
+        for g, sp in enumerate(spaces):
+            for o, (lg, (gx, gy, gz)) in enumerate(zip(sp.logs, sp.dims)):
+                call("mad_detect", _ptr(lg), gx, gy, gz, o, 12, C.c_float(5e-2), C.c_void_p(cand[g * cap].data_ptr()), cap,
+                     C.c_void_p(counts[g:].data_ptr()), st)
+        n_cand = np.array(_Readback.read(counts), dtype=np.int64)
+        if n_cand.max() <= cap:
+            break
+        cap = int(n_cand.max() * 1.25) + 16                         # rare: a candidate region overflowed, redo with room
+    for sp in spaces:
+        sp.logs = []
+    n = int(n_cand.sum())
+    kp_table = torch.empty((max(n, 1), 12), dtype=torch.int32, device=dev)
+    kp_off_dev = torch.empty(G + 1, dtype=torch.int32, device=dev)
+    ws_bytes = _lib.lib.mad_sort_keypoints_many_workspace_bytes(n, G)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    call("mad_sort_keypoints_many", _ptr(cand), cap, _ptr(counts), G, n, _ptr(dims_dev), _ptr(kp_table), _ptr(kp_off_dev),
+         _ptr(ws), ws_bytes, st)
+    del cand, ws
+    # gradient tiles within reach of every keypoint (ensure_gradient), then the masked gradient per map and octave
+    up, base = gradient_reach(r)
+    flags = _to_device([[sp.grad_flags[0].data_ptr(), sp.grad_flags[1].data_ptr()] for sp in spaces], dev)
+    call("mad_gradient_mark_many", _ptr(kp_table), _ptr(kp_off_dev), n, G, _ptr(dims_dev), _ptr(flags), up, base, st)
+    for sp in spaces:
+        for o, (gx, gy, gz) in enumerate(sp.dims[:sp.n_oct]):
+            call("mad_gradient_masked", _ptr(sp._gauss[o]), gx, gy, gz, _ptr(sp.grad4[o]), _ptr(sp.grad_flags[o]), st)
+        sp._gauss = []
+    # a7-a10 over the batch (mad/Orientator.py:68-343)
+    tb = device_tables(dev)
+    grads = np.array([[sp.grad4[0].data_ptr(), sp.grad4[1].data_ptr()] for sp in spaces], dtype=np.int64)
+    n_ori = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
+    slots = torch.empty((max(n, 1), MAX_ORI), dtype=torch.int32, device=dev)
+    if n:
+        n_cand_i32 = n_cand.astype(np.int32)
+        call("mad_orient_many", _dptr(grads), _dptr(dims), _dptr(n_cand_i32), G, _ptr(kp_table), _ptr(kp_off_dev), int(r),
+             C.byref(tb.z_ori), _ptr(tb.r1), 6, 6, _ptr(n_ori), _ptr(slots), st)
+    ori_cap = max(n * MAX_ORI, 1)
+    ori_table = torch.empty((ori_cap, 2), dtype=torch.int32, device=dev)
+    ori_off_dev = torch.empty(G + 1, dtype=torch.int32, device=dev)
+    ws_bytes = _lib.lib.mad_compact_oriented_many_workspace_bytes(n)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    call("mad_compact_oriented_many", _ptr(n_ori), _ptr(slots), n, _ptr(kp_off_dev), G, _ptr(ori_table), ori_cap,
+         _ptr(ori_off_dev), _ptr(ws), ws_bytes, st)
+    del n_ori, slots, ws
+    offs = np.array(_Readback.read(kp_off_dev, ori_off_dev), dtype=np.int64)
+    kp_off, ori_off = offs[:G + 1], offs[G + 1:]
+    # a11/a12 over the batch (mad/Descriptor.py:106-202)
+    d = int(ori_off[-1])
+    dsc_table = torch.empty((d, DSC_LEN), dtype=torch.int16, device=dev)
+    if d:
+        kp_off_i32, ori_off_i32 = kp_off.astype(np.int32), ori_off.astype(np.int32)
+        call("mad_describe_many", _dptr(grads), _dptr(dims), _dptr(kp_off_i32), _dptr(ori_off_i32), G, _ptr(kp_table),
+             _ptr(ori_table), int(r), C.byref(tb.z_dsc), _ptr(tb.rf), _ptr(tb.rf_inv), tb.ori_zones, _ptr(dsc_table), st)
+    return DescribedMaps(kp_table, ori_table, dsc_table, kp_off, ori_off, kp_off_dev, ori_off_dev)
+
+
 # ---------------------------------------------------------------------------------------------
 # a15 matching
 # ---------------------------------------------------------------------------------------------
@@ -907,6 +1051,27 @@ class FeatureTable(object):
         self.subv = torch.from_numpy(self.subv_host).to(dev)
 
     @classmethod
+    def _from_columns(cls, dsc, meta, subv):
+        t = cls.__new__(cls)
+        t.set = dsc if isinstance(dsc, DescriptorSet) else DescriptorSet(dsc)
+        t.meta, t.subv = meta, subv
+        return t
+
+    @classmethod
+    def from_device(cls, kp, ori, dsc, voxelsp, origin):
+        """From the device tables of one map (Keypoints, Oriented, int16 descriptors, as ``describe_struct`` or
+        ``describe_many`` return them) without a trip to the host: meta and subv are built by ``mad_feature_meta`` and
+        equal, bit for bit, those of ``from_features`` on the map's DensityFeature list.  voxelsp: the per-octave voxel
+        sizes (``MapSpace.voxelsp_list``), origin: the padded origin (``MapSpace`` (xi, yi, zi)).  (The host copies
+        ``meta_host`` / ``subv_host`` are not made.)"""
+        _require_cuda()
+        dev = kp.table.device
+        n = len(ori)
+        meta, subv = _feature_meta(kp.table, ori.table, n, _to_device([0, len(kp)], dev, np.int32),
+                                   _to_device([0, n], dev, np.int32), [voxelsp], [origin])
+        return cls._from_columns(dsc[:n], meta, subv)
+
+    @classmethod
     def from_features(cls, df_list):
         """From a list of DensityFeature (the reference's ``lo_dsc_list`` / ``hi_dsc_list``)."""
         dsc = np.array([df.lin_ar_subeqsp for df in df_list], dtype=np.int16).reshape(-1, DSC_LEN)
@@ -1078,11 +1243,6 @@ def match_dsc_lists(lo_dsc_list, hi_dsc_list, anchor_dist_thresh=4, cc_threshold
 # ---------------------------------------------------------------------------------------------
 # one map against G structures (subunits of an assembly, frames of an ensemble) in one batch
 # ---------------------------------------------------------------------------------------------
-def _to_device(values, dev):
-    """Small int64 host list -> device tensor through pinned memory (no synchronisation)."""
-    return torch.tensor(np.asarray(values, dtype=np.int64)).pin_memory().to(dev, non_blocking=True)
-
-
 class AnchorClouds(object):
     """AnchorCloud for G segments in one pass (``mad_anchor_cloud_many``): segment g holds the entries [off[g], off[g+1]) of
     ``used``; shared_rows=False: the entries are rows of ``subv`` (the stacked hi rows), True: entry e of segment g is row
