@@ -463,6 +463,45 @@ int mad_normalise_f64(double* grid, long long n, void* scratch8, void* stream);
 int mad_conv_full_f64(const double* in, long long outer, int n, long long inner, const double* w_dev, int radius,
                       void* out, int out_is_f32, void* stream);
 
+/* A batch of G structures simulated together (PDB.density_many).  One record per structure; the caller fills min,
+ * n_atoms, dims and margin, mad_density_layout the rest.  Stage s of a structure is its box grown by 2 radius along the
+ * first s axes: stage 0 the splat [px][py][pz], stages 1 and 2 after the x and y passes (float64), stage 3 the float32 map
+ * [px + 2r][py + 2r][pz + 2r]; off[s] is its first element in the batch's flat buffer of that stage. */
+typedef struct MadDensityBox {
+    double min[3];         /* lattice-registered minimum corner of the atoms (mad/PDB.py:246-251) */
+    long long atom0;       /* its first atom in xyz / mass (the atoms of the batch are concatenated) */
+    long long off[4];      /* first element of each stage */
+    int n_atoms;
+    int dims[3];           /* splat box dims (mad/PDB.py:252-254) */
+    int margin;            /* 2 + pad */
+} MadDensityBox;
+/* mad_density_layout (host only): atom0 and off of boxes[G] from n_atoms, dims and radius; totals[5] = (atoms, elements of
+ * stages 0..3).  MAD_ERR_ARG for G outside [1, 65535], a structure without atoms, a dim < 1, margin < 1, or more than
+ * 2^31 - 1 corner contributions (8 per atom) in the batch.
+ * Every batched call below takes boxes_host = the table mad_density_layout laid out (checked: MAD_ERR_ARG otherwise,
+ * before any device work) and boxes = its device copy, made by the caller; its kernels run one CTA row per structure. */
+int mad_density_layout(MadDensityBox* boxes, int G, int radius, long long* totals);
+/* Deterministic splat of the batch into grid (stage 0, float64, zeroed by the call): the 8 corner contributions of every
+ * atom, in the order and with the products of mad/PDB.py:278-285, are stably radix-sorted by their global voxel, and one
+ * thread per voxel adds its run from 0.0 in that order.  Each voxel thus gets exactly the sum the reference's loop forms;
+ * no atomics.  xyz [atoms][3] and mass [atoms] float64, concatenated in the order of the table. */
+size_t mad_density_splat_many_workspace_bytes(int n_atoms);
+int mad_density_splat_many(const double* xyz, const double* mass, const MadDensityBox* boxes_host, int G,
+                           const MadDensityBox* boxes, double voxelsp, double* grid, void* workspace, size_t workspace_bytes,
+                           void* stream);
+/* mad_normalise_f64 for every structure's stage 0 (its own maximum); scratch = 8 G device bytes. */
+int mad_normalise_f64_many(double* grid, const MadDensityBox* boxes_host, int G, const MadDensityBox* boxes, void* scratch,
+                           void* stream);
+/* Pass `pass` (0 = x, 1 = y, 2 = z) of the "full" convolution for every structure: stage pass (in, float64) -> stage
+ * pass + 1 (out; float32 for pass 2).  A voxel is computed with the same fma chain as mad_conv_full_f64. */
+int mad_conv_full_f64_many(const double* in, const MadDensityBox* boxes_host, int G, const MadDensityBox* boxes, int pass,
+                           const double* w_dev, int radius, void* out, void* stream);
+/* Every map (stage 3) divided by its own maximum, then, when isovalue != 0, cut at it: what mad_grid_max,
+ * mad_threshold_normalise(-inf, max, 1) and mad_threshold_normalise(isovalue, 1, 0) do, with the maximum kept on the
+ * device.  scratch = 4 G device bytes. */
+int mad_map_normalise_many(float* maps, const MadDensityBox* boxes_host, int G, const MadDensityBox* boxes, int radius,
+                           float isovalue, void* scratch, void* stream);
+
 /* ---- next component (SURVEY.md 8f rank 4): scoring reductions and rigid refinement on HBM-resident grids -------- */
 /* One pass over the common box of two float32 grids [x][y][z]: box_host[9] = (x1, y1, z1, x2, y2, z2, ex, ey, ez), the box
  * start in each grid and its extent (the bounds of mad/Dmap.py:172-246).  out8 (device float64): [0] sum a b, [1] sum a a,
@@ -473,6 +512,25 @@ size_t mad_box_scores_workspace_bytes(int ex, int ey, int ez);
 int mad_box_scores(const float* g1, int nx1, int ny1, int nz1, const float* g2, int nx2, int ny2, int nz2,
                    const int* box_host, float isovalue, double* out8, void* workspace, size_t workspace_bytes,
                    void* stream);
+/* G grids against one target grid g1 (Dmap.get_CCC_with_grids).  One record per grid; the caller fills grid, dims and box
+ * (as box_host of mad_box_scores, g1 first; an extent <= 0 marks an empty box), mad_box_scores_layout the partition:
+ * (bx, by) = the one mad_box_scores picks for that box, part0 = its first CTA and partial in the batch.
+ * mad_box_scores_many: out [G][8], row g = mad_box_scores' out8 for grid g, bit for bit (same partition, partial layout
+ * and finish order); one launch for all partials, one finish CTA per grid.  workspace >= 64 max(1, n_partial) bytes.
+ * boxes_host = the laid-out table (checked, MAD_ERR_ARG otherwise), boxes = its device copy.
+ * mad_threshold_many: every grid of the table cut at isovalue in place (v < isovalue -> 0), in one launch. */
+typedef struct MadScoreBox {
+    const float* grid;
+    int dims[3];
+    int box[9];
+    long long part0;
+    int bx, by;
+} MadScoreBox;
+int mad_box_scores_layout(MadScoreBox* boxes, int G, long long* n_partial);
+int mad_box_scores_many(const float* g1, int nx1, int ny1, int nz1, const MadScoreBox* boxes_host, int G,
+                        const MadScoreBox* boxes, float isovalue, double* out, void* workspace, size_t workspace_bytes,
+                        void* stream);
+int mad_threshold_many(const MadScoreBox* boxes_host, int G, const MadScoreBox* boxes, float isovalue, void* stream);
 /* *out (device, reset by the call) = #{grid > thr}: np.count_nonzero(grid > isovalue), mad/Dmap.py:354. */
 int mad_grid_count_gt(const float* grid, long long n, float thr, unsigned long long* out, void* stream);
 /* Dmap.mask_with (mad/Dmap.py:99-151): g1 is zeroed outside [lo, hi) on any axis and wherever

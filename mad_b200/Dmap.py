@@ -227,6 +227,59 @@ class Dmap(object):
             return 0
         return s[0] / np.sqrt(s[1] * s[2])
 
+    def get_CCC_with_grids(self, grids, origins, isovalue=0):
+        """``get_CCC_with_grid`` of this map against G grids (e.g. ``PDB.density_many(...).grids``) with origins [G][3]:
+        float64 array [G] whose element g equals ``get_CCC_with_grid(grids[g], *origins[g], isovalue)`` exactly.  As there,
+        this map and every CUDA grid are cut at the isovalue in place (the G grids in one launch); a NumPy grid is uploaded.
+        The common boxes are checked before any device work (``ValueError`` naming the structure); a disjoint box scores 0.
+        One host read for the batch.  A batch holds at most 65535 grids (one CTA row each); a longer list is refused
+        (``ValueError``, before any device work), not split."""
+        from .pipeline import _Readback
+        G = len(grids)
+        if G > 65535:
+            raise ValueError("get_CCC_with_grids: %d grids; a batch holds at most 65535 (split it)" % G)
+        origins = np.asarray(origins, dtype=np.float64).reshape(G, 3) if G else np.zeros((0, 3))
+        voxsp = self.voxsp
+        o1 = [self.xi / voxsp, self.yi / voxsp, self.zi / voxsp]
+        boxes = (_lib.MadScoreBox * max(G, 1))()
+        disjoint = np.zeros(G, dtype=bool)
+        for g in range(G):
+            shape = [int(v) for v in grids[g].shape]
+            if len(shape) != 3 or (isinstance(grids[g], torch.Tensor) and (not grids[g].is_cuda or grids[g].dtype != torch.float32)):
+                raise ValueError("structure %d: a grid must be a float32 CUDA tensor or a NumPy array [x][y][z]" % g)
+            xi2, yi2, zi2 = origins[g]
+            try:
+                box = self._common_box(o1, [self.xb, self.yb, self.zb], [xi2 / voxsp, yi2 / voxsp, zi2 / voxsp], shape)
+            except ValueError as e:
+                raise ValueError("structure %d: %s" % (g, e))
+            disjoint[g] = box is None
+            boxes[g].dims[:] = shape
+            boxes[g].box[:] = box if box is not None else [0] * 9
+        if G == 0:
+            return np.zeros(0, dtype=np.float64)
+        dev = self._dev.device
+        st = _stream()
+        g2s = [self._as_device_grid(grid, dev) for grid in grids]
+        for g in range(G):
+            boxes[g].grid = g2s[g].data_ptr()
+        n_partial = C.c_longlong()
+        call("mad_box_scores_layout", boxes, G, C.byref(n_partial))
+        d_boxes = torch.from_numpy(np.frombuffer(bytearray(boxes), dtype=np.uint8)).pin_memory().to(dev, non_blocking=True)
+        call("mad_threshold_normalise", _ptr(self._dev), self._dev.numel(), C.c_float(isovalue), C.c_float(1.0), 0, st)
+        call("mad_threshold_many", boxes, G, _ptr(d_boxes), C.c_float(isovalue), st)
+        self._host = None
+        ws = torch.empty(max(1, n_partial.value) * 8, dtype=torch.float64, device=dev)
+        out = torch.empty((G, 8), dtype=torch.float64, device=dev)
+        n1 = [int(v) for v in self._dev.shape]
+        call("mad_box_scores_many", _ptr(self._dev), n1[0], n1[1], n1[2], boxes, G, _ptr(d_boxes), C.c_float(0.0), _ptr(out),
+             _ptr(ws), ws.numel() * 8, st)
+        s = np.array(_Readback.read(out.view(torch.int64)), dtype=np.int64).view(np.float64).reshape(G, 8)
+        res = np.zeros(G, dtype=np.float64)
+        for g in range(G):
+            if not disjoint[g]:
+                res[g] = s[g][0] / np.sqrt(s[g][1] * s[g][2])
+        return res
+
     def get_CCC_with_dmap(self, m2, isovalue=0):
         """mad/Dmap.py:260-372: overlap-normalised score against another Dmap."""
         if self.voxsp != m2.voxsp:

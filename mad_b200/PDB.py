@@ -48,6 +48,163 @@ def write_situs(outname, grid, voxelsp, dxi, dyi, dzi):
                     voxi += 1
 
 
+def _splat_box(xyz, voxelsp, margin):
+    """Lattice-registered minimum corner and splat box dims of atoms xyz [n][3] (host scalars, mad/PDB.py:236-254)."""
+    minx = voxelsp * floor(np.amin(xyz[:, 0]) / voxelsp)
+    maxx = voxelsp * ceil(np.amax(xyz[:, 0]) / voxelsp)
+    miny = voxelsp * floor(np.amin(xyz[:, 1]) / voxelsp)
+    maxy = voxelsp * ceil(np.amax(xyz[:, 1]) / voxelsp)
+    minz = voxelsp * floor(np.amin(xyz[:, 2]) / voxelsp)
+    maxz = voxelsp * ceil(np.amax(xyz[:, 2]) / voxelsp)
+    pxb = ceil((maxx - minx) / voxelsp) + 2 * margin + 1
+    pyb = ceil((maxy - miny) / voxelsp) + 2 * margin + 1
+    pzb = ceil((maxz - minz) / voxelsp) + 2 * margin + 1
+    return (minx, miny, minz), (pxb, pyb, pzb)
+
+
+def _gauss_1d(resolution, voxelsp):
+    """(r, w): radius and float64 weights [2r + 1] of the 1-D factor of the Gaussian, mad/PDB.py:138-150 (the 3-D kernel
+    exp(-(x^2+y^2+z^2) / 2 sig^2) / sum is a product of 1-D kernels)."""
+    sig = resolution / (np.pi * sqrt(2)) / voxelsp
+    r = int(ceil(3.0 * sig))
+    t = np.arange(-r, r + 1)
+    g1 = np.exp(-(t * t) / (2.0 * sig ** 2))
+    return r, np.ascontiguousarray(g1 / g1.sum())
+
+
+def _pinned_to(a, dev):
+    """One asynchronous host -> device copy through pinned memory (the caching host allocator keeps the pinned block until
+    the copy has run)."""
+    return torch.from_numpy(np.ascontiguousarray(a)).pin_memory().to(dev, non_blocking=True)
+
+
+MAX_BATCH = 65535          # structures per batch: the batched kernels run one CTA row (grid y) per structure
+MAX_DIM = 1 << 30          # a map's extent per axis (splat box + 2r), as mad_density_layout bounds it
+
+
+def _batch_atoms(structures, masses):
+    """(xyz [g] float64 [n_g][3], mass [g] float64 [n_g]) of density_many's inputs, checked on the host."""
+    if not structures:
+        raise _lib.MadError("density_many: no structures")
+    if len(structures) > MAX_BATCH:
+        raise _lib.MadError("density_many: %d structures; a batch holds at most %d (split it)" % (len(structures), MAX_BATCH))
+    per_structure = isinstance(masses, (list, tuple))
+    if per_structure and len(masses) != len(structures):
+        raise _lib.MadError("density_many: %d mass arrays for %d structures" % (len(masses), len(structures)))
+    xyzs, ms = [], []
+    for g, s in enumerate(structures):
+        if isinstance(s, PDB):                                    # density_many refuses masses next to PDB objects
+            xyz = np.asarray(s.coords, dtype=np.float64)
+            m = s._masses()
+        else:
+            xyz = np.asarray(s, dtype=np.float64)
+            if masses is None:
+                raise _lib.MadError("density_many: structure %d is a coordinate array and no masses were given" % g)
+            m = masses[g] if per_structure else masses
+        m = np.ascontiguousarray(m, dtype=np.float64).reshape(-1)
+        if xyz.ndim != 2 or xyz.shape[1] != 3 or xyz.shape[0] == 0:
+            raise _lib.MadError("density_many: structure %d has no atoms (coordinates of shape %s)" % (g, xyz.shape))
+        if not np.isfinite(xyz).all():
+            raise _lib.MadError("density_many: structure %d has non-finite coordinates" % g)
+        if len(m) != len(xyz):
+            raise _lib.MadError("density_many: structure %d has %d atoms and %d masses" % (g, len(xyz), len(m)))
+        xyzs.append(np.ascontiguousarray(xyz))
+        ms.append(m)
+    return xyzs, ms
+
+
+def _density_layout(xyzs, voxelsp, r, margin):
+    """The batch's MadDensityBox table laid out by mad_density_layout, the totals, and the map origins [G][3] (host)."""
+    G = len(xyzs)
+    boxes = (_lib.MadDensityBox * G)()
+    origins = np.empty((G, 3), dtype=np.float64)
+    for g, xyz in enumerate(xyzs):
+        mins, dims = _splat_box(xyz, voxelsp, margin)
+        if any(d + 2 * r >= MAX_DIM for d in dims):
+            raise _lib.MadError("density_many: structure %d spans a box of %s voxels (+ %d per axis for the Gaussian); "
+                                "each axis must stay below %d" % (g, list(dims), 2 * r, MAX_DIM))
+        b = boxes[g]
+        b.min[:] = mins
+        b.dims[:] = dims
+        b.n_atoms = len(xyz) if len(xyz) < (1 << 31) else -1
+        b.margin = margin
+        origins[g] = [mn - (r + margin) * voxelsp for mn in mins]
+    totals = (C.c_longlong * 5)()
+    call("mad_density_layout", boxes, G, r, totals)
+    return boxes, list(totals), origins
+
+
+class DensityBatch(object):
+    """The simulated maps of a batch: ``grids[g]`` = float32 CUDA view [x][y][z] of structure g's map in one flat buffer,
+    ``origins`` [G][3] = its (dxi, dyi, dzi) (host float64), ``voxelsp``."""
+
+    def __init__(self, maps, grids, origins, voxelsp):
+        self.maps = maps
+        self.grids = grids
+        self.origins = origins
+        self.voxelsp = voxelsp
+
+    def __len__(self):
+        return len(self.grids)
+
+    def host(self, g):
+        """What ``structure_to_density`` returns for structure g: (grid float32 [x][y][z], dxi, dyi, dzi)."""
+        dxi, dyi, dzi = (float(v) for v in self.origins[g])
+        return self.grids[g].cpu().numpy().astype(np.float32), dxi, dyi, dzi
+
+
+def density_many(structures, resolution, voxelsp, isovalue=0.0, pad=0, masses=None):
+    """``structure_to_density_device`` for G structures in one batch, with no host read and no device synchronisation.
+
+    ``structures``: ``PDB`` objects (masses from their elements; ``masses`` must then be None) or coordinate arrays
+    [n_g][3]; for arrays, ``masses`` is one array shared by every structure (poses of one structure) or a list / tuple of
+    one array per structure.  Every structure's float64 splat equals the reference's sequential loop (mad/PDB.py:278-285)
+    bit for bit (sorted contributions instead of atomics), and the map does not depend on the rest of the batch.  The
+    later stages are those of the single path.  Raises ``MadError`` naming the structure, before any device work, for an
+    empty list, a structure without atoms, non-finite coordinates, a mass count that does not match, or a box of 2^30
+    voxels or more along an axis.  A batch holds at most 65535 structures (one CTA row each); a longer list is refused,
+    not split."""
+    structures = list(structures)
+    if masses is not None and any(isinstance(s, PDB) for s in structures):
+        raise _lib.MadError("density_many: masses are taken from the PDB objects' elements")
+    xyzs, ms = _batch_atoms(structures, masses)
+    margin = 2 + pad
+    r, w = _gauss_1d(resolution, voxelsp)
+    boxes, totals, origins = _density_layout(xyzs, voxelsp, r, margin)
+    if not torch.cuda.is_available():
+        raise _lib.MadError("mad_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
+    G = len(xyzs)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    st = _stream()
+    d_xyz = _pinned_to(np.concatenate(xyzs), dev)
+    d_mass = _pinned_to(np.concatenate(ms), dev)
+    d_w = _pinned_to(w, dev)
+    d_boxes = _pinned_to(np.frombuffer(bytearray(boxes), dtype=np.uint8), dev)
+    ws = torch.empty(max(1, int(_lib.lib.mad_density_splat_many_workspace_bytes(int(totals[0])))), dtype=torch.uint8, device=dev)
+    splat = torch.empty(totals[1], dtype=torch.float64, device=dev)
+    call("mad_density_splat_many", _ptr(d_xyz), _ptr(d_mass), boxes, G, _ptr(d_boxes), C.c_double(voxelsp), _ptr(splat),
+         _ptr(ws), ws.numel(), st)
+    del ws, d_xyz, d_mass
+    scratch = torch.empty(G, dtype=torch.int64, device=dev)
+    call("mad_normalise_f64_many", _ptr(splat), boxes, G, _ptr(d_boxes), _ptr(scratch), st)
+    xpass = torch.empty(totals[2], dtype=torch.float64, device=dev)
+    call("mad_conv_full_f64_many", _ptr(splat), boxes, G, _ptr(d_boxes), 0, _ptr(d_w), r, _ptr(xpass), st)
+    del splat
+    ypass = torch.empty(totals[3], dtype=torch.float64, device=dev)
+    call("mad_conv_full_f64_many", _ptr(xpass), boxes, G, _ptr(d_boxes), 1, _ptr(d_w), r, _ptr(ypass), st)
+    del xpass
+    maps = torch.empty(totals[4], dtype=torch.float32, device=dev)
+    call("mad_conv_full_f64_many", _ptr(ypass), boxes, G, _ptr(d_boxes), 2, _ptr(d_w), r, _ptr(maps), st)
+    del ypass
+    call("mad_map_normalise_many", _ptr(maps), boxes, G, _ptr(d_boxes), r, C.c_float(isovalue), _ptr(scratch), st)
+    grids = []
+    for g in range(G):
+        shape = tuple(int(d) + 2 * r for d in boxes[g].dims)
+        o = int(boxes[g].off[3])
+        grids.append(maps[o:o + shape[0] * shape[1] * shape[2]].view(shape))
+    return DensityBatch(maps, grids, origins, voxelsp)
+
+
 class PDB(object):
     def __init__(self, pdb_file):
         self.pdb_file = pdb_file
@@ -146,17 +303,8 @@ class PDB(object):
         st = _stream()
         xyz = np.ascontiguousarray(self.coords, dtype=np.float64)
         mass = self._masses()
-        # lattice registration and box size (host scalars), mad/PDB.py:236-254
-        minx = voxelsp * floor(np.amin(xyz[:, 0]) / voxelsp)
-        maxx = voxelsp * ceil(np.amax(xyz[:, 0]) / voxelsp)
-        miny = voxelsp * floor(np.amin(xyz[:, 1]) / voxelsp)
-        maxy = voxelsp * ceil(np.amax(xyz[:, 1]) / voxelsp)
-        minz = voxelsp * floor(np.amin(xyz[:, 2]) / voxelsp)
-        maxz = voxelsp * ceil(np.amax(xyz[:, 2]) / voxelsp)
         margin = 2 + pad
-        pxb = ceil((maxx - minx) / voxelsp) + 2 * margin + 1
-        pyb = ceil((maxy - miny) / voxelsp) + 2 * margin + 1
-        pzb = ceil((maxz - minz) / voxelsp) + 2 * margin + 1
+        (minx, miny, minz), (pxb, pyb, pzb) = _splat_box(xyz, voxelsp, margin)
         d_xyz = torch.from_numpy(xyz).to(dev)
         d_mass = torch.from_numpy(mass).to(dev)
         grid = torch.empty((pxb, pyb, pzb), dtype=torch.float64, device=dev)
@@ -166,11 +314,8 @@ class PDB(object):
         scratch = torch.empty(1, dtype=torch.int64, device=dev)
         call("mad_normalise_f64", _ptr(grid), grid.numel(), _ptr(scratch), st)
         # Gaussian, mad/PDB.py:138-150: the 3-D kernel exp(-(x^2+y^2+z^2) / 2 sig^2) / sum is a product of 1-D kernels
-        sig = resolution / (np.pi * sqrt(2)) / voxelsp
-        r = int(ceil(3.0 * sig))
-        t = np.arange(-r, r + 1)
-        g1 = np.exp(-(t * t) / (2.0 * sig ** 2))
-        w = torch.from_numpy(np.ascontiguousarray(g1 / g1.sum())).to(dev)
+        r, w = _gauss_1d(resolution, voxelsp)
+        w = torch.from_numpy(w).to(dev)
         a = torch.empty((pxb + 2 * r, pyb, pzb), dtype=torch.float64, device=dev)
         call("mad_conv_full_f64", _ptr(grid), 1, pxb, pyb * pzb, _ptr(w), r, _ptr(a), 0, st)
         b = torch.empty((pxb + 2 * r, pyb + 2 * r, pzb), dtype=torch.float64, device=dev)

@@ -51,6 +51,16 @@ class MadCloudSeg(C.Structure):
                 ("org", C.c_double * 3), ("hi_n", C.c_int32), ("lo_n", C.c_int32), ("dims", C.c_int32 * 3), ("pad", C.c_int32)]
 
 
+class MadDensityBox(C.Structure):
+    _fields_ = [("min", C.c_double * 3), ("atom0", C.c_longlong), ("off", C.c_longlong * 4), ("n_atoms", C.c_int32),
+                ("dims", C.c_int32 * 3), ("margin", C.c_int32)]
+
+
+class MadScoreBox(C.Structure):
+    _fields_ = [("grid", C.c_void_p), ("dims", C.c_int32 * 3), ("box", C.c_int32 * 9), ("part0", C.c_longlong),
+                ("bx", C.c_int32), ("by", C.c_int32)]
+
+
 _P = C.c_void_p
 _I = C.c_int
 _SZ = C.c_size_t
@@ -115,6 +125,12 @@ SIGNATURES = {
     "mad_density_splat": (_I, [_P, _P, _I, _P, C.c_double, _I, _I, _I, _I, _P, _P]),
     "mad_normalise_f64": (_I, [_P, C.c_longlong, _P, _P]),
     "mad_conv_full_f64": (_I, [_P, C.c_longlong, _I, C.c_longlong, _P, _I, _P, _I, _P]),
+    "mad_density_layout": (_I, [_P, _I, _I, _P]),
+    "mad_density_splat_many_workspace_bytes": (_SZ, [_I]),
+    "mad_density_splat_many": (_I, [_P, _P, _P, _I, _P, C.c_double, _P, _P, _SZ, _P]),
+    "mad_normalise_f64_many": (_I, [_P, _P, _I, _P, _P, _P]),
+    "mad_conv_full_f64_many": (_I, [_P, _P, _I, _P, _I, _P, _I, _P, _P]),
+    "mad_map_normalise_many": (_I, [_P, _P, _I, _P, _I, C.c_float, _P, _P]),
     "mad_mark_used": (_I, [_P, C.c_longlong, _P, _P]),
     "mad_repeat_grid_cell": (C.c_double, [C.c_double]),
     "mad_repeatability": (_I, [_P, _P, _P, C.c_longlong, _P, _P, _P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _P, _P,
@@ -137,6 +153,9 @@ SIGNATURES = {
     "mad_repeat_rows_many": (_I, [_P, _P, _P, C.c_longlong, _P, _I, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P]),
     "mad_box_scores_workspace_bytes": (_SZ, [_I, _I, _I]),
     "mad_box_scores": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, C.c_float, _P, _P, _SZ, _P]),
+    "mad_box_scores_layout": (_I, [_P, _I, _P]),
+    "mad_box_scores_many": (_I, [_P, _I, _I, _I, _P, _I, _P, C.c_float, _P, _P, _SZ, _P]),
+    "mad_threshold_many": (_I, [_P, _I, _P, C.c_float, _P]),
     "mad_grid_count_gt": (_I, [_P, C.c_longlong, C.c_float, _P, _P]),
     "mad_mask_with": (_I, [_P, _I, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P]),
     "mad_refine_rigid": (_I, [_P, _I, _I, _I, _P, _P, _P, C.c_double, _P, _P, _P, _I, _I, _I, C.c_double, C.c_double,

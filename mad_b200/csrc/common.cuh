@@ -51,6 +51,24 @@ __host__ __device__ __forceinline__ int mad_segment_of(Off off, int G, long long
 
 int mad_sm_count();
 
+// ---- float32 grid maximum and isovalue cut / normalisation, shared by the single-grid (dmap.cu) and batched (density.cu)
+// kernels, so that a voxel of either goes through the same operations.
+// order-preserving map float -> unsigned (for atomicMax on floats of either sign); 0 lies below every float's image
+__device__ __forceinline__ unsigned int mad_f2ord(float f) {
+    const unsigned int u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__host__ __device__ __forceinline__ unsigned int mad_ord2bits(unsigned int ord) {
+    return (ord & 0x80000000u) ? (ord & 0x7FFFFFFFu) : ~ord;
+}
+// v < isovalue -> 0 (mad/Dmap.py:50-54), then v / vmax with a correctly rounded float32 division (:66-67; numpy divides
+// float32 by float32).  divide = 0 skips the normalisation.
+__device__ __forceinline__ float mad_threshold_normalise_one(float v, float isovalue, float vmax, int divide) {
+    if (v < isovalue) v = 0.f;
+    if (divide) v = __fdiv_rn(v, vmax);
+    return v;
+}
+
 // ---- per-map arguments of the batched orientation / description launches (mad_orient_many, mad_describe_many) ----
 // The table travels as one __grid_constant__ kernel parameter, so every read of it is a constant-bank operand, as the
 // single-map kernels' own arguments are; a batch of more maps is split into launches of kMadBatchMaps maps.

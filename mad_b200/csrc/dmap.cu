@@ -7,32 +7,20 @@
 
 namespace {
 
-// order-preserving map float -> unsigned (for atomicMax on floats of either sign)
-__device__ __forceinline__ unsigned int f2ord(float f) {
-    const unsigned int u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 __global__ void __launch_bounds__(256)
 grid_max_kernel(const float* __restrict__ g, long long n, unsigned int* __restrict__ out_ord) {
     unsigned int m = 0u;                                         // below every finite float's image
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
-        m = max(m, f2ord(__ldg(g + i)));
+        m = max(m, mad_f2ord(__ldg(g + i)));
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xFFFFFFFFu, m, o));
     if ((threadIdx.x & 31) == 0 && m) atomicMax(out_ord, m);
 }
 
-// v < isovalue -> 0 (mad/Dmap.py:50-54), then v / vmax with a correctly rounded float32 division
-// (:66-67; numpy divides float32 by float32).  divide = 0 skips the normalisation.
 __global__ void __launch_bounds__(256)
 threshold_normalise_kernel(float* __restrict__ g, long long n, float isovalue, float vmax, int divide) {
-    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        float v = g[i];
-        if (v < isovalue) v = 0.f;
-        if (divide) v = __fdiv_rn(v, vmax);
-        g[i] = v;
-    }
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        g[i] = mad_threshold_normalise_one(g[i], isovalue, vmax, divide);
 }
 
 // bbox[0..2] = min index of a non-zero voxel per axis, bbox[3..5] = max (mad/Dmap.py:77-80).
@@ -102,7 +90,7 @@ extern "C" int mad_grid_max(const float* grid, long long n, float* out_max, void
 }
 
 extern "C" float mad_grid_max_decode(unsigned int ord) {
-    const unsigned int u = (ord & 0x80000000u) ? (ord & 0x7FFFFFFFu) : ~ord;
+    const unsigned int u = mad_ord2bits(ord);
     float f;
     memcpy(&f, &u, sizeof(f));
     return f;

@@ -9,6 +9,8 @@
 // result is reproducible from run to run.
 #include <math.h>
 
+#include <vector>
+
 #include "common.cuh"
 
 namespace {
@@ -66,8 +68,8 @@ box_scores_kernel(const float* __restrict__ g1, int ny1, int nz1, const float* _
     }
 }
 
-__global__ void __launch_bounds__(256)
-box_scores_finish_kernel(const double* __restrict__ partial, int n_partial, double* __restrict__ out) {
+// sum of the n_partial partials in a fixed order (per thread, warp shuffle, then the 8 warps)
+__device__ __forceinline__ void box_scores_finish_cta(const double* __restrict__ partial, int n_partial, double* __restrict__ out) {
     __shared__ double red[8][kBoxSlots];
     double acc[kBoxSlots];
 #pragma unroll
@@ -86,6 +88,81 @@ box_scores_finish_kernel(const double* __restrict__ partial, int n_partial, doub
         for (int w = 0; w < 8; ++w) s += red[w][threadIdx.x];
         out[threadIdx.x] = s;
     }
+}
+
+__global__ void __launch_bounds__(256)
+box_scores_finish_kernel(const double* __restrict__ partial, int n_partial, double* __restrict__ out) {
+    box_scores_finish_cta(partial, n_partial, out);
+}
+
+// ---- G grids against one target (mad_box_scores_many): a 1-D grid over the CTAs of every structure's partition --------
+// CTA (bxi, byi) of structure g's (bx, by) partition does what CTA (bxi, byi) of box_scores_kernel's grid does for that
+// box: the same columns, slabs, sums and partial slot.  (A device function shared with box_scores_kernel changed that
+// kernel's instruction schedule, so its loop is restated here rather than shared.)
+__global__ void __launch_bounds__(kBoxThreads)
+box_scores_many_kernel(const float* __restrict__ g1, int ny1, int nz1, const MadScoreBox* __restrict__ boxes, int G, float iso,
+                       double* __restrict__ partial_all) {
+    const int g = mad_segment_of([&](int s) { return boxes[s].part0; }, G, (long long)blockIdx.x);
+    const MadScoreBox& bx_ = boxes[g];
+    const unsigned local = blockIdx.x - (unsigned)bx_.part0, gbx = (unsigned)bx_.bx, gby = (unsigned)bx_.by;
+    const unsigned bxi = local % gbx, byi = local / gbx;
+    const float* __restrict__ g2 = bx_.grid;
+    const int ny2 = bx_.dims[1], nz2 = bx_.dims[2];
+    const int x1 = bx_.box[0], y1 = bx_.box[1], z1 = bx_.box[2], x2 = bx_.box[3], y2 = bx_.box[4], z2 = bx_.box[5];
+    const int ex = bx_.box[6], ey = bx_.box[7], ez = bx_.box[8];
+    double* partial = partial_all + (size_t)bx_.part0 * kBoxSlots;
+    const unsigned plane = (unsigned)ey * (unsigned)ez;
+    const unsigned p = bxi * (unsigned)kBoxThreads + threadIdx.x;
+    double acc[kBoxSlots];
+#pragma unroll
+    for (int k = 0; k < kBoxSlots; ++k) acc[k] = 0.0;
+    if (p < plane) {
+        const int j = (int)(p / (unsigned)ez), k = (int)(p - (unsigned)j * (unsigned)ez);
+        const float* a_ptr = g1 + ((long long)x1 * ny1 + (y1 + j)) * nz1 + (z1 + k);
+        const float* b_ptr = g2 + ((long long)x2 * ny2 + (y2 + j)) * nz2 + (z2 + k);
+        const long long sa = (long long)ny1 * nz1, sb = (long long)ny2 * nz2;
+        unsigned n_iso = 0, n_pos = 0;
+        for (int i = byi; i < ex; i += gby) {
+            const double a = (double)__ldg(a_ptr + i * sa), b = (double)__ldg(b_ptr + i * sb);
+            acc[0] += a * b;
+            acc[1] += a * a;
+            acc[2] += b * b;
+            if (b > 0.0) acc[3] += a * a;
+            if (a > 0.0) acc[4] += b * b;
+            n_iso += (a > (double)iso && b > (double)iso);
+            n_pos += (a > 0.0 && b > 0.0);
+        }
+        acc[5] = (double)n_iso;
+        acc[6] = (double)n_pos;
+    }
+    __shared__ double red[kBoxThreads / 32][kBoxSlots];
+#pragma unroll
+    for (int k = 0; k < kBoxSlots; ++k) {
+        const double s = warp_sum(acc[k]);
+        if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5][k] = s;
+    }
+    __syncthreads();
+    if (threadIdx.x < kBoxSlots) {
+        double s = 0.0;
+        for (int w = 0; w < kBoxThreads / 32; ++w) s += red[w][threadIdx.x];
+        partial[((size_t)byi * gbx + bxi) * kBoxSlots + threadIdx.x] = s;
+    }
+}
+
+__global__ void __launch_bounds__(256)
+box_scores_finish_many_kernel(const MadScoreBox* __restrict__ boxes, const double* __restrict__ partial, double* __restrict__ out) {
+    const MadScoreBox& b = boxes[blockIdx.x];
+    box_scores_finish_cta(partial + (size_t)b.part0 * kBoxSlots, b.bx * b.by, out + (size_t)blockIdx.x * kBoxSlots);
+}
+
+// every grid of the table cut at the isovalue in place (threshold_normalise_kernel without the division)
+__global__ void __launch_bounds__(256)
+threshold_many_kernel(const MadScoreBox* __restrict__ boxes, float isovalue) {
+    const MadScoreBox& b = boxes[blockIdx.y];
+    float* g = const_cast<float*>(b.grid);
+    const long long n = (long long)b.dims[0] * b.dims[1] * b.dims[2];
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        g[i] = mad_threshold_normalise_one(g[i], isovalue, 1.f, 0);
 }
 
 __global__ void __launch_bounds__(256)
@@ -308,10 +385,20 @@ refine_kernel(const float4* __restrict__ grad, int nx, int ny, int nz, const dou
 
 }  // namespace
 
+namespace {
+
+// the (bx, by) partition of a non-empty common box: one CTA per 256 (y, z) columns, x split into slabs up to 8 CTAs per SM
+void box_partition(int ex, int ey, int ez, long long* bx, long long* by) {
+    *bx = mad_ceil_div((long long)ey * ez, kBoxThreads);
+    *by = std::min<long long>(ex, std::max<long long>(1, (long long)mad_sm_count() * 8 / *bx));
+}
+
+}  // namespace
+
 extern "C" size_t mad_box_scores_workspace_bytes(int ex, int ey, int ez) {
     if (ex <= 0 || ey <= 0 || ez <= 0) return 8 * sizeof(double);
-    const long long bx = mad_ceil_div((long long)ey * ez, kBoxThreads);
-    const long long by = std::min<long long>(ex, std::max<long long>(1, (long long)mad_sm_count() * 8 / bx));
+    long long bx, by;
+    box_partition(ex, ey, ez, &bx, &by);
     return (size_t)(bx * by) * kBoxSlots * sizeof(double);
 }
 
@@ -329,8 +416,8 @@ extern "C" int mad_box_scores(const float* g1, int nx1, int ny1, int nz1, const 
     MAD_CHECK_ARG(x1 >= 0 && y1 >= 0 && z1 >= 0 && x1 + ex <= nx1 && y1 + ey <= ny1 && z1 + ez <= nz1);
     MAD_CHECK_ARG(x2 >= 0 && y2 >= 0 && z2 >= 0 && x2 + ex <= nx2 && y2 + ey <= ny2 && z2 + ez <= nz2);
     MAD_CHECK_ARG(workspace_bytes >= mad_box_scores_workspace_bytes(ex, ey, ez));
-    const long long bx = mad_ceil_div((long long)ey * ez, kBoxThreads);
-    const long long by = std::min<long long>(ex, std::max<long long>(1, (long long)mad_sm_count() * 8 / bx));
+    long long bx, by;
+    box_partition(ex, ey, ez, &bx, &by);
     MAD_CHECK_ARG(bx < (1LL << 31) && by <= 65535);
     {
         MAD_PROF("box_scores_kernel", st);
@@ -343,6 +430,91 @@ extern "C" int mad_box_scores(const float* g1, int nx1, int ny1, int nz1, const 
         box_scores_finish_kernel<<<1, 256, 0, st>>>(static_cast<const double*>(workspace), (int)(bx * by), out8);
         MAD_LAUNCH_OK();
     }
+    return MAD_OK;
+}
+
+namespace {
+
+// bx, by and part0 of every record from its box; *n_partial = the partials of the whole batch
+int score_layout(MadScoreBox* boxes, int G, long long* n_partial) {
+    MAD_CHECK_ARG(boxes && n_partial && G >= 1);
+    long long n = 0;
+    for (int g = 0; g < G; ++g) {
+        MadScoreBox& b = boxes[g];
+        long long bx = 0, by = 0;
+        if (b.box[6] > 0 && b.box[7] > 0 && b.box[8] > 0) box_partition(b.box[6], b.box[7], b.box[8], &bx, &by);
+        MAD_CHECK_ARG(bx * by < (1LL << 31));
+        b.part0 = n;
+        b.bx = (int)bx;
+        b.by = (int)by;
+        n += bx * by;
+    }
+    MAD_CHECK_ARG(n < (1LL << 31));
+    *n_partial = n;
+    return MAD_OK;
+}
+
+// boxes_host must be the table mad_box_scores_layout laid out, every grid non-null with positive dims
+int check_score_layout(const MadScoreBox* boxes_host, int G, long long* n_partial) {
+    MAD_CHECK_ARG(boxes_host && G >= 1 && G <= 65535);
+    std::vector<MadScoreBox> laid(boxes_host, boxes_host + G);
+    const int rc = score_layout(laid.data(), G, n_partial);
+    if (rc != MAD_OK) return rc;
+    for (int g = 0; g < G; ++g) {
+        const MadScoreBox& b = boxes_host[g];
+        MAD_CHECK_ARG(laid[g].part0 == b.part0 && laid[g].bx == b.bx && laid[g].by == b.by);
+        MAD_CHECK_ARG(b.grid && b.dims[0] > 0 && b.dims[1] > 0 && b.dims[2] > 0);
+    }
+    return MAD_OK;
+}
+
+}  // namespace
+
+extern "C" int mad_box_scores_layout(MadScoreBox* boxes, int G, long long* n_partial) { return score_layout(boxes, G, n_partial); }
+
+extern "C" int mad_box_scores_many(const float* g1, int nx1, int ny1, int nz1, const MadScoreBox* boxes_host, int G,
+                                   const MadScoreBox* boxes, float isovalue, double* out, void* workspace,
+                                   size_t workspace_bytes, void* stream) {
+    MAD_CHECK_ARG(g1 && boxes && out && workspace);
+    long long n_partial;
+    const int rc = check_score_layout(boxes_host, G, &n_partial);
+    if (rc != MAD_OK) return rc;
+    for (int g = 0; g < G; ++g) {
+        const MadScoreBox& b = boxes_host[g];
+        const int* x = b.box;
+        if (x[6] <= 0 || x[7] <= 0 || x[8] <= 0) continue;              // empty common box: its row is zero
+        MAD_CHECK_ARG(x[0] >= 0 && x[1] >= 0 && x[2] >= 0 && x[0] + x[6] <= nx1 && x[1] + x[7] <= ny1 && x[2] + x[8] <= nz1);
+        MAD_CHECK_ARG(x[3] >= 0 && x[4] >= 0 && x[5] >= 0 && x[3] + x[6] <= b.dims[0] && x[4] + x[7] <= b.dims[1] &&
+                      x[5] + x[8] <= b.dims[2]);
+        MAD_CHECK_ARG(b.by <= 65535);
+    }
+    MAD_CHECK_ARG(workspace_bytes >= (size_t)std::max<long long>(n_partial, 1) * kBoxSlots * sizeof(double));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (n_partial > 0) {
+        MAD_PROF("box_scores_many_kernel", st);
+        box_scores_many_kernel<<<(unsigned)n_partial, kBoxThreads, 0, st>>>(g1, ny1, nz1, boxes, G, isovalue,
+                                                                           static_cast<double*>(workspace));
+        MAD_LAUNCH_OK();
+    }
+    MAD_PROF("box_scores_finish_many_kernel", st);
+    box_scores_finish_many_kernel<<<G, 256, 0, st>>>(boxes, static_cast<const double*>(workspace), out);
+    MAD_LAUNCH_OK();
+    return MAD_OK;
+}
+
+extern "C" int mad_threshold_many(const MadScoreBox* boxes_host, int G, const MadScoreBox* boxes, float isovalue, void* stream) {
+    MAD_CHECK_ARG(boxes);
+    long long n_partial;
+    const int rc = check_score_layout(boxes_host, G, &n_partial);
+    if (rc != MAD_OK) return rc;
+    long long max_n = 0;
+    for (int g = 0; g < G; ++g)
+        max_n = std::max(max_n, (long long)boxes_host[g].dims[0] * boxes_host[g].dims[1] * boxes_host[g].dims[2]);
+    const long long cap = std::max<long long>(1, (long long)mad_sm_count() * 16 / G);
+    const unsigned bx = (unsigned)std::max<long long>(1, std::min<long long>(mad_ceil_div(max_n, 256 * 4), cap));
+    MAD_PROF("threshold_many_kernel", stream);
+    threshold_many_kernel<<<dim3(bx, (unsigned)G), 256, 0, (cudaStream_t)stream>>>(boxes, isovalue);
+    MAD_LAUNCH_OK();
     return MAD_OK;
 }
 
